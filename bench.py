@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: MCTS simulations/s (and self-play games/s) for Connect4 self-play on B200, network in the loop.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload.  N = 1: BASELINE.json configs[2] — 16384 concurrent games x 800 simulations/move with a bf16 ResNet-style
@@ -26,6 +26,9 @@ move (`az_sample_moves`: record the samples, draw the moves, recycle finished ga
           simulation step exactly as search.py:82-84 does, on all host cores; each step a bounded sample (fewer games) of the
           same workload.  When baseline/_ref holds the reference's own Python (scripts/install_reference.py), its
           `EpisodeGenerator` is timed as well (`reference_python`: BASELINE config 1 exactly, E = 100, and one process per core).
+`--dump-outputs DIR`  the episodes the drain after the last timed step returned (rank 0), sorted as `EpisodeGenerator` yields
+          them, one float64 DIR/<field>.npy per `EpisodeBatch` field (at most 64 MB: above that, a seeded sample of whole episodes).
+          The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -35,6 +38,7 @@ import os
 import sys
 import time
 
+sys.dont_write_bytecode = True  # the tree may be read-only: the benchmark writes nothing there
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -61,7 +65,12 @@ def parse_args():
     ap.add_argument("--cpu-games", type=int, default=256, help="games of the CPU arm's bounded sample")
     ap.add_argument("--cpu-seconds", type=float, default=20.0)
     ap.add_argument("--trunk-variant", type=int, default=None, help="64-channel ResNet kernel: 4 = filter rows fused, N = 192 (csrc/az_resnet_wide.cu, default), 2 = layer-pipelined, two CTAs per SM (csrc/az_resnet_pipe.cu), 0 = one CTA per SM, 1 = ping-pong (csrc/az_conv.cu)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the episodes drained after the last timed step to DIR/<field>.npy (float64) for output comparison between builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def total_games(args, world: int) -> int:
@@ -196,7 +205,6 @@ def cpu_arm_net(spec: str, E: int, S: int, target_s: float, max_steps: int = 10*
     from oracle import c4oracle
     from oracle.net_eval import TorchNetEvaluator
 
-    c4oracle.build()
     cores = host_cores()
     cores = c4oracle.set_threads(cores)  # explicit: torchrun exports OMP_NUM_THREADS=1 to its workers
     torch.set_num_threads(cores)
@@ -221,7 +229,6 @@ def cpu_arm_builtin(E: int, S: int, kind: int, target_s: float = 8.0):
 
     from oracle import c4oracle
 
-    c4oracle.build()
     cores = c4oracle.set_threads(host_cores())
     rng = np.random.RandomState(0)
     c4oracle.selfplay(E, S, rng.random_sample((2, E)), quota=10**9, eval_kind=kind)
@@ -316,6 +323,31 @@ def concat_device(parts: list[dict]) -> dict:
     for k in parts[0]:
         out[k] = torch.cat(offs) if k == "ep_offset" else torch.cat([p[k] for p in parts])
     return out
+
+
+DUMP_LIMIT_BYTES = 63 << 20  # array bytes: with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir: str, drained: dict, limit: int = DUMP_LIMIT_BYTES) -> None:
+    """The episodes one drain returned, in the order the public API yields them (move step, then slot), as one float64 .npy per
+    `EpisodeBatch` field (bitboards use 49 bits, so float64 holds them exactly).  Above `limit` bytes a fixed seeded sample of
+    whole episodes is written instead; the sort comes first, so the sample does not depend on the ring's completion order."""
+    import dataclasses
+
+    import numpy as np
+
+    from alphazero_implementation_b200.engine import sort_episode_batch
+
+    b = sort_episode_batch({k: v.cpu().numpy() for k, v in drained.items()})
+    cost = 8 * (6 + 10 * b.ep_len.astype(np.int64))  # per episode: slot, step, len, offset, outcome[2]; per sample: bb0, bb1, player, counts[7]
+    if cost.sum() > limit:
+        order = np.random.RandomState(0).permutation(len(b))
+        keep = np.sort(order[np.cumsum(cost[order]) <= limit])
+        b = sort_episode_batch(dict(ep_slot=b.ep_slot[keep], ep_step=b.ep_step[keep], ep_len=b.ep_len[keep], ep_offset=b.ep_offset[keep],
+                                    ep_outcome=b.ep_outcome[keep], s_bb0=b.s_bb0, s_bb1=b.s_bb1, s_player=b.s_player, s_counts=b.s_counts))
+    os.makedirs(out_dir, exist_ok=True)
+    for f in dataclasses.fields(b):
+        np.save(os.path.join(out_dir, f.name + ".npy"), getattr(b, f.name).astype(np.float64))
 
 
 def kernel_timing_step(search, eng, u):
@@ -479,7 +511,7 @@ def run_b200(args):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     from alphazero_implementation_b200.distributed import all_gather_episodes, shard_range
 
-    W, K = max(3, args.warmup), max(1, args.steps)
+    W, K = max(3, args.warmup), args.steps
     G, S = total_games(args, world), args.sims
     lo, hi = shard_range(G, rank, world)
     E = hi - lo
@@ -552,6 +584,8 @@ def run_b200(args):
         k_region = {"launches": launch1 - launch0, "mean_ms": float(dur.mean().item()), "min_ms": float(dur.min().item()), "max_ms": float(dur.max().item())}
     az_lib.load().az_resnet_wide_set_timing(None, 0)  # off for everything that follows (extras build their own graphs)
     st = diff(st0, eng.stats())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, drained[-1])  # the last timed step always drains
     total_ms, ag_ms = ev0.elapsed_time(ev1), ag0.elapsed_time(ev1)
     step_ms = [step_ev[i].elapsed_time(step_ev[i + 1]) for i in range(K)]
     n_eps_job = int(merged["ep_len"].numel())
