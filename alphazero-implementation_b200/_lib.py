@@ -84,6 +84,10 @@ class AzStats(C.Structure):
                                            "moves", "episodes", "children_scanned")]
 
 
+class AzEvalCacheStats(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in ("rows", "hits", "followers", "failed_claims", "evictions")]
+
+
 class AzResnetDesc(C.Structure):
     _fields_ = [
         ("num_blocks", C.c_int32), ("num_channels", C.c_int32), ("operand_format", C.c_int32), ("variant", C.c_int32),
@@ -149,6 +153,9 @@ SIGNATURES = {
     "az_leaf_players": (I32, [P, C.POINTER(P)]),
     "az_leaf_compact": (I32, [P, C.POINTER(P), C.POINTER(P)]),
     "az_set_leaf_compaction": (I32, [P, I32]),
+    "az_set_eval_cache": (I32, [P, I32]),
+    "az_bump_eval_epoch": (I32, [P, P]),
+    "az_get_eval_cache_stats": (I32, [P, C.POINTER(AzEvalCacheStats), P]),
     "az_trunk_weight_bytes": (I64, [I32]),
     "az_resnet_pipe_weight_bytes": (I64, [I32, I32]),
     "az_trunk_forward_leaves": (I32, [P, P, P, I32, P, P]),

@@ -47,8 +47,22 @@ namespace {
 
 constexpr int PATH_STRIDE = 44;  // root + at most 42 plies (+1 pad)
 constexpr int MAX_PLIES = 42;
-constexpr int NSTAT = 7;  // per-tree counters: sims, evals, levels, children, moves, episodes, children scanned
+constexpr int NSTAT = 11;  // per-tree counters: sims, evals, levels, children, moves, episodes, children scanned, then the evaluation
+                           // cache's hits, followers, failed claims, evictions
 constexpr unsigned FULL = 0xFFFFFFFFu;
+
+// One entry of the evaluation cache (az_set_eval_cache), two per 128-byte bucket.  `ctrl` is the entry's state word: kind in
+// bits 0-1, the selection launch that set it in bits 2-31, a slot in bits 32-63.  Key, tag and payload are written only while
+// the entry is BUSY (taken by a CAS on ctrl), so a reader that sees the same non-BUSY ctrl before and after reading them holds
+// a consistent copy (a seqlock); ctrl never returns to an earlier value, because a slot claims or publishes at most once per launch.
+struct __align__(64) CacheEntry {
+    float4 p0, p1;  // outputs 0..7 as the evaluator wrote them: logits 0..6, value 0
+    float v1;       // output 8: value 1
+    uint32_t tag;   // weights epoch * 2 + side to move
+    unsigned long long ctrl;
+    unsigned long long b0, b1;  // the position
+};
+static_assert(sizeof(CacheEntry) == 64, "two entries per 128-byte bucket");
 
 struct Arena {
     double *W;
@@ -68,6 +82,13 @@ struct Arena {
     uint32_t *tstats;  // [E][NSTAT]
     int32_t *eval_list;   // [E] slots whose leaf waits for the evaluator: ascending (k_compact_leaves) or in ticket order (k_expand_select<COMPACT>)
     int32_t *eval_count;  // [4] [0] = entries in eval_list; [2..3] one 64-bit word: tickets | warps through << 32 (k_expand_select<COMPACT>; zero between launches)
+    // evaluation cache (az_set_eval_cache; the kernels that use it are the CACHE instantiations)
+    CacheEntry *cache;         // [2 * (cache_mask + 1)]: buckets of two entries
+    uint32_t cache_mask;       // buckets - 1
+    uint32_t *cache_ctl;       // [0] selection launches so far (advanced once after each selection launch), [1] weights epoch
+    uint32_t *leaf_src;        // [E] row the leaf's outputs come from: the slot itself, the leader slot of a follower, or SRC_HIT
+    uint32_t *leaf_claim;      // [E] entry the leaf claimed (its expansion publishes the row there), NO_CLAIM if none
+    float4 *cached_out;        // [E][3] the 9 outputs of a leaf served by a hit
     // game in progress per slot
     uint64_t *g_bb0, *g_bb1;  // [E][42]
     uint8_t *g_player;        // [E][42]
@@ -725,9 +746,162 @@ __global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, d
 }
 
 // ------------------------------------------------------------------------------------------------
+// evaluation cache (az_set_eval_cache).  The evaluator's row is a pure function of the position for a fixed set of weights, so a
+// position evaluated before (same weights epoch) is served from the table, and a position that another tree claimed in the same
+// selection launch reuses that tree's row: the search computes the same bits from fewer evaluator rows.
+constexpr uint32_t CE_BUSY = 1, CE_PENDING = 2, CE_READY = 3;
+constexpr uint32_t SRC_HIT = 0xFFFFFFFFu;   // leaf_src: the outputs are in cached_out
+constexpr uint32_t NO_CLAIM = 0xFFFFFFFFu;  // leaf_claim: nothing to publish
+constexpr uint32_t LAUNCH_MASK = 0x3FFFFFFFu;
+constexpr int PROBE_ATTEMPTS = 8;  // re-reads of a bucket another tree is writing before the leaf is evaluated uncached
+
+__device__ __forceinline__ unsigned long long ce_ctrl(uint32_t kind, uint32_t launch, uint32_t slot) {
+    return (unsigned long long)kind | ((unsigned long long)(launch & LAUNCH_MASK) << 2) | ((unsigned long long)slot << 32);
+}
+__device__ __forceinline__ uint32_t ce_kind(unsigned long long c) { return (uint32_t)c & 3u; }
+__device__ __forceinline__ uint32_t ce_launch(unsigned long long c) { return ((uint32_t)c >> 2) & LAUNCH_MASK; }
+
+__device__ __forceinline__ unsigned long long ld_acquire_u64(const unsigned long long *p) {
+    unsigned long long v;
+    asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ unsigned long long ld_relaxed_u64(const unsigned long long *p) {
+    unsigned long long v;
+    asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ uint4 ld_volatile_v4(const void *p) {
+    uint4 v;
+    asm volatile("ld.volatile.global.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ unsigned long long atom_add_acq_rel_u64(unsigned long long *p, unsigned long long v) {
+    unsigned long long old;
+    asm volatile("atom.acq_rel.gpu.global.add.u64 %0, [%1], %2;" : "=l"(old) : "l"(p), "l"(v) : "memory");
+    return old;
+}
+
+// The launch number and weights epoch of this launch, read by lane 0 of the warp (the lane whose ticket atomic in
+// k_expand_select<COMPACT> orders the read before the last warp advances the launch number) and broadcast.
+__device__ __forceinline__ void load_cache_ctl(const Arena &a, uint32_t &launch, uint32_t &epoch) {
+    uint32_t l = 0, e = 0;
+    if ((threadIdx.x & 31) == 0) {
+        l = *reinterpret_cast<const volatile uint32_t *>(a.cache_ctl);
+        e = *reinterpret_cast<const volatile uint32_t *>(a.cache_ctl + 1);
+    }
+    launch = __shfl_sync(FULL, l, 0);
+    epoch = __shfl_sync(FULL, e, 0);
+}
+
+// Probe of slot t's non-terminal leaf (one lane per tree).  Returns the leaf's status: AZ_LEAF_SERVED for a hit (outputs copied to
+// cached_out[t]) or a follower (leaf_src[t] = the slot whose row it reuses), AZ_LEAF_EVAL otherwise - with an entry claimed as
+// PENDING for this launch (leaf_claim[t]; the expansion publishes the row there) unless every entry of the bucket is taken.
+__device__ __forceinline__ uint8_t cache_probe(const Arena &a, int t, uint64_t b0, uint64_t b1, int pl, uint32_t launch, uint32_t epoch,
+                                            uint32_t *st) {
+    const uint32_t tag = epoch * 2u + (uint32_t)pl;
+    const uint64_t h = azeval::mix64(b0 ^ azeval::mix64(b1 + (uint64_t)tag));
+    CacheEntry *bk = a.cache + 2 * (size_t)((uint32_t)h & a.cache_mask);
+    const uint32_t now = launch & LAUNCH_MASK;
+    uint32_t claim = NO_CLAIM, src = (uint32_t)t;
+    uint8_t status = AZ_LEAF_EVAL;
+    int outcome = 2;  // st[] column - 7: 0 hit, 1 follower, 2 failed claim
+    for (int attempt = 0; attempt < PROBE_ATTEMPTS; ++attempt) {
+        if (attempt) __nanosleep(64);
+        unsigned long long c[2];
+        uint4 key[2], meta[2];  // {b0, b1}, {v1, tag, ctrl}
+#pragma unroll
+        for (int e = 0; e < 2; ++e) c[e] = ld_acquire_u64(&bk[e].ctrl);
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            key[e] = ld_volatile_v4(&bk[e].b0);
+            meta[e] = ld_volatile_v4(&bk[e].v1);
+        }
+        int match = -1, victim = -1;
+        bool busy = false, evict = false;
+        uint32_t best_age = 0;
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            const uint32_t kind = ce_kind(c[e]);
+            const bool same = key[e].x == (uint32_t)b0 && key[e].y == (uint32_t)(b0 >> 32) && key[e].z == (uint32_t)b1 &&
+                              key[e].w == (uint32_t)(b1 >> 32) && meta[e].y == tag;
+            const bool live_pending = kind == CE_PENDING && ce_launch(c[e]) == now;  // claimed in this launch: its row is coming
+            if (same && (kind == CE_READY || live_pending) && match < 0) match = e;
+            busy = busy || kind == CE_BUSY;
+            if (kind == CE_BUSY || live_pending) continue;
+            // free first (empty, a claim of an earlier launch, an older epoch's result), else the least recently published
+            const bool current = kind == CE_READY && (meta[e].y >> 1) == epoch;
+            const uint32_t age = current ? ((now - ce_launch(c[e])) & LAUNCH_MASK) : 0xFFFFFFFFu;
+            if (victim < 0 || age > best_age) {
+                victim = e;
+                best_age = age;
+                evict = current;
+            }
+        }
+        if (match >= 0) {  // (selects, not indexing: the arrays stay in registers)
+            const CacheEntry *m = bk + match;
+            const unsigned long long cm = match ? c[1] : c[0];
+            uint4 p0 = make_uint4(0u, 0u, 0u, 0u), p1 = p0;
+            const bool hit = ce_kind(cm) == CE_READY;
+            if (hit) {
+                p0 = ld_volatile_v4(&m->p0);
+                p1 = ld_volatile_v4(&m->p1);
+            }
+            __threadfence();
+            if (ld_relaxed_u64(&m->ctrl) != cm) continue;  // rewritten while we read it
+            if (hit) {
+                a.cached_out[(size_t)t * 3] = make_float4(__uint_as_float(p0.x), __uint_as_float(p0.y), __uint_as_float(p0.z), __uint_as_float(p0.w));
+                a.cached_out[(size_t)t * 3 + 1] = make_float4(__uint_as_float(p1.x), __uint_as_float(p1.y), __uint_as_float(p1.z), __uint_as_float(p1.w));
+                a.cached_out[(size_t)t * 3 + 2] = make_float4(__uint_as_float(match ? meta[1].x : meta[0].x), 0.0f, 0.0f, 0.0f);
+                src = SRC_HIT;
+                outcome = 0;
+            } else {
+                src = (uint32_t)(cm >> 32);
+                outcome = 1;
+            }
+            status = AZ_LEAF_SERVED;
+            break;
+        }
+        if (busy || victim < 0) continue;  // another tree is writing this bucket (perhaps this position): look again
+        CacheEntry *v = bk + victim;
+        const unsigned long long cv = victim ? c[1] : c[0];
+        if (atomicCAS(&v->ctrl, cv, ce_ctrl(CE_BUSY, now, (uint32_t)t)) != cv) continue;
+        __threadfence();
+        v->b0 = b0;
+        v->b1 = b1;
+        v->tag = tag;
+        __threadfence();
+        *reinterpret_cast<volatile unsigned long long *>(&v->ctrl) = ce_ctrl(CE_PENDING, now, (uint32_t)t);
+        claim = (uint32_t)(v - a.cache);
+        st[10] += evict ? 1u : 0u;
+        outcome = -1;
+        break;
+    }
+    if (outcome >= 0) st[7 + outcome] += 1u;
+    a.leaf_src[t] = src;
+    a.leaf_claim[t] = claim;
+    return status;
+}
+
+// The expansion of a leaf that claimed entry `claim` in the previous launch publishes its row there (one lane per tree); a claim
+// that another tree has taken over meanwhile (it counts as empty one launch later) is dropped.
+__device__ __forceinline__ void cache_publish(const Arena &a, uint32_t claim, int t, uint32_t launch, float4 p0, float4 p1, float v1) {
+    CacheEntry *e = a.cache + claim;
+    const unsigned long long want = ce_ctrl(CE_PENDING, launch - 1u, (uint32_t)t);
+    if (atomicCAS(&e->ctrl, want, ce_ctrl(CE_BUSY, launch, (uint32_t)t)) != want) return;
+    __threadfence();
+    e->p0 = p0;
+    e->p1 = p1;
+    e->v1 = v1;
+    __threadfence();
+    *reinterpret_cast<volatile unsigned long long *>(&e->ctrl) = ce_ctrl(CE_READY, launch, (uint32_t)t);
+}
+
+// ------------------------------------------------------------------------------------------------
 // split path, step 1: search.py:69-79
-template <int TPW, bool LAT>
-__device__ __forceinline__ bool select_body(const Arena &a, int n_active, double c_puct) {
+// CACHE: non-terminal leaves are probed in the evaluation cache; launch / epoch from load_cache_ctl
+template <int TPW, bool LAT, bool CACHE>
+__device__ __forceinline__ bool select_body(const Arena &a, int n_active, double c_puct, uint32_t launch, uint32_t epoch) {
     constexpr int TREES = 2 * TPW;
     constexpr int NL = 32 / TPW;
     const int lane = threadIdx.x & 31;
@@ -768,33 +942,38 @@ __device__ __forceinline__ bool select_body(const Arena &a, int n_active, double
     if (writer) path[0] = 0;
     uint32_t levels = 0, scanned = 0;
     Leaf L = descend<LAT>(tm, tb, rb0, rb1, rpl, c_puct, rm.z, root_sq, r_legal, rch, alive, writer, path, levels, scanned);
+    uint8_t status = L.term ? AZ_LEAF_TERMINAL : AZ_LEAF_EVAL;
     if (writer) {
+        uint32_t *st = a.tstats + (size_t)t * NSTAT;
+        if (CACHE && !L.term) status = cache_probe(a, t, L.b0, L.b1, L.pl, launch, epoch, st);
         a.leaf_node[t] = L.node;
         a.leaf_bb0[t] = L.b0;
         a.leaf_bb1[t] = L.b1;
         a.leaf_player[t] = (uint8_t)L.pl;
         a.leaf_depth[t] = (uint8_t)L.depth;
-        a.leaf_status[t] = L.term ? AZ_LEAF_TERMINAL : AZ_LEAF_EVAL;
-        uint32_t *st = a.tstats + (size_t)t * NSTAT;
+        a.leaf_status[t] = status;
         st[0] += 1u;
         st[2] += levels;
         st[6] += scanned;
     }
     __syncwarp();
     if (alive && L.term) backup(tm, path, L.depth, L.win ? 1.0 : 0.0, true, lit, NL);
-    return writer && !L.term;  // this lane wrote AZ_LEAF_EVAL for its tree
+    return writer && status == AZ_LEAF_EVAL;  // this lane wrote AZ_LEAF_EVAL for its tree
 }
 
 // split path, step 3: search.py:87-91 with the evaluator's outputs
-template <int TPW, bool LAT>
+template <int TPW, bool LAT, bool CACHE>
 __global__ void __launch_bounds__(64) k_select(Arena a, int n_active, double c_puct) {
-    select_body<TPW, LAT>(a, n_active, c_puct);
+    uint32_t launch = 0, epoch = 0;
+    if (CACHE) load_cache_ctl(a, launch, epoch);
+    select_body<TPW, LAT, CACHE>(a, n_active, c_puct, launch, epoch);
 }
 
 // split path, step 3: search.py:87-91 with the evaluator's outputs
-template <int TPW>
+// CACHE: a SERVED leaf takes its outputs from cached_out or from its leader's row, and a leaf that claimed an entry publishes its row
+template <int TPW, bool CACHE>
 __device__ __forceinline__ void expand_backup_body(const Arena &a, int n_active, const float *__restrict__ policy,
-                                                   const float *__restrict__ values, int policy_kind) {
+                                                   const float *__restrict__ values, int policy_kind, uint32_t launch) {
     constexpr int TREES = 2 * TPW;
     constexpr int NL = 32 / TPW;
     const int lane = threadIdx.x & 31;
@@ -815,10 +994,19 @@ __device__ __forceinline__ void expand_backup_body(const Arena &a, int n_active,
     const uint32_t used = a.used[tt];
     const uint32_t *path = a.path + (size_t)tt * PATH_STRIDE;
     const uint32_t my_idx = path[lit < PATH_STRIDE ? lit : 0];
-    const float x_raw = policy[(size_t)tt * 7 + (c < 7 ? c : 0)];
-    const float v0 = values[(size_t)tt * 2], v1 = values[(size_t)tt * 2 + 1];
-    const bool alive = (t < n_active) && status == AZ_LEAF_EVAL;
+    float x_raw = policy[(size_t)tt * 7 + (c < 7 ? c : 0)];
+    float v0 = values[(size_t)tt * 2], v1 = values[(size_t)tt * 2 + 1];
+    const uint32_t src = CACHE ? a.leaf_src[tt] : 0u;
+    const uint32_t claim = CACHE ? a.leaf_claim[tt] : NO_CLAIM;
+    const bool served = CACHE && status == AZ_LEAF_SERVED;
+    const bool alive = (t < n_active) && (status == AZ_LEAF_EVAL || served);
     if (!__any_sync(FULL, alive)) return;
+    if (served && alive) {  // the rows of SERVED leaves were not evaluated: the outputs are the leader's row or the cached copy
+        const float *o = src == SRC_HIT ? reinterpret_cast<const float *>(a.cached_out + (size_t)tt * 3) : policy + (size_t)src * 7;
+        x_raw = o[c < 7 ? c : 0];
+        v0 = src == SRC_HIT ? o[7] : values[(size_t)src * 2];
+        v1 = src == SRC_HIT ? o[8] : values[(size_t)src * 2 + 1];
+    }
     const bool writer = alive && lit == 0;
     const bool first_q = lit < 8;
     const size_t base = (size_t)tt * a.cap;
@@ -874,12 +1062,24 @@ __device__ __forceinline__ void expand_backup_body(const Arena &a, int n_active,
         }
         for (int i = lit + NL; i <= depth; i += NL) visit_node(tm, path[i], backup_sign(v, depth, i, false));
     }
+    if (CACHE) {
+        const bool publish = alive && status == AZ_LEAF_EVAL && claim != NO_CLAIM;
+        if (__any_sync(FULL, publish)) {
+            const int l0 = lane - lit;  // the tree's first lane: lanes l0 + 0..6 hold the row's 7 logits
+            float o[7];
+#pragma unroll
+            for (int j = 0; j < 7; ++j) o[j] = __shfl_sync(FULL, x_raw, l0 + j);
+            if (publish && writer) cache_publish(a, claim, t, launch, make_float4(o[0], o[1], o[2], o[3]), make_float4(o[4], o[5], o[6], v0), v1);
+        }
+    }
 }
 
-template <int TPW>
+template <int TPW, bool CACHE>
 __global__ void __launch_bounds__(64)
 k_expand_backup(Arena a, int n_active, const float *__restrict__ policy, const float *__restrict__ values, int policy_kind) {
-    expand_backup_body<TPW>(a, n_active, policy, values, policy_kind);
+    uint32_t launch = 0, epoch = 0;
+    if (CACHE) load_cache_ctl(a, launch, epoch);
+    expand_backup_body<TPW, CACHE>(a, n_active, policy, values, policy_kind, launch);
 }
 
 // Steps 3 and 1 of consecutive simulations in one launch: expansion + backup of simulation k, then the selection of simulation
@@ -891,22 +1091,28 @@ k_expand_backup(Arena a, int n_active, const float *__restrict__ policy, const f
 // in eval_count[0] and zeroes the word for the next launch.  No fences: the next kernel on the stream is the first reader.  The
 // list is a permutation of k_compact_leaves' ascending one (the order is the order of the tickets); the evaluators scatter their
 // outputs to the slots' rows and a position's outputs do not depend on the batch it falls into, so the search is unchanged.
-template <int TPW, bool LAT, bool COMPACT>
+// CACHE: both halves use the evaluation cache; with COMPACT the last warp also advances the launch number (the ticket atomic is then
+// acq_rel, so that every warp's read of the number at its start precedes the advance).
+template <int TPW, bool LAT, bool COMPACT, bool CACHE>
 __global__ void __launch_bounds__(64)
 k_expand_select(Arena a, int n_active, const float *__restrict__ policy, const float *__restrict__ values, int policy_kind, double c_puct) {
-    expand_backup_body<TPW>(a, n_active, policy, values, policy_kind);
+    uint32_t launch = 0, epoch = 0;
+    if (CACHE) load_cache_ctl(a, launch, epoch);
+    expand_backup_body<TPW, CACHE>(a, n_active, policy, values, policy_kind, launch);
     __syncwarp();
-    const bool wants = select_body<TPW, LAT>(a, n_active, c_puct);
+    const bool wants = select_body<TPW, LAT, CACHE>(a, n_active, c_puct, launch, epoch);
     if (COMPACT) {
         const int lane = threadIdx.x & 31;
         const unsigned m = __ballot_sync(FULL, wants);
         unsigned long long *word = reinterpret_cast<unsigned long long *>(a.eval_count + 2);
         unsigned long long old = 0ull;
         if (lane == 0) {
-            old = atomicAdd(word, (1ull << 32) | (unsigned long long)__popc(m));
+            const unsigned long long ticket = (1ull << 32) | (unsigned long long)__popc(m);
+            old = CACHE ? atom_add_acq_rel_u64(word, ticket) : atomicAdd(word, ticket);
             if ((unsigned)(old >> 32) == gridDim.x * 2u - 1u) {  // every other warp of the launch has its ticket
                 a.eval_count[0] = (int32_t)((unsigned)old + (unsigned)__popc(m));
                 *word = 0ull;
+                if (CACHE) a.cache_ctl[0] = launch + 1u;
             }
         }
         const int at = (int)__shfl_sync(FULL, (unsigned)old, 0);
@@ -920,11 +1126,14 @@ k_expand_select(Arena a, int n_active, const float *__restrict__ policy, const f
 // each thread counts its contiguous stretch of slots, a block-wide exclusive scan gives its offset (deterministic order, no atomics).
 // Thread t owns the slots [t * per, t * per + per), per a multiple of 16, and reads them as 16-byte vectors (the status array is
 // padded by 16 bytes): one L2 round trip per thread instead of one per slot.
-__device__ __forceinline__ uint32_t eval_bits(uint32_t w) { return ~(w | (w >> 1)) & 0x01010101u; }  // bit 8 i set <=> byte i == AZ_LEAF_EVAL (0); bytes are 0 / 1 / 2
-__global__ void __launch_bounds__(1024) k_compact_leaves(const uint8_t *__restrict__ status, int n, int32_t *__restrict__ list, int32_t *__restrict__ count, int staged) {
-    static_assert(AZ_LEAF_EVAL == 0 && AZ_LEAF_TERMINAL == 1 && AZ_LEAF_IDLE == 2, "eval_bits relies on the status encoding");
+__device__ __forceinline__ uint32_t eval_bits(uint32_t w) { return ~(w | (w >> 1)) & 0x01010101u; }  // bit 8 i set <=> byte i == AZ_LEAF_EVAL (0); bytes are 0 .. 3
+// `advance` (the evaluation cache's launch number, or null): one more selection launch is over.
+__global__ void __launch_bounds__(1024) k_compact_leaves(const uint8_t *__restrict__ status, int n, int32_t *__restrict__ list, int32_t *__restrict__ count, int staged,
+                                                         uint32_t *advance) {
+    static_assert(AZ_LEAF_EVAL == 0 && AZ_LEAF_TERMINAL == 1 && AZ_LEAF_IDLE == 2 && AZ_LEAF_SERVED == 3, "eval_bits relies on the status encoding");
     __shared__ int warp_tot[32];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (advance && tid == 0) *advance += 1u;
     const int per = (((n + 1023) / 1024) + 15) & ~15;
     const int lo = tid * per;
     int mine = 0;
@@ -1037,7 +1246,7 @@ k_encode(const uint64_t *__restrict__ bb0, const uint64_t *__restrict__ bb1, con
     if (t < n) {
         uint64_t b0 = bb0[t], b1 = bb1[t];
         const int pl = player[t] & 1;
-        const bool live = status ? (status[t] == AZ_LEAF_EVAL) : true;
+        const bool live = status ? (status[t] == AZ_LEAF_EVAL || status[t] == AZ_LEAF_SERVED) : true;
         if (LAYOUT == AZ_LAYOUT_GRID_F32) {
             // state.grid as f32: -1 empty / 0 / 1 owner (basic.py:41-47)
             const uint64_t m0 = to_row_major(b0), m1 = to_row_major(b1);
@@ -1299,7 +1508,7 @@ k_leaf_info(Arena a, int n, uint64_t *o0, uint64_t *o1, uint8_t *opl, uint8_t *o
     if (o0) o0[t] = a.leaf_bb0[t];
     if (o1) o1[t] = a.leaf_bb1[t];
     if (opl) opl[t] = a.leaf_player[t];
-    if (olegal) olegal[t] = st == AZ_LEAF_EVAL ? (uint8_t)c4::legal_mask(a.leaf_bb0[t] | a.leaf_bb1[t]) : 0;
+    if (olegal) olegal[t] = (st == AZ_LEAF_EVAL || st == AZ_LEAF_SERVED) ? (uint8_t)c4::legal_mask(a.leaf_bb0[t] | a.leaf_bb1[t]) : 0;
     if (ostatus) ostatus[t] = st;
 }
 
@@ -1465,7 +1674,7 @@ k_selftest_div(const double *__restrict__ rcp, int tab_n, unsigned long long see
 }
 
 __global__ void __launch_bounds__(256) k_sum_stats(const uint32_t *__restrict__ tstats, int E, unsigned long long *tot) {
-    unsigned long long loc[NSTAT] = {0, 0, 0, 0, 0, 0, 0};
+    unsigned long long loc[NSTAT] = {};
     for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < E; t += gridDim.x * blockDim.x)
         for (int q = 0; q < NSTAT; ++q) loc[q] += tstats[(size_t)t * NSTAT + q];
     for (int q = 0; q < NSTAT; ++q) {
@@ -1474,6 +1683,8 @@ __global__ void __launch_bounds__(256) k_sum_stats(const uint32_t *__restrict__ 
         if ((threadIdx.x & 31) == 0 && x) atomicAdd(&tot[q], x);
     }
 }
+
+__global__ void k_add_u32(uint32_t *p, uint32_t v) { *p += v; }
 
 __global__ void __launch_bounds__(256) k_zero_u32(uint32_t *p, long long n) {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
@@ -1509,12 +1720,16 @@ struct az_engine {
     int sims_done;  // simulations run on the current roots (arena and tables are sized for num_simulations)
     int compact;         // az_set_leaf_compaction: 1 = every selection is followed by k_compact_leaves, 2 = az_expand_backup_select builds the list itself
     bool compact_valid;  // eval_list / eval_count describe the leaves of the last selection
+    int cache_log2;      // az_set_eval_cache: 0 = off
+    void *cache_mem;
+    bool sel_pending;    // a selection's leaves wait for their expansion
+    bool cache_sel;      // ... and that selection used the evaluation cache (the expansion must, too)
     uint64_t init0, init1;
     int initpl;
     bool have_init;
     int64_t bytes;
     int64_t launches;
-    unsigned long long *d_tot;   // [8] stats totals (device)
+    unsigned long long *d_tot;   // [16] stats totals (device)
     unsigned long long acc_tot[NSTAT];  // totals folded on the host across resets
     void *allocs[96];
     int n_allocs;
@@ -1660,7 +1875,7 @@ int32_t az_create(const az_config *cfg, az_engine **out) {
     AL(a.root_bb0, E); AL(a.root_bb1, E); AL(a.root_player, E); AL(a.used, E); AL(a.tree_err, E);
     AL(a.leaf_node, E); AL(a.leaf_bb0, E); AL(a.leaf_bb1, E); AL(a.leaf_player, E); AL(a.leaf_status, E + 16);
     AL(a.leaf_depth, E); AL(a.path, (size_t)E * PATH_STRIDE); AL(a.tstats, (size_t)E * NSTAT);
-    AL(a.eval_list, E); AL(a.eval_count, 4);
+    AL(a.eval_list, E); AL(a.eval_count, 4); AL(a.cache_ctl, 4);
     AL(a.g_bb0, (size_t)E * MAX_PLIES); AL(a.g_bb1, (size_t)E * MAX_PLIES); AL(a.g_player, (size_t)E * MAX_PLIES);
     AL(a.g_counts, (size_t)E * MAX_PLIES * 7); AL(a.g_len, E);
     for (int r = 0; r < 2; ++r) {
@@ -1670,7 +1885,7 @@ int32_t az_create(const az_config *cfg, az_engine **out) {
         AL(g.ep_outcome, a.ep_cap * 2);
         AL(g.s_bb0, a.s_cap); AL(g.s_bb1, a.s_cap); AL(g.s_player, a.s_cap); AL(g.s_counts, a.s_cap * 7);
     }
-    AL(h->d_tot, 8);
+    AL(h->d_tot, 16);
 #undef AL
     if (rc != AZ_OK) {
         snprintf(g_create_error, sizeof g_create_error, "az_create: %s", h->err);
@@ -1687,9 +1902,10 @@ int32_t az_create(const az_config *cfg, az_engine **out) {
     cudaMemset(h->rings[0].ring, 0, 4 * sizeof(unsigned long long));
     cudaMemset(h->rings[1].ring, 0, 4 * sizeof(unsigned long long));
     use_ring(h, 0);
-    cudaMemset(h->d_tot, 0, 8 * sizeof(unsigned long long));
+    cudaMemset(h->d_tot, 0, 16 * sizeof(unsigned long long));
     cudaMemset(a.g_len, 0, (size_t)E * sizeof(int32_t));
     cudaMemset(a.eval_count, 0, 4 * sizeof(int32_t));
+    cudaMemset(a.cache_ctl, 0, 4 * sizeof(uint32_t));
     // every slot starts at the empty board, player 0 (Config.sample_initial_state())
     k_set_roots<<<blocks_for(E, 256), 256>>>(a, nullptr, nullptr, nullptr, 0ull, 0ull, 0, E, 1);
     h->launches++;
@@ -1713,6 +1929,7 @@ int32_t az_destroy(az_engine *h) {
     cudaSetDevice(h->cfg.device);
     cudaDeviceSynchronize();
     for (int i = 0; i < h->n_allocs; ++i) cudaFree(h->allocs[i]);
+    if (h->cache_mem) cudaFree(h->cache_mem);
     free(h);
     return AZ_OK;
 }
@@ -1855,6 +2072,7 @@ int32_t az_reset_games(az_engine *h, uint64_t init_bb0, uint64_t init_bb1, int32
     h->n_active = E;
     h->step = 0;
     h->sims_done = 0;
+    h->sel_pending = false;
     return AZ_OK;
 }
 
@@ -1867,6 +2085,7 @@ int32_t az_set_roots(az_engine *h, const uint64_t *bb0, const uint64_t *bb1, con
     AZ_LAUNCH_CHECK(h, "k_set_roots");
     h->n_active = n;
     h->sims_done = 0;
+    h->sel_pending = false;
     return AZ_OK;
 }
 
@@ -1991,6 +2210,10 @@ static int32_t run_sims_impl(az_engine *h, int32_t num_sims, int32_t eval_kind, 
     return AZ_OK;
 }
 
+// The selections probe the evaluation cache while it exists and the evaluator walks the compacted leaf list (the list's kernel, or the
+// last warp of k_expand_select<COMPACT>, advances the launch number that tells this launch's claims from earlier ones).
+static bool cache_active(const az_engine *h) { return h->a.cache != nullptr && h->compact != 0; }
+
 int32_t az_select_leaves(az_engine *h, void *stream) {
     if (!h) return AZ_E_INVALID;
     if (int rc = set_device(h)) return rc;
@@ -1999,10 +2222,16 @@ int32_t az_select_leaves(az_engine *h, void *stream) {
         return fail(h, AZ_E_INVALID, "%s", "az_select_leaves: more simulations on these roots than the arena holds");
     const int tpb = 2 * (32 / h->G);
     const bool lat = latency_variant(h, blocks_for(n, tpb));
-#define AZ_SEL(TPW_)                                                                                         \
-    do {                                                                                                     \
-        if (lat) k_select<TPW_, true><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct);     \
-        else k_select<TPW_, false><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct);        \
+    const bool cache = cache_active(h);
+#define AZ_SEL(TPW_)                                                                                                  \
+    do {                                                                                                              \
+        if (cache) {                                                                                                  \
+            if (lat) k_select<TPW_, true, true><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct);    \
+            else k_select<TPW_, false, true><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct);       \
+        } else {                                                                                                      \
+            if (lat) k_select<TPW_, true, false><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct);   \
+            else k_select<TPW_, false, false><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct);      \
+        }                                                                                                             \
     } while (0)
     if (h->G == 32) AZ_SEL(1);
     else if (h->G == 16) AZ_SEL(2);
@@ -2011,10 +2240,13 @@ int32_t az_select_leaves(az_engine *h, void *stream) {
     AZ_LAUNCH_CHECK(h, "k_select");
     h->compact_valid = h->compact != 0;
     if (h->compact) {
-        k_compact_leaves<<<1, 1024, 0, S(stream)>>>(h->a.leaf_status, n, h->a.eval_list, h->a.eval_count, env_int("AZ_COMPACT_STAGE", 1));
+        k_compact_leaves<<<1, 1024, 0, S(stream)>>>(h->a.leaf_status, n, h->a.eval_list, h->a.eval_count, env_int("AZ_COMPACT_STAGE", 1),
+                                                    cache ? h->a.cache_ctl : nullptr);
         AZ_LAUNCH_CHECK(h, "k_compact_leaves");
     }
     h->sims_done += 1;
+    h->sel_pending = true;
+    h->cache_sel = cache;
     return AZ_OK;
 }
 
@@ -2033,11 +2265,19 @@ int32_t az_expand_backup(az_engine *h, const float *policy, const float *values,
     if (policy_kind != AZ_POLICY_LOGITS && policy_kind != AZ_POLICY_PRIORS) return fail(h, AZ_E_INVALID, "%s", "az_expand_backup: bad policy_kind");
     if (int rc = set_device(h)) return rc;
     const int n = h->n_active;
-    if (h->G == 32) k_expand_backup<1><<<blocks_for(n, 2), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind);
-    else if (h->G == 16) k_expand_backup<2><<<blocks_for(n, 4), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind);
-    else k_expand_backup<4><<<blocks_for(n, 8), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind);
+    const bool cache = h->sel_pending && h->cache_sel;  // SERVED leaves and claims exist only after a cached selection
+#define AZ_EB(TPW_)                                                                                                   \
+    do {                                                                                                              \
+        if (cache) k_expand_backup<TPW_, true><<<blocks_for(n, 2 * TPW_), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind);  \
+        else k_expand_backup<TPW_, false><<<blocks_for(n, 2 * TPW_), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind);  \
+    } while (0)
+    if (h->G == 32) AZ_EB(1);
+    else if (h->G == 16) AZ_EB(2);
+    else AZ_EB(4);
+#undef AZ_EB
     AZ_LAUNCH_CHECK(h, "k_expand_backup");
     h->compact_valid = false;  // the leaves are consumed
+    h->sel_pending = false;
     return AZ_OK;
 }
 
@@ -2054,27 +2294,39 @@ int32_t az_expand_backup_select(az_engine *h, const float *policy, const float *
     const int tpb = 2 * (32 / h->G);
     const bool lat = latency_variant(h, blocks_for(n, tpb));
     const bool fused = h->compact == 2;
-#define AZ_ES(TPW_)                                                                                                                   \
+    const bool cache = cache_active(h);
+    if (h->sel_pending && h->cache_sel != cache)
+        return fail(h, AZ_E_STATE, "%s", "az_expand_backup_select: the evaluation cache or leaf compaction changed between a selection and its expansion");
+#define AZ_ES2(TPW_, LAT_, CMP_)                                                                                                      \
     do {                                                                                                                              \
-        if (fused) {                                                                                                                  \
-            if (lat) k_expand_select<TPW_, true, true><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct);  \
-            else k_expand_select<TPW_, false, true><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct);     \
-        } else {                                                                                                                      \
-            if (lat) k_expand_select<TPW_, true, false><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct); \
-            else k_expand_select<TPW_, false, false><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct);    \
-        }                                                                                                                             \
+        if (cache) k_expand_select<TPW_, LAT_, CMP_, true><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct);  \
+        else k_expand_select<TPW_, LAT_, CMP_, false><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct);  \
+    } while (0)
+#define AZ_ES(TPW_)                               \
+    do {                                          \
+        if (fused) {                              \
+            if (lat) AZ_ES2(TPW_, true, true);    \
+            else AZ_ES2(TPW_, false, true);       \
+        } else {                                  \
+            if (lat) AZ_ES2(TPW_, true, false);   \
+            else AZ_ES2(TPW_, false, false);      \
+        }                                         \
     } while (0)
     if (h->G == 32) AZ_ES(1);
     else if (h->G == 16) AZ_ES(2);
     else AZ_ES(4);
 #undef AZ_ES
+#undef AZ_ES2
     AZ_LAUNCH_CHECK(h, "k_expand_select");
     h->compact_valid = h->compact != 0;
     if (h->compact == 1) {
-        k_compact_leaves<<<1, 1024, 0, S(stream)>>>(h->a.leaf_status, n, h->a.eval_list, h->a.eval_count, env_int("AZ_COMPACT_STAGE", 1));
+        k_compact_leaves<<<1, 1024, 0, S(stream)>>>(h->a.leaf_status, n, h->a.eval_list, h->a.eval_count, env_int("AZ_COMPACT_STAGE", 1),
+                                                    cache ? h->a.cache_ctl : nullptr);
         AZ_LAUNCH_CHECK(h, "k_compact_leaves");
     }
     h->sims_done += 1;
+    h->sel_pending = true;
+    h->cache_sel = cache;
     return AZ_OK;
 }
 
@@ -2236,17 +2488,21 @@ int32_t az_read_episode_ring(az_engine *h, int32_t ring, int64_t n_episodes, int
                      S(stream));
 }
 
-int32_t az_get_stats(az_engine *h, az_stats *out, void *stream) {
-    if (!h || !out) return AZ_E_INVALID;
+static int sum_stats(az_engine *h, unsigned long long (&r)[NSTAT], cudaStream_t st) {
     if (int rc = set_device(h)) return rc;
-    cudaStream_t st = S(stream);
-    AZ_CUDA(h, cudaMemsetAsync(h->d_tot, 0, 8 * sizeof(unsigned long long), st));
+    AZ_CUDA(h, cudaMemsetAsync(h->d_tot, 0, NSTAT * sizeof(unsigned long long), st));
     k_sum_stats<<<148, 256, 0, st>>>(h->a.tstats, h->a.E, h->d_tot);
     AZ_LAUNCH_CHECK(h, "k_sum_stats");
-    unsigned long long r[8];
     AZ_CUDA(h, cudaMemcpyAsync(r, h->d_tot, sizeof r, cudaMemcpyDeviceToHost, st));
     AZ_CUDA(h, cudaStreamSynchronize(st));
     for (int q = 0; q < NSTAT; ++q) r[q] += h->acc_tot[q];
+    return AZ_OK;
+}
+
+int32_t az_get_stats(az_engine *h, az_stats *out, void *stream) {
+    if (!h || !out) return AZ_E_INVALID;
+    unsigned long long r[NSTAT];
+    if (int rc = sum_stats(h, r, S(stream))) return rc;
     out->simulations = r[0];
     out->evaluations = r[1];
     out->levels = r[2];
@@ -2255,6 +2511,65 @@ int32_t az_get_stats(az_engine *h, az_stats *out, void *stream) {
     out->moves = r[4];
     out->episodes = r[5];
     out->children_scanned = r[6];
+    return AZ_OK;
+}
+
+int32_t az_get_eval_cache_stats(az_engine *h, az_eval_cache_stats *out, void *stream) {
+    if (!h || !out) return AZ_E_INVALID;
+    unsigned long long r[NSTAT];
+    if (int rc = sum_stats(h, r, S(stream))) return rc;
+    out->rows = r[1] - r[7] - r[8];
+    out->hits = r[7];
+    out->followers = r[8];
+    out->failed_claims = r[9];
+    out->evictions = r[10];
+    return AZ_OK;
+}
+
+int32_t az_set_eval_cache(az_engine *h, int32_t log2_entries) {
+    if (!h) return AZ_E_INVALID;
+    if (log2_entries != 0 && (log2_entries < 10 || log2_entries > 30))
+        return fail(h, AZ_E_INVALID, "%s", "az_set_eval_cache: log2_entries must be 0 (off) or 10 .. 30");
+    if (h->sel_pending && h->cache_sel) return fail(h, AZ_E_STATE, "%s", "az_set_eval_cache: a cached selection waits for its expansion");
+    if (log2_entries == h->cache_log2) return AZ_OK;
+    if (int rc = set_device(h)) return rc;
+    if (h->cache_mem) {
+        AZ_CUDA(h, cudaDeviceSynchronize());
+        AZ_CUDA(h, cudaFree(h->cache_mem));
+        h->bytes -= (int64_t)sizeof(CacheEntry) << h->cache_log2;
+        h->cache_mem = nullptr;
+    }
+    h->a.cache = nullptr;
+    h->a.cache_mask = 0;
+    h->cache_log2 = 0;
+    if (log2_entries == 0) return AZ_OK;
+    if (!h->a.leaf_src) {
+        const int E = h->a.E;
+        int rc = dev_alloc(h, &h->a.leaf_src, E);
+        if (rc == AZ_OK) rc = dev_alloc(h, &h->a.leaf_claim, E);
+        if (rc == AZ_OK) rc = dev_alloc(h, &h->a.cached_out, (size_t)E * 3);
+        if (rc != AZ_OK) return rc;
+    }
+    const size_t bytes = sizeof(CacheEntry) << log2_entries;
+    cudaError_t e = cudaMalloc(&h->cache_mem, bytes);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        h->cache_mem = nullptr;
+        return fail(h, AZ_E_NOMEM, "az_set_eval_cache: cudaMalloc failed: %s", cudaGetErrorString(e));
+    }
+    AZ_CUDA(h, cudaMemset(h->cache_mem, 0, bytes));  // every entry EMPTY
+    h->bytes += (int64_t)bytes;
+    h->a.cache = static_cast<CacheEntry *>(h->cache_mem);
+    h->a.cache_mask = (1u << (log2_entries - 1)) - 1u;
+    h->cache_log2 = log2_entries;
+    return AZ_OK;
+}
+
+int32_t az_bump_eval_epoch(az_engine *h, void *stream) {
+    if (!h) return AZ_E_INVALID;
+    if (int rc = set_device(h)) return rc;
+    k_add_u32<<<1, 1, 0, S(stream)>>>(h->a.cache_ctl + 1, 1u);
+    AZ_LAUNCH_CHECK(h, "k_add_u32");
     return AZ_OK;
 }
 

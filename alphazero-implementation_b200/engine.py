@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import AzConfig, AzStats
+from ._lib import AzConfig, AzEvalCacheStats, AzStats
 
 EVAL_UNIFORM = 1
 EVAL_HASH = 2
@@ -21,7 +21,7 @@ LAYOUT_PLANES_BF16 = 2
 LAYOUT_PLANES_BF16_NHWC = 3
 POLICY_LOGITS = 0
 POLICY_PRIORS = 1
-LEAF_EVAL, LEAF_TERMINAL, LEAF_IDLE = 0, 1, 2
+LEAF_EVAL, LEAF_TERMINAL, LEAF_IDLE, LEAF_SERVED = 0, 1, 2, 3
 TREE_ROOT_ENDED = 3
 
 _LAYOUT_SHAPE = {
@@ -94,6 +94,7 @@ class Engine:
         self.n_active = self.num_games
         self.leaf_compaction = False
         self.leaf_compaction_fused = False
+        self.eval_cache_log2 = 0
         self.tree_capacity = self.lib.az_tree_capacity(self.h)
 
     # -- plumbing --------------------------------------------------------------------------------
@@ -190,6 +191,27 @@ class Engine:
         self._check(self.lib.az_set_leaf_compaction(self.h, mode), "az_set_leaf_compaction")
         self.leaf_compaction = bool(on)
         self.leaf_compaction_fused = mode == 2
+
+    def set_eval_cache(self, log2_entries: int | None):
+        """Evaluation cache of the leaves (`az_set_eval_cache`, active while leaf compaction is on): 2^log2_entries entries of 64
+        bytes, 0 = off.  None = sized for this engine: about one entry per simulation of a move step (at least 2^10, at most 2^24 =
+        1 GiB), so that the positions of the current and the previous move step fit at under half load.  Only for evaluators whose
+        output row is a pure function of the position; call it before a CUDA graph of the search is captured."""
+        if log2_entries is None:
+            log2_entries = min(24, max(10, (self.num_games * self.num_simulations - 1).bit_length()))
+        self._check(self.lib.az_set_eval_cache(self.h, int(log2_entries)), "az_set_eval_cache")
+        self.eval_cache_log2 = int(log2_entries)
+
+    def bump_eval_epoch(self):
+        """Cached evaluations stop matching (the evaluator's weights changed)."""
+        self._check(self.lib.az_bump_eval_epoch(self.h, _stream()), "az_bump_eval_epoch")
+
+    def eval_cache_stats(self) -> dict:
+        """rows (leaves the evaluator computed), hits, followers (leaves that reused another tree's row of the same selection),
+        failed_claims, evictions - totals since creation / `reset_stats`."""
+        st = AzEvalCacheStats()
+        self._check(self.lib.az_get_eval_cache_stats(self.h, C.byref(st), _stream()), "az_get_eval_cache_stats")
+        return {n: int(getattr(st, n)) for n, _ in AzEvalCacheStats._fields_}
 
     def run_simulations(self, num_sims: int, eval_kind: int):
         self._check(self.lib.az_run_simulations(self.h, int(num_sims), int(eval_kind), _stream()), "az_run_simulations")

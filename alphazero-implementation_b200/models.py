@@ -683,6 +683,12 @@ class InferenceNet(nn.Module):
         return self.trunk is not None
 
     @property
+    def position_only_outputs(self) -> bool:
+        """A leaf's outputs are a pure function of its position (deterministic, independent of the batch it falls in), so the
+        engine's evaluation cache may serve them: k_resnet_wide (tests/test_gpu_resnet_pipe.py pins both properties)."""
+        return isinstance(self.trunk, TensorCoreTrunk) and self.trunk.variant == 4
+
+    @property
     def kernel_name(self) -> str:
         if self.fused is not None:
             return "k_mlp_fused"

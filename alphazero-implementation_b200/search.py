@@ -88,11 +88,14 @@ class _GraphedStep:
 
     UNROLL = int(os.environ.get("AZ_GRAPH_UNROLL", "32"))  # simulations per replayed graph (a second capture; 1 = none): 16384 x 800, ResNet 4x64: 381.8 -> 372.7 ms per move step
 
-    def __init__(self, engine: Engine, net, layout: int):
+    def __init__(self, engine: Engine, net, layout: int, cache: bool | int = True):
         self.engine, self.net, self.layout = engine, net, layout
         # before the first selection (and any capture).  AZ_COMPACT_FUSED=0: the list of the leaves to evaluate comes from one more
         # launch per simulation (k_compact_leaves) instead of from k_expand_select itself
         engine.set_leaf_compaction(getattr(net, "wants_leaf_compaction", False), fused=os.environ.get("AZ_COMPACT_FUSED", "1") != "0")
+        # the evaluation cache changes no result bit when a leaf's outputs depend on its position alone
+        exact = engine.leaf_compaction and getattr(net, "position_only_outputs", False)
+        engine.set_eval_cache((None if cache is True else int(cache)) if cache and exact else 0)
         self.graph = None
         self.graph_unrolled = None
         self.n = -1
@@ -180,8 +183,12 @@ class _GraphedStep:
 class AlphaZeroSearch:
     def __init__(self, *, model, num_simulations: int, exploration_weight: float = 1.0, device: int | None = None,
                  lanes_per_tree: int = 0, inference_dtype: torch.dtype | None = None, use_cuda_graph: bool = True,
-                 use_tensor_core_kernels: bool = True, trunk_variant: int | None = None):
+                 use_tensor_core_kernels: bool = True, trunk_variant: int | None = None, eval_cache: bool | int = True):
+        """`eval_cache`: serve repeated leaf positions from the engine's evaluation cache (`Engine.set_eval_cache`) when the
+        evaluator's outputs depend on the position alone (`InferenceNet.position_only_outputs`); same results, fewer evaluator rows.
+        True = a table sized for the engine, False = off, an int = log2 of its entry count."""
         self.inference_model = model.get_inference_clone()
+        self.eval_cache = eval_cache
         self.num_simulations = int(num_simulations)
         self.exploration_weight = exploration_weight
         self.device_index = device
@@ -228,6 +235,9 @@ class AlphaZeroSearch:
             torch.cuda.current_stream(dev).synchronize()
         else:
             self._mode, self._net, self._graphed = "predict", None, None
+        if self._engine is not None:
+            self._engine.bump_eval_epoch()  # other weights or another evaluator: what the cache holds no longer applies
+            torch.cuda.current_stream(self._engine.device).synchronize()
 
     @property
     def evaluator_name(self) -> str:
@@ -276,7 +286,7 @@ class AlphaZeroSearch:
             engine.run_simulations(S, self.inference_model.az_builtin_eval_kind)
         elif self._mode == "net":
             if self._graphed is None or self._graphed.engine is not engine:
-                self._graphed = _GraphedStep(engine, self._net, self._net.input_layout)
+                self._graphed = _GraphedStep(engine, self._net, self._net.input_layout, self.eval_cache)
             self._graphed.run(S, self.use_cuda_graph, evaluator_events)
         else:
             self._simulate_predict(engine, S)

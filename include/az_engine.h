@@ -68,6 +68,8 @@ extern "C" {
 #define AZ_LEAF_EVAL 0     /* non-terminal leaf waiting for the evaluator */
 #define AZ_LEAF_TERMINAL 1 /* terminal leaf, already backed up (search.py:75-77) */
 #define AZ_LEAF_IDLE 2     /* slot inactive or in error */
+#define AZ_LEAF_SERVED 3   /* non-terminal leaf whose outputs come from the evaluation cache (az_set_eval_cache), not from
+                              a row of its own: it is not in the evaluator's list, and expand + backup treat it like AZ_LEAF_EVAL */
 
 /* per-tree error flags (az_root_stats `err`) */
 #define AZ_TREE_OK 0
@@ -172,6 +174,29 @@ int32_t az_leaf_players(az_engine *h, const uint8_t **player);
  * az_select_leaves (once per search) still takes the extra launch. */
 int32_t az_set_leaf_compaction(az_engine *h, int32_t on);
 int32_t az_leaf_compact(az_engine *h, const int32_t **eval_list, const int32_t **eval_count);
+
+/* Evaluation cache of the network-in-the-loop path: an open-addressed table in HBM (2-entry buckets of one 128-byte line)
+ * keyed by (position, side to move, weights epoch) that holds the evaluator's 9 outputs (7 logits, 2 values) exactly as it
+ * wrote them.  Only for evaluators whose output row is a pure function of the position (deterministic and independent of the
+ * batch it falls in): the search then computes the same bits with fewer evaluator rows.  Each selection probes the table for
+ * every non-terminal leaf: a published entry serves the leaf (AZ_LEAF_SERVED, no row), a position another tree of the same
+ * selection already claimed reuses that tree's row, and otherwise the leaf claims an entry and is evaluated; its expansion
+ * publishes the row.  Active while leaf compaction is on (az_set_leaf_compaction 1 or 2).
+ * az_set_eval_cache: 2^log2_entries entries of 64 bytes (10 <= log2_entries <= 30), 0 = off; a new size starts an empty table.
+ * Call it before capturing a CUDA graph of the search: launches bake the table's address in. */
+int32_t az_set_eval_cache(az_engine *h, int32_t log2_entries);
+/* Entries written before this call stop matching (a device word, so captured graphs see it): call it whenever the evaluator's
+ * weights change in place or another evaluator takes over. */
+int32_t az_bump_eval_epoch(az_engine *h, void *stream);
+typedef struct az_eval_cache_stats {
+    uint64_t rows;          /* non-terminal leaves the evaluator computed a row for */
+    uint64_t hits;          /* leaves served from a published entry */
+    uint64_t followers;     /* leaves that reused the row of another tree's leaf in the same selection */
+    uint64_t failed_claims; /* leaves evaluated without caching: no entry of their bucket could be claimed */
+    uint64_t evictions;     /* published entries of the current epoch replaced by a claim */
+} az_eval_cache_stats;
+/* totals since az_create / az_reset_stats (az_stats.evaluations = rows + hits + followers).  Synchronises. */
+int32_t az_get_eval_cache_stats(az_engine *h, az_eval_cache_stats *out_host, void *stream);
 
 /* ---- results ---- */
 /* root statistics of every active tree, per column (0 on illegal columns):
