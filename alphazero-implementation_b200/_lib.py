@@ -88,6 +88,10 @@ class AzEvalCacheStats(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in ("rows", "hits", "followers", "failed_claims", "evictions")]
 
 
+class AzRootNoise(C.Structure):
+    _fields_ = [("alpha", C.c_double), ("fraction", C.c_float), ("seed", C.c_uint64), ("slot_offset", C.c_int64)]
+
+
 class AzResnetDesc(C.Structure):
     _fields_ = [
         ("num_blocks", C.c_int32), ("num_channels", C.c_int32), ("operand_format", C.c_int32), ("variant", C.c_int32),
@@ -156,6 +160,10 @@ SIGNATURES = {
     "az_set_eval_cache": (I32, [P, I32]),
     "az_bump_eval_epoch": (I32, [P, P]),
     "az_get_eval_cache_stats": (I32, [P, C.POINTER(AzEvalCacheStats), P]),
+    "az_set_root_noise": (I32, [P, C.POINTER(AzRootNoise)]),
+    "az_apply_root_noise": (I32, [P, P]),
+    "az_root_noise_values": (I32, [P, P, P]),
+    "az_set_greedy_from": (I32, [P, I32]),
     "az_trunk_weight_bytes": (I64, [I32]),
     "az_resnet_pipe_weight_bytes": (I64, [I32, I32]),
     "az_trunk_forward_leaves": (I32, [P, P, P, I32, P, P]),

@@ -1515,8 +1515,12 @@ k_leaf_info(Arena a, int n, uint64_t *o0, uint64_t *o1, uint8_t *opl, uint8_t *o
 // ------------------------------------------------------------------------------------------------
 // This slot's part of a move step: record the sample, draw and play the move, emit the episode header if the game ended.
 // Returns through copy_len / copy_dst the finished game's samples still to be copied into the ring.
+// GREEDY (az_set_greedy_from): from ply `greedy_from` of the game on, the move is the most visited root child, the lowest
+// column on ties (select_action of deepmind_alphazero_pseudocode.py past num_sampling_moves); earlier plies are sampled.
+template <bool GREEDY>
 __device__ __forceinline__ void sample_move_slot(const Arena &a, int t, const double *__restrict__ uniforms, uint8_t *finished, int step,
-                                                 uint64_t init0, uint64_t init1, int initpl, int &copy_len, long long &copy_dst) {
+                                                 uint64_t init0, uint64_t init1, int initpl, int greedy_from, int &copy_len,
+                                                 long long &copy_dst) {
     if (finished) finished[t] = 0;
     if (a.tree_err[t]) return;
     const size_t base = (size_t)t * a.cap;
@@ -1558,15 +1562,27 @@ __device__ __forceinline__ void sample_move_slot(const Arena &a, int t, const do
         for (int c = 0; c < 7; ++c) a.g_counts[o * 7 + c] = cnt[c];
     }
     const int new_len = len + 1;
-    // np.random.choice(k, p): cdf /= cdf[-1]; idx = searchsorted(cdf, u, side='right') = #{cdf <= u}
-    const double u = uniforms[t];
-    const double last = acc;
-    int idx = 0;
+    int col;
+    if (GREEDY && len >= greedy_from) {
+        int32_t best = -1;
+        col = 0;
 #pragma unroll
-    for (int c = 0; c < 7; ++c)
-        if (((legal >> c) & 1u) && __ddiv_rn(cdf[c], last) <= u) ++idx;
-    if (idx >= k) idx = k - 1;
-    const int col = c4::nth_legal_column(legal, idx);
+        for (int c = 0; c < 7; ++c)
+            if (((legal >> c) & 1u) && cnt[c] > best) {  // strict '>': the first maximum
+                best = cnt[c];
+                col = c;
+            }
+    } else {
+        // np.random.choice(k, p): cdf /= cdf[-1]; idx = searchsorted(cdf, u, side='right') = #{cdf <= u}
+        const double u = uniforms[t];
+        const double last = acc;
+        int idx = 0;
+#pragma unroll
+        for (int c = 0; c < 7; ++c)
+            if (((legal >> c) & 1u) && __ddiv_rn(cdf[c], last) <= u) ++idx;
+        if (idx >= k) idx = k - 1;
+        col = c4::nth_legal_column(legal, idx);
+    }
     const uint64_t bit = c4::drop_bit(b0 | b1, col);
     if (pl == 0) b0 |= bit; else b1 |= bit;
     const bool win = c4::has4(pl ? b1 : b0);
@@ -1608,14 +1624,15 @@ __device__ __forceinline__ void sample_move_slot(const Arena &a, int t, const do
 // self-play move step (episode_generator.py:53-78, node.py:23-42): one thread per slot for the move itself; the samples of
 // games that ended (up to 42 x 45 bytes each, cold in L2 / HBM) are then copied into the ring by the whole warp, one
 // lane per sample, so the few threads with a finished game do not serialise dozens of dependent loads.
+template <bool GREEDY>
 __global__ void __launch_bounds__(128)
 k_sample_moves(Arena a, int n, const double *__restrict__ uniforms, uint8_t *finished, int step, uint64_t init0,
-               uint64_t init1, int initpl) {
+               uint64_t init1, int initpl, int greedy_from) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
     int copy_len = 0;
     long long copy_dst = 0;
-    if (t < n) sample_move_slot(a, t, uniforms, finished, step, init0, init1, initpl, copy_len, copy_dst);
+    if (t < n) sample_move_slot<GREEDY>(a, t, uniforms, finished, step, init0, init1, initpl, greedy_from, copy_len, copy_dst);
     __syncwarp();  // the sample recorded by this step is visible to the lanes that copy it
     unsigned todo = __ballot_sync(FULL, copy_len > 0);
     while (todo) {
@@ -1631,6 +1648,86 @@ k_sample_moves(Arena a, int n, const double *__restrict__ uniforms, uint8_t *fin
         }
         for (int i = lane; i < len * 7; i += 32) a.s_counts[dst * 7 + i] = a.g_counts[g0 * 7 + i];
     }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Dirichlet noise on the root priors (az_set_root_noise / az_apply_root_noise; add_exploration_noise of
+// deepmind_alphazero_pseudocode.py).  η of a tree is a pure function of (seed, global slot, draw number, column): Philox4x32-10
+// keyed by the seed, counter {global slot lo, hi, draw, column << 24 | attempt}, so a sharded run draws what the unsharded run
+// draws for the same games.  Gamma variates by Marsaglia-Tsang, every attempt of the rejection loop on its own counter; for
+// alpha < 1 in log space, log G(alpha + 1) + log(U) / alpha, normalised with a max-subtracted exp, so that a small alpha cannot
+// underflow every component to 0.
+constexpr int NOISE_MAX_ATTEMPTS = 1 << 16;  // acceptance is >= 95 % per attempt: never reached in practice
+
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
+        c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+        k.x += 0x9E3779B9u;
+        k.y += 0xBB67AE85u;
+    }
+    return c;
+}
+
+__device__ __forceinline__ double u01_open(uint32_t x) { return ((double)x + 0.5) * 0x1p-32; }  // (0, 1)
+
+// log of a Gamma(alpha, 1) variate
+__device__ double log_gamma_variate(double alpha, uint2 key, uint4 ctr) {
+    const bool boost = alpha < 1.0;
+    const double d = (boost ? alpha + 1.0 : alpha) - 1.0 / 3.0;
+    const double cc = 1.0 / sqrt(9.0 * d);
+    double lg = log(d), ub = 0.5;
+    for (uint32_t attempt = 0; attempt < (uint32_t)NOISE_MAX_ATTEMPTS; ++attempt) {
+        const uint4 r = philox4x32_10(make_uint4(ctr.x, ctr.y, ctr.z, ctr.w | attempt), key);
+        const double x = sqrt(-2.0 * log(u01_open(r.x))) * cospi(2.0 * u01_open(r.y));  // Box-Muller
+        double v = 1.0 + cc * x;
+        if (v <= 0.0) continue;
+        v = v * v * v;
+        if (log(u01_open(r.z)) < 0.5 * x * x + d - d * v + d * log(v)) {
+            lg = log(d * v);
+            ub = u01_open(r.w);  // not part of the acceptance test: an independent uniform
+            break;
+        }
+    }
+    return boost ? lg + log(ub) / alpha : lg;
+}
+
+// eight lanes per tree, lane c < 7 = column c.  Trees in error or without children (the first simulation did not expand the
+// root) are left alone; their η rows, and those of inactive slots, are 0.
+__global__ void __launch_bounds__(256)
+k_root_noise(Arena a, int n_active, double alpha, float fraction, unsigned long long seed, long long slot_offset, uint32_t draw,
+             float *__restrict__ eta) {
+    const int t = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 3);
+    const int c = threadIdx.x & 7;
+    const int tt = t < a.E ? t : 0;
+    const size_t base = (size_t)tt * a.cap;
+    const uint32_t cb = a.M[base].z;
+    const bool act = t < n_active && a.tree_err[tt] == 0 && cb != 0;
+    const uint32_t legal = act ? c4::legal_mask(a.root_bb0[tt] | a.root_bb1[tt]) : 0u;
+    const bool mine = c < 7 && ((legal >> c) & 1u);
+    double lg = -INFINITY;
+    if (mine) {
+        const unsigned long long g = (unsigned long long)(slot_offset + t);
+        const uint2 key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
+        lg = log_gamma_variate(alpha, key, make_uint4((uint32_t)g, (uint32_t)(g >> 32), draw, (uint32_t)c << 24));
+    }
+    double m = lg;
+#pragma unroll
+    for (int off = 4; off >= 1; off >>= 1) m = fmax(m, __shfl_xor_sync(FULL, m, off));
+    const double e = mine ? exp(lg - m) : 0.0;
+    double s = e;
+#pragma unroll
+    for (int off = 4; off >= 1; off >>= 1) s += __shfl_xor_sync(FULL, s, off);
+    const float h = mine ? (float)(e / s) : 0.0f;
+    if (mine) {
+        // P' = RN(RN(RN(1 - eps) * P) + RN(eps * eta)), fp32, one rounding per operation
+        uint32_t *py = reinterpret_cast<uint32_t *>(a.M + base + cb + __popc(legal & ((1u << c) - 1u))) + 1;
+        const float p = __uint_as_float(*py);
+        *py = __float_as_uint(__fadd_rn(__fmul_rn(__fsub_rn(1.0f, fraction), p), __fmul_rn(fraction, h)));
+    }
+    if (t < a.E && c < 7) eta[(size_t)t * 7 + c] = h;
 }
 
 __global__ void __launch_bounds__(256) k_init_tables(double *rcp, double *sqt, double2 *t2, int n) {
@@ -1727,6 +1824,16 @@ struct az_engine {
     uint64_t init0, init1;
     int initpl;
     bool have_init;
+    // az_set_root_noise / az_apply_root_noise / az_root_noise_values
+    bool noise_on;
+    bool noise_applied;  // the current roots were noised already
+    double noise_alpha;
+    float noise_fraction;
+    uint64_t noise_seed;
+    int64_t noise_slot_offset;
+    uint32_t noise_draws;  // applications since az_set_root_noise: the draw number of the next one
+    float *noise_eta;      // [E][7] η of the last application
+    int greedy_from;       // az_set_greedy_from: -1 = off
     int64_t bytes;
     int64_t launches;
     unsigned long long *d_tot;   // [16] stats totals (device)
@@ -1920,6 +2027,7 @@ int32_t az_create(const az_config *cfg, az_engine **out) {
     h->init1 = 0;
     h->initpl = 0;
     h->have_init = true;
+    h->greedy_from = -1;
     *out = h;
     return AZ_OK;
 }
@@ -2072,6 +2180,7 @@ int32_t az_reset_games(az_engine *h, uint64_t init_bb0, uint64_t init_bb1, int32
     h->n_active = E;
     h->step = 0;
     h->sims_done = 0;
+    h->noise_applied = false;
     h->sel_pending = false;
     return AZ_OK;
 }
@@ -2085,6 +2194,7 @@ int32_t az_set_roots(az_engine *h, const uint64_t *bb0, const uint64_t *bb1, con
     AZ_LAUNCH_CHECK(h, "k_set_roots");
     h->n_active = n;
     h->sims_done = 0;
+    h->noise_applied = false;
     h->sel_pending = false;
     return AZ_OK;
 }
@@ -2124,10 +2234,16 @@ int32_t az_run_move_step(az_engine *h, int32_t num_sims, int32_t eval_kind, cons
     if (!uniforms) return fail(h, AZ_E_INVALID, "%s", "az_run_move_step: null uniforms");
     if (!h->have_init) return fail(h, AZ_E_STATE, "%s", "az_run_move_step: call az_reset_games first");
     if (num_sims < 1) return fail(h, AZ_E_INVALID, "%s", "az_run_move_step: num_sims < 1");
+    if (h->greedy_from >= 0) {  // the greedy rule lives in k_sample_moves only: the search, then the move, as two launches
+        const int32_t rc = run_sims_impl(h, num_sims, eval_kind, nullptr, nullptr, false, stream);
+        if (rc != AZ_OK) return rc;
+        return az_sample_moves(h, uniforms, finished, stream);
+    }
     const int32_t rc = run_sims_impl(h, num_sims, eval_kind, uniforms, finished, true, stream);
     if (rc != AZ_OK) return rc;
     h->step++;
     h->sims_done = 0;
+    h->noise_applied = false;
     return AZ_OK;
 }
 
@@ -2404,11 +2520,77 @@ int32_t az_sample_moves(az_engine *h, const double *uniforms, uint8_t *finished,
     if (!h->have_init) return fail(h, AZ_E_STATE, "%s", "az_sample_moves: call az_reset_games first");
     if (int rc = set_device(h)) return rc;
     const int n = h->n_active;
-    k_sample_moves<<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0, h->init1,
-                                                             h->initpl);
+    if (h->greedy_from >= 0)
+        k_sample_moves<true><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0, h->init1,
+                                                                       h->initpl, h->greedy_from);
+    else
+        k_sample_moves<false><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0, h->init1,
+                                                                        h->initpl, -1);
     AZ_LAUNCH_CHECK(h, "k_sample_moves");
     h->step++;
     h->sims_done = 0;
+    h->noise_applied = false;
+    return AZ_OK;
+}
+
+int32_t az_set_root_noise(az_engine *h, const az_root_noise *cfg) {
+    if (!h) return AZ_E_INVALID;
+    if (!cfg) {
+        h->noise_on = false;
+        return AZ_OK;
+    }
+    if (!(cfg->alpha > 0.0 && cfg->alpha <= 1e6))
+        return fail(h, AZ_E_INVALID, "%s", "az_set_root_noise: alpha must be in (0, 1e6]");
+    if (!(cfg->fraction >= 0.0f && cfg->fraction <= 1.0f))
+        return fail(h, AZ_E_INVALID, "%s", "az_set_root_noise: fraction must be in [0, 1]");
+    if (cfg->slot_offset < 0 || cfg->slot_offset > ((int64_t)1 << 62))
+        return fail(h, AZ_E_INVALID, "%s", "az_set_root_noise: slot_offset must be in [0, 2^62]");
+    if (int rc = set_device(h)) return rc;
+    if (!h->noise_eta) {
+        if (int rc = dev_alloc(h, &h->noise_eta, (size_t)h->a.E * 7)) return rc;
+        AZ_CUDA(h, cudaMemset(h->noise_eta, 0, (size_t)h->a.E * 7 * sizeof(float)));
+    }
+    h->noise_on = true;
+    h->noise_alpha = cfg->alpha;
+    h->noise_fraction = cfg->fraction;
+    h->noise_seed = cfg->seed;
+    h->noise_slot_offset = cfg->slot_offset;
+    h->noise_draws = 0;
+    return AZ_OK;
+}
+
+int32_t az_apply_root_noise(az_engine *h, void *stream) {
+    if (!h) return AZ_E_INVALID;
+    if (!h->noise_on) return fail(h, AZ_E_STATE, "%s", "az_apply_root_noise: no noise configured (az_set_root_noise)");
+    if (h->sims_done != 1 || h->sel_pending || h->noise_applied)
+        return fail(h, AZ_E_STATE, "%s", "az_apply_root_noise: valid once, after exactly one complete simulation on the current roots");
+    if (int rc = set_device(h)) return rc;
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    AZ_CUDA(h, cudaStreamIsCapturing(S(stream), &cap));
+    if (cap != cudaStreamCaptureStatusNone)
+        return fail(h, AZ_E_STATE, "%s", "az_apply_root_noise: not inside a CUDA graph capture (the draw number is a launch argument)");
+    const int E = h->a.E;
+    k_root_noise<<<blocks_for((long long)E * 8, 256), 256, 0, S(stream)>>>(h->a, h->n_active, h->noise_alpha, h->noise_fraction,
+                                                                          h->noise_seed, h->noise_slot_offset, h->noise_draws,
+                                                                          h->noise_eta);
+    AZ_LAUNCH_CHECK(h, "k_root_noise");
+    h->noise_draws++;
+    h->noise_applied = true;
+    return AZ_OK;
+}
+
+int32_t az_root_noise_values(az_engine *h, float *eta, void *stream) {
+    if (!h) return AZ_E_INVALID;
+    if (!eta) return fail(h, AZ_E_INVALID, "%s", "az_root_noise_values: null output");
+    if (!h->noise_eta) return fail(h, AZ_E_STATE, "%s", "az_root_noise_values: no noise configured (az_set_root_noise)");
+    if (int rc = set_device(h)) return rc;
+    AZ_CUDA(h, cudaMemcpyAsync(eta, h->noise_eta, (size_t)h->a.E * 7 * sizeof(float), cudaMemcpyDeviceToDevice, S(stream)));
+    return AZ_OK;
+}
+
+int32_t az_set_greedy_from(az_engine *h, int32_t plies) {
+    if (!h) return AZ_E_INVALID;
+    h->greedy_from = plies < 0 ? -1 : plies;
     return AZ_OK;
 }
 

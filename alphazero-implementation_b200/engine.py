@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import AzConfig, AzEvalCacheStats, AzStats
+from ._lib import AzConfig, AzEvalCacheStats, AzRootNoise, AzStats
 
 EVAL_UNIFORM = 1
 EVAL_HASH = 2
@@ -95,6 +95,8 @@ class Engine:
         self.leaf_compaction = False
         self.leaf_compaction_fused = False
         self.eval_cache_log2 = 0
+        self.root_noise = None  # (alpha, fraction, seed, slot_offset) while noise is configured
+        self.greedy_from = -1
         self.tree_capacity = self.lib.az_tree_capacity(self.h)
 
     # -- plumbing --------------------------------------------------------------------------------
@@ -212,6 +214,35 @@ class Engine:
         st = AzEvalCacheStats()
         self._check(self.lib.az_get_eval_cache_stats(self.h, C.byref(st), _stream()), "az_get_eval_cache_stats")
         return {n: int(getattr(st, n)) for n, _ in AzEvalCacheStats._fields_}
+
+    def set_root_noise(self, alpha: float | None, fraction: float = 0.25, seed: int = 0, slot_offset: int = 0):
+        """Dirichlet noise on the root priors (`az_set_root_noise`); `alpha=None` turns it off.  Resets the draw counter: the
+        n-th `apply_root_noise` after this call draws the same eta for the same (seed, slot_offset + slot)."""
+        if alpha is None:
+            self._check(self.lib.az_set_root_noise(self.h, None), "az_set_root_noise")
+            self.root_noise = None
+            return
+        cfg = AzRootNoise(float(alpha), float(fraction), int(seed) & (2**64 - 1), int(slot_offset))
+        self._check(self.lib.az_set_root_noise(self.h, C.byref(cfg)), "az_set_root_noise")
+        self.root_noise = (float(alpha), float(fraction), int(seed), int(slot_offset))
+
+    def apply_root_noise(self):
+        """Mix fresh noise into the root priors of every active tree: exactly once per search, after its first simulation."""
+        self._check(self.lib.az_apply_root_noise(self.h, _stream()), "az_apply_root_noise")
+
+    def root_noise_values(self, out: torch.Tensor | None = None) -> torch.Tensor:
+        """eta [num_games, 7] f32 of the last `apply_root_noise` (0 on illegal columns and for the trees it skipped)."""
+        if out is None:
+            out = self.empty((self.num_games, 7), torch.float32)
+        self._check(self.lib.az_root_noise_values(self.h, _ptr(out), _stream()), "az_root_noise_values")
+        return out
+
+    def set_greedy_from(self, plies: int | None):
+        """From ply `plies` of every game on, the move step plays the most visited root child (lowest column on ties) instead of
+        sampling; None or negative = off."""
+        plies = -1 if plies is None or plies < 0 else int(plies)
+        self._check(self.lib.az_set_greedy_from(self.h, plies), "az_set_greedy_from")
+        self.greedy_from = plies
 
     def run_simulations(self, num_sims: int, eval_kind: int):
         self._check(self.lib.az_run_simulations(self.h, int(num_sims), int(eval_kind), _stream()), "az_run_simulations")

@@ -21,7 +21,13 @@ from .search import AlphaZeroSearch
 
 class EpisodeGenerator:
     def __init__(self, *, model, num_simulations: int, num_episodes: int, game_initial_state: State,
-                 exploration_weight: float = 1.0, uniform_source: Callable[[int, int], np.ndarray] | None = None, **search_kwargs):
+                 exploration_weight: float = 1.0, uniform_source: Callable[[int, int], np.ndarray] | None = None,
+                 sampling_moves: int | None = None, **search_kwargs):
+        """`sampling_moves` = n: the first n plies of every game are sampled from the visit counts as in the reference, later
+        ones play the most visited move (lowest column on ties; `num_sampling_moves` of DeepMind's AlphaZero pseudocode).  The
+        uniform of every (step, slot) is still drawn, so NumPy's global stream advances exactly as without it.  None = off.
+        Root noise comes through `search_kwargs` (`root_noise=RootNoise(...)`)."""
+        self.sampling_moves = sampling_moves
         self.search = AlphaZeroSearch(model=model, num_simulations=num_simulations, exploration_weight=exploration_weight,
                                       **search_kwargs)
         self.num_episodes = int(num_episodes)
@@ -51,6 +57,7 @@ class EpisodeGenerator:
             initial_state = self.game_initial_state
         E = self.num_episodes
         eng = self.search.engine_for(E, exact=True)  # the slots are the games: an engine grown by a larger run_simulations call is replaced
+        eng.set_greedy_from(self.sampling_moves)
         if reset:
             eng.reset_games(initial_state.bb0, initial_state.bb1, initial_state.player)
         elif eng.n_active != E:

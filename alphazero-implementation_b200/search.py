@@ -11,6 +11,7 @@ children with their statistics (what `improved_policy`, `value` and `select_next
 from __future__ import annotations
 
 import os
+from dataclasses import dataclass
 
 import numpy as np
 import torch
@@ -75,6 +76,20 @@ class Node:
     @property
     def is_root(self) -> bool:
         return self.parent is None
+
+
+@dataclass(frozen=True)
+class RootNoise:
+    """Dirichlet noise on the root priors of every search (`add_exploration_noise` of DeepMind's AlphaZero pseudocode):
+    after the first simulation has expanded the root, each root child's prior becomes (1 - fraction) * P + fraction * eta,
+    eta ~ Dirichlet(alpha) over the legal columns (`Engine.set_root_noise`).  Draws are a function of (seed, slot_offset + slot,
+    search number, column) only: `slot_offset` is the global index of the engine's first game, so sharded self-play draws what
+    the unsharded run draws.  Off (None) by default: then the search is the reference's, bit for bit."""
+
+    alpha: float = 1.0
+    fraction: float = 0.25
+    seed: int = 0
+    slot_offset: int = 0
 
 
 class _GraphedStep:
@@ -183,12 +198,16 @@ class _GraphedStep:
 class AlphaZeroSearch:
     def __init__(self, *, model, num_simulations: int, exploration_weight: float = 1.0, device: int | None = None,
                  lanes_per_tree: int = 0, inference_dtype: torch.dtype | None = None, use_cuda_graph: bool = True,
-                 use_tensor_core_kernels: bool = True, trunk_variant: int | None = None, eval_cache: bool | int = True):
+                 use_tensor_core_kernels: bool = True, trunk_variant: int | None = None, eval_cache: bool | int = True,
+                 root_noise: RootNoise | None = None):
         """`eval_cache`: serve repeated leaf positions from the engine's evaluation cache (`Engine.set_eval_cache`) when the
         evaluator's outputs depend on the position alone (`InferenceNet.position_only_outputs`); same results, fewer evaluator rows.
-        True = a table sized for the engine, False = off, an int = log2 of its entry count."""
+        True = a table sized for the engine, False = off, an int = log2 of its entry count.
+        `root_noise`: every search runs one simulation, mixes Dirichlet noise into the root priors (`RootNoise`), then runs the
+        other num_simulations - 1; None (default) = no noise."""
         self.inference_model = model.get_inference_clone()
         self.eval_cache = eval_cache
+        self.root_noise = root_noise
         self.num_simulations = int(num_simulations)
         self.exploration_weight = exploration_weight
         self.device_index = device
@@ -248,17 +267,35 @@ class AlphaZeroSearch:
             return self._net.kernel_name
         return "user predict()"
 
+    def _search_runs(self, S: int) -> list[int]:
+        """A search of S simulations as runs of consecutive simulations: with root noise, one simulation, the noise, the rest."""
+        return [1, S - 1] if self.root_noise is not None and S > 0 else [S]
+
     def launches_per_move_step(self) -> int:
         """Kernels of libaz_engine.so per self-play move step (`simulate_and_move`)."""
-        if self._mode == "builtin":
-            return 1
-        # k_select; S - 1 x (evaluator or gather, k_expand_select); evaluator, k_expand_backup; k_sample_moves - plus, when the
-        # evaluator walks the compacted leaf list, one k_compact_leaves after k_select (the later lists come out of k_expand_select)
-        # or, AZ_COMPACT_FUSED=0, one per selection
         S = self.num_simulations
+        runs = [n for n in self._search_runs(S) if n > 0]
+        noise = 1 if self.root_noise is not None else 0
+        greedy = self._engine is not None and self._engine.greedy_from >= 0
+        if self._mode == "builtin":
+            # one k_run_sims per run, the last one with the move fused in - unless the greedy cutoff (or a search of one simulation
+            # with noise) leaves the move to k_sample_moves
+            return len(runs) + noise + (1 if greedy or noise and S == 1 else 0)
+        # per run of n: k_select; n - 1 x (evaluator or gather, k_expand_select); evaluator, k_expand_backup.  Then k_root_noise
+        # between the runs and k_sample_moves.  When the evaluator walks the compacted leaf list: one k_compact_leaves after
+        # every k_select (the later lists come out of k_expand_select) or, AZ_COMPACT_FUSED=0, one per selection
+        n = sum(2 * r + 1 for r in runs) + noise + 1
         if not getattr(self._net, "wants_leaf_compaction", False):
-            return 2 * S + 2
-        return 2 * S + 2 + (1 if os.environ.get("AZ_COMPACT_FUSED", "1") != "0" else S)
+            return n
+        return n + (len(runs) if os.environ.get("AZ_COMPACT_FUSED", "1") != "0" else S)
+
+    def _configure_noise(self, engine: Engine):
+        rn = self.root_noise
+        if rn is None:
+            if engine.root_noise is not None:
+                engine.set_root_noise(None)
+        elif engine.root_noise != (float(rn.alpha), float(rn.fraction), int(rn.seed), int(rn.slot_offset)):
+            engine.set_root_noise(rn.alpha, rn.fraction, rn.seed, rn.slot_offset)
 
     def close(self):
         if self._engine is not None:
@@ -279,9 +316,20 @@ class AlphaZeroSearch:
         return self._engine
 
     def simulate(self, engine: Engine, num_simulations: int | None = None, evaluator_events: list | None = None):
-        """`num_simulations` simulations on every active tree of `engine` (roots already set).  `evaluator_events` (network
-        evaluators only): run the steps un-graphed and collect a CUDA-event pair around every evaluator call."""
+        """`num_simulations` simulations on every active tree of `engine` (fresh roots already set); with `root_noise`, the noise
+        is mixed into the root priors after the first.  `evaluator_events` (network evaluators only): run the steps un-graphed and
+        collect a CUDA-event pair around every evaluator call."""
         S = self.num_simulations if num_simulations is None else num_simulations
+        self._configure_noise(engine)
+        runs = self._search_runs(S)
+        for i, n in enumerate(runs):
+            if i:
+                engine.apply_root_noise()
+            self._simulate_run(engine, n, evaluator_events)
+
+    def _simulate_run(self, engine: Engine, S: int, evaluator_events: list | None):
+        if S <= 0:
+            return
         if self._mode == "builtin":
             engine.run_simulations(S, self.inference_model.az_builtin_eval_kind)
         elif self._mode == "net":
@@ -295,7 +343,16 @@ class AlphaZeroSearch:
         """One self-play move step: `simulate` then `Engine.sample_moves(uniforms)`.  With a built-in evaluator both run in
         one launch (`az_run_move_step`), with identical results."""
         if self._mode == "builtin":
-            engine.run_move_step(self.num_simulations, self.inference_model.az_builtin_eval_kind, uniforms, finished)
+            kind = self.inference_model.az_builtin_eval_kind
+            self._configure_noise(engine)
+            *head, last = self._search_runs(self.num_simulations)
+            for n in head:
+                engine.run_simulations(n, kind)
+                engine.apply_root_noise()
+            if last > 0:
+                engine.run_move_step(last, kind, uniforms, finished)
+            else:
+                engine.sample_moves(uniforms, finished)
         else:
             self.simulate(engine)
             engine.sample_moves(uniforms, finished)

@@ -8,6 +8,7 @@ iteration k+1 runs on a background thread — here with its own CUDA stream — 
 """
 from __future__ import annotations
 
+import dataclasses
 import time
 
 import torch
@@ -131,7 +132,8 @@ class Trainer:
     def train(self, *, num_iterations: int, episodes_per_iter: int, simulations_per_episode: int, epochs_per_iter: int,
               initial_state, buffer_size: int, save_every_n_iterations: int = 0, batch_size: int = 32, seed: int = 0,
               overlap: bool = True, inference_dtype: torch.dtype | None = None, precision: str = "32-true",
-              cuda_graph: bool = True, trainer_share: float | None = None, save_dir: str | None = None):
+              cuda_graph: bool = True, trainer_share: float | None = None, save_dir: str | None = None, root_noise=None,
+              sampling_moves: int | None = None):
         """`overlap=True` reproduces the reference's pipeline (datamodule.py:89-101): the self-play of iteration k+1 runs on a
         background thread (own CUDA stream, weights as of the end of iteration k-1's training) while iteration k trains.
         `precision`: "32-true" (the reference's Lightning default) or "bf16-mixed" (forward / backward under bf16 autocast,
@@ -141,7 +143,10 @@ class Trainer:
         writes the replay deque as `<save_dir>/episodes_iter{N}.json` (`DataModule._save_episodes`, datamodule.py:71-80,109-112;
         default directory "episodes", datamodule.py:63) and, after that iteration's training, a Lightning-shaped checkpoint
         `<save_dir>/model_iter{N}.ckpt` (`{"state_dict", "hyper_parameters", "epoch", "global_step"}`, the reference's
-        `ModelCheckpoint(every_n_epochs=...)`, trainer.py:66-70; read back with `Model.load_from_checkpoint`, scripts/play.py:19)."""
+        `ModelCheckpoint(every_n_epochs=...)`, trainer.py:66-70; read back with `Model.load_from_checkpoint`, scripts/play.py:19).
+        `root_noise` (`search.RootNoise`) and `sampling_moves` (`EpisodeGenerator`): AlphaZero's self-play exploration, off by
+        default.  Each rank's noise is keyed by the global index of its games (`slot_offset` = the first slot of its shard), so
+        the draws do not depend on how the games are sharded."""
         import threading
 
         world = dist.get_world_size() if dist.is_initialized() else 1
@@ -155,8 +160,10 @@ class Trainer:
         lo, hi = shards[rank]
         model = self.model.to(self.device)
         kw = {} if inference_dtype is None else dict(inference_dtype=inference_dtype)
+        if root_noise is not None:
+            kw["root_noise"] = dataclasses.replace(root_noise, slot_offset=lo)
         gen = EpisodeGenerator(model=model, num_simulations=simulations_per_episode, num_episodes=hi - lo,
-                               game_initial_state=initial_state, device=self.device_index, **kw)
+                               game_initial_state=initial_state, device=self.device_index, sampling_moves=sampling_moves, **kw)
         replay = ReplayBuffer(buffer_size, simulations_per_episode, self.device)
         opt = model.configure_optimizers()
         for group in opt.param_groups:  # Adam's step counter on the device, so that optimiser steps can be captured

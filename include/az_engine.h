@@ -225,6 +225,36 @@ int32_t az_sample_moves(az_engine *h, const double *uniforms /*[E]*/, uint8_t *f
  * The root's child statistics never leave the registers and the discarded tree is not written back. */
 int32_t az_run_move_step(az_engine *h, int32_t num_sims, int32_t evaluator_kind, const double *uniforms /*[E]*/, uint8_t *finished,
                          void *stream);
+/* ---- self-play exploration (absent from the reference, which ships DeepMind's pseudocode for them only; both off by default,
+ * and with both off every result is the reference's) ---- */
+/* Dirichlet noise on the root priors: add_exploration_noise of deepmind_alphazero_pseudocode.py.  A search on fresh roots runs
+ * one simulation (which expands a non-terminal root), then az_apply_root_noise, then the remaining S - 1 simulations.  For
+ * every active tree whose root has children it draws eta ~ Dirichlet(alpha, ..., alpha) over the k legal columns (ascending;
+ * 0 on illegal columns; k = 1 gives 1) and rewrites each root child's prior in place, in fp32 with one rounding per operation:
+ *   P' = RN(RN(RN(1 - fraction) * P) + RN(fraction * eta)).
+ * eta is a pure function of (seed, slot_offset + slot, number of applications since az_set_root_noise, column): a run is
+ * reproduced from its seed, and an engine over slots [lo, hi) with slot_offset = lo draws the rows [lo, hi) of an engine over
+ * all slots.  (Philox4x32-10 counters, Marsaglia-Tsang Gamma variates, log space for alpha < 1: see k_root_noise.)
+ * az_set_root_noise: alpha in (0, 1e6], fraction in [0, 1], slot_offset >= 0, else AZ_E_INVALID; NULL = off.  Resets the
+ * application counter. */
+typedef struct az_root_noise {
+    double alpha;        /* Dirichlet concentration (pseudocode: root_dirichlet_alpha) */
+    float fraction;      /* weight of the noise (pseudocode: root_exploration_fraction) */
+    uint64_t seed;
+    int64_t slot_offset; /* global index of this engine's slot 0 */
+} az_root_noise;
+int32_t az_set_root_noise(az_engine *h, const az_root_noise *cfg);
+/* the mixing, once per search: valid only after exactly one complete simulation on the current roots (AZ_E_STATE otherwise,
+ * and inside a CUDA graph capture).  One k_root_noise launch; increments the application counter. */
+int32_t az_apply_root_noise(az_engine *h, void *stream);
+/* eta[num_games][7] (device) of the last application (0 for trees it skipped: inactive, in error or without children) */
+int32_t az_root_noise_values(az_engine *h, float *eta, void *stream);
+/* Temperature cutoff: select_action of deepmind_alphazero_pseudocode.py with num_sampling_moves = plies.  From ply `plies` of a
+ * game on, az_sample_moves / az_run_move_step play the most visited root child (the lowest column on ties) instead of sampling
+ * node.py:31-35; the uniform of the slot is still an argument and the sample is recorded as before.  Negative = off (default).
+ * With the cutoff on, az_run_move_step runs as az_run_simulations + az_sample_moves (two launches, same results). */
+int32_t az_set_greedy_from(az_engine *h, int32_t plies);
+
 /* number of finished episodes / samples waiting in the ring.  Synchronises on `stream`. */
 int32_t az_episode_counts(az_engine *h, int64_t *n_episodes_host, int64_t *n_samples_host, void *stream);
 /* copy the ring out (device buffers sized from az_episode_counts) and empty it.  Episodes appear in
