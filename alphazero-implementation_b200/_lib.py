@@ -164,6 +164,9 @@ SIGNATURES = {
     "az_apply_root_noise": (I32, [P, P]),
     "az_root_noise_values": (I32, [P, P, P]),
     "az_set_greedy_from": (I32, [P, I32]),
+    "az_set_symmetric_eval": (I32, [P, I32]),
+    "az_leaf_mirror": (I32, [P, C.POINTER(P)]),
+    "az_mirror_states": (I32, [P, P, P, P, I64, P, P, P]),
     "az_trunk_weight_bytes": (I64, [I32]),
     "az_resnet_pipe_weight_bytes": (I64, [I32, I32]),
     "az_trunk_forward_leaves": (I32, [P, P, P, I32, P, P]),

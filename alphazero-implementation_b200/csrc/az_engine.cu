@@ -900,8 +900,12 @@ __device__ __forceinline__ void cache_publish(const Arena &a, uint32_t claim, in
 // ------------------------------------------------------------------------------------------------
 // split path, step 1: search.py:69-79
 // CACHE: non-terminal leaves are probed in the evaluation cache; launch / epoch from load_cache_ctl
-template <int TPW, bool LAT, bool CACHE>
-__device__ __forceinline__ bool select_body(const Arena &a, int n_active, double c_puct, uint32_t launch, uint32_t epoch) {
+// SYM: a non-terminal leaf is written (and probed) in its canonical form, leaf_mirror[t] = 1 when that is its mirror (the array
+// is a trailing kernel argument rather than an Arena member, so that the other kernels' parameter layout stays as it was); every
+// evaluator then evaluates the canonical position, so the search runs with f_sym(x) = unmirror_if_flagged(f(canon(x)))
+template <int TPW, bool LAT, bool CACHE, bool SYM>
+__device__ __forceinline__ bool select_body(const Arena &a, int n_active, double c_puct, uint32_t launch, uint32_t epoch,
+                                            uint8_t *leaf_mirror) {
     constexpr int TREES = 2 * TPW;
     constexpr int NL = 32 / TPW;
     const int lane = threadIdx.x & 31;
@@ -926,7 +930,10 @@ __device__ __forceinline__ bool select_body(const Arena &a, int n_active, double
     const uint4 rm = tm.gM[0];
     const bool alive = in_range && err == 0;
     const int lit = lane & (NL - 1);
-    if (in_range && !alive && lit == 0) a.leaf_status[t] = AZ_LEAF_IDLE;
+    if (in_range && !alive && lit == 0) {
+        a.leaf_status[t] = AZ_LEAF_IDLE;
+        if (SYM) leaf_mirror[t] = 0;
+    }
     if (!__any_sync(FULL, alive)) return false;
     const bool writer = alive && lit == 0;
     uint32_t *path = a.path + (size_t)tt * PATH_STRIDE;
@@ -945,10 +952,18 @@ __device__ __forceinline__ bool select_body(const Arena &a, int n_active, double
     uint8_t status = L.term ? AZ_LEAF_TERMINAL : AZ_LEAF_EVAL;
     if (writer) {
         uint32_t *st = a.tstats + (size_t)t * NSTAT;
-        if (CACHE && !L.term) status = cache_probe(a, t, L.b0, L.b1, L.pl, launch, epoch, st);
+        uint64_t lb0 = L.b0, lb1 = L.b1;
+        if (SYM) {
+            const c4::Canonical k = c4::canonical(L.b0, L.b1);
+            const bool mir = k.mirrored && !L.term;
+            lb0 = mir ? k.b0 : L.b0;
+            lb1 = mir ? k.b1 : L.b1;
+            leaf_mirror[t] = mir ? 1 : 0;
+        }
+        if (CACHE && !L.term) status = cache_probe(a, t, lb0, lb1, L.pl, launch, epoch, st);
         a.leaf_node[t] = L.node;
-        a.leaf_bb0[t] = L.b0;
-        a.leaf_bb1[t] = L.b1;
+        a.leaf_bb0[t] = lb0;
+        a.leaf_bb1[t] = lb1;
         a.leaf_player[t] = (uint8_t)L.pl;
         a.leaf_depth[t] = (uint8_t)L.depth;
         a.leaf_status[t] = status;
@@ -962,18 +977,21 @@ __device__ __forceinline__ bool select_body(const Arena &a, int n_active, double
 }
 
 // split path, step 3: search.py:87-91 with the evaluator's outputs
-template <int TPW, bool LAT, bool CACHE>
-__global__ void __launch_bounds__(64) k_select(Arena a, int n_active, double c_puct) {
+template <int TPW, bool LAT, bool CACHE, bool SYM>
+__global__ void __launch_bounds__(64) k_select(Arena a, int n_active, double c_puct, uint8_t *leaf_mirror) {
     uint32_t launch = 0, epoch = 0;
     if (CACHE) load_cache_ctl(a, launch, epoch);
-    select_body<TPW, LAT, CACHE>(a, n_active, c_puct, launch, epoch);
+    select_body<TPW, LAT, CACHE, SYM>(a, n_active, c_puct, launch, epoch, leaf_mirror);
 }
 
 // split path, step 3: search.py:87-91 with the evaluator's outputs
 // CACHE: a SERVED leaf takes its outputs from cached_out or from its leader's row, and a leaf that claimed an entry publishes its row
-template <int TPW, bool CACHE>
+// SYM: lane c works on column c of the canonical leaf the evaluator saw (legal mask, logit, softmax, published row); for a mirrored
+// leaf that is actual column 6 - c, whose index among the actual children (ascending columns) is k - 1 - j instead of j
+template <int TPW, bool CACHE, bool SYM>
 __device__ __forceinline__ void expand_backup_body(const Arena &a, int n_active, const float *__restrict__ policy,
-                                                   const float *__restrict__ values, int policy_kind, uint32_t launch) {
+                                                   const float *__restrict__ values, int policy_kind, uint32_t launch,
+                                                   const uint8_t *leaf_mirror) {
     constexpr int TREES = 2 * TPW;
     constexpr int NL = 32 / TPW;
     const int lane = threadIdx.x & 31;
@@ -998,6 +1016,7 @@ __device__ __forceinline__ void expand_backup_body(const Arena &a, int n_active,
     float v0 = values[(size_t)tt * 2], v1 = values[(size_t)tt * 2 + 1];
     const uint32_t src = CACHE ? a.leaf_src[tt] : 0u;
     const uint32_t claim = CACHE ? a.leaf_claim[tt] : NO_CLAIM;
+    const bool mir = SYM && leaf_mirror[tt] != 0;
     const bool served = CACHE && status == AZ_LEAF_SERVED;
     const bool alive = (t < n_active) && (status == AZ_LEAF_EVAL || served);
     if (!__any_sync(FULL, alive)) return;
@@ -1046,7 +1065,7 @@ __device__ __forceinline__ void expand_backup_body(const Arena &a, int n_active,
     }
     __syncwarp();  // every lane has read used / leaf_* before the writer updates them
     if (alive) {
-        if (can && first_q) store_new_child(tm, used + j, prior);
+        if (can && first_q) store_new_child(tm, used + (mir ? k - 1 - j : j), prior);
         const double v = (double)(pl ? v1 : v0);  // value[node.state.player] (search.py:91)
         if (writer) {
             set_first_child(tm, node, used);
@@ -1074,12 +1093,13 @@ __device__ __forceinline__ void expand_backup_body(const Arena &a, int n_active,
     }
 }
 
-template <int TPW, bool CACHE>
+template <int TPW, bool CACHE, bool SYM>
 __global__ void __launch_bounds__(64)
-k_expand_backup(Arena a, int n_active, const float *__restrict__ policy, const float *__restrict__ values, int policy_kind) {
+k_expand_backup(Arena a, int n_active, const float *__restrict__ policy, const float *__restrict__ values, int policy_kind,
+                const uint8_t *leaf_mirror) {
     uint32_t launch = 0, epoch = 0;
     if (CACHE) load_cache_ctl(a, launch, epoch);
-    expand_backup_body<TPW, CACHE>(a, n_active, policy, values, policy_kind, launch);
+    expand_backup_body<TPW, CACHE, SYM>(a, n_active, policy, values, policy_kind, launch, leaf_mirror);
 }
 
 // Steps 3 and 1 of consecutive simulations in one launch: expansion + backup of simulation k, then the selection of simulation
@@ -1093,14 +1113,15 @@ k_expand_backup(Arena a, int n_active, const float *__restrict__ policy, const f
 // outputs to the slots' rows and a position's outputs do not depend on the batch it falls into, so the search is unchanged.
 // CACHE: both halves use the evaluation cache; with COMPACT the last warp also advances the launch number (the ticket atomic is then
 // acq_rel, so that every warp's read of the number at its start precedes the advance).
-template <int TPW, bool LAT, bool COMPACT, bool CACHE>
+template <int TPW, bool LAT, bool COMPACT, bool CACHE, bool SYM>
 __global__ void __launch_bounds__(64)
-k_expand_select(Arena a, int n_active, const float *__restrict__ policy, const float *__restrict__ values, int policy_kind, double c_puct) {
+k_expand_select(Arena a, int n_active, const float *__restrict__ policy, const float *__restrict__ values, int policy_kind, double c_puct,
+                uint8_t *leaf_mirror) {
     uint32_t launch = 0, epoch = 0;
     if (CACHE) load_cache_ctl(a, launch, epoch);
-    expand_backup_body<TPW, CACHE>(a, n_active, policy, values, policy_kind, launch);
+    expand_backup_body<TPW, CACHE, SYM>(a, n_active, policy, values, policy_kind, launch, leaf_mirror);
     __syncwarp();
-    const bool wants = select_body<TPW, LAT, CACHE>(a, n_active, c_puct, launch, epoch);
+    const bool wants = select_body<TPW, LAT, CACHE, SYM>(a, n_active, c_puct, launch, epoch, leaf_mirror);
     if (COMPACT) {
         const int lane = threadIdx.x & 31;
         const unsigned m = __ballot_sync(FULL, wants);
@@ -1402,6 +1423,40 @@ k_state_info(const uint64_t *__restrict__ bb0, const uint64_t *__restrict__ bb1,
         oreward[2 * i] = T.reward0;
         oreward[2 * i + 1] = (int8_t)-T.reward0;
     }
+}
+
+// Left-right mirror of n positions (c4::mirror of both bitboards); flags (may be null = every row): only rows with a non-zero flag
+// are mirrored, the others are copied.  Four positions per thread with 16-byte loads / stores of the bitboards and one 32-bit load
+// of the flags when `vec` (every pointer 16-byte aligned), else one position per thread.  Each thread reads its positions before it
+// writes them, so the output may be the input.
+__global__ void __launch_bounds__(256)
+k_mirror_states(const uint64_t *bb0, const uint64_t *bb1, const uint8_t *flags, long long n, uint64_t *o0, uint64_t *o1, int vec) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (vec) {
+        if (4 * i + 3 >= n) return;
+        const uint4 *v0 = reinterpret_cast<const uint4 *>(bb0) + 2 * i, *v1 = reinterpret_cast<const uint4 *>(bb1) + 2 * i;
+        const uint4 a0 = v0[0], a1 = v0[1], c0 = v1[0], c1 = v1[1];
+        const uint32_t fw = flags ? reinterpret_cast<const uint32_t *>(flags)[i] : 0x01010101u;
+        uint64_t x[4] = {(uint64_t)a0.y << 32 | a0.x, (uint64_t)a0.w << 32 | a0.z, (uint64_t)a1.y << 32 | a1.x, (uint64_t)a1.w << 32 | a1.z};
+        uint64_t y[4] = {(uint64_t)c0.y << 32 | c0.x, (uint64_t)c0.w << 32 | c0.z, (uint64_t)c1.y << 32 | c1.x, (uint64_t)c1.w << 32 | c1.z};
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const bool m = ((fw >> (8 * k)) & 0xFFu) != 0u;
+            x[k] = m ? c4::mirror(x[k]) : x[k];
+            y[k] = m ? c4::mirror(y[k]) : y[k];
+        }
+        uint4 *w0 = reinterpret_cast<uint4 *>(o0) + 2 * i, *w1 = reinterpret_cast<uint4 *>(o1) + 2 * i;
+        w0[0] = make_uint4((uint32_t)x[0], (uint32_t)(x[0] >> 32), (uint32_t)x[1], (uint32_t)(x[1] >> 32));
+        w0[1] = make_uint4((uint32_t)x[2], (uint32_t)(x[2] >> 32), (uint32_t)x[3], (uint32_t)(x[3] >> 32));
+        w1[0] = make_uint4((uint32_t)y[0], (uint32_t)(y[0] >> 32), (uint32_t)y[1], (uint32_t)(y[1] >> 32));
+        w1[1] = make_uint4((uint32_t)y[2], (uint32_t)(y[2] >> 32), (uint32_t)y[3], (uint32_t)(y[3] >> 32));
+        return;
+    }
+    if (i >= n) return;
+    const uint64_t b0 = bb0[i], b1 = bb1[i];
+    const bool m = !flags || flags[i] != 0;
+    o0[i] = m ? c4::mirror(b0) : b0;
+    o1[i] = m ? c4::mirror(b1) : b1;
 }
 
 // One row of the legal-only softmax (models/games/connect4/model.py:29-35), fp32; x[] in, priors out (0 on illegal columns).
@@ -1834,6 +1889,9 @@ struct az_engine {
     uint32_t noise_draws;  // applications since az_set_root_noise: the draw number of the next one
     float *noise_eta;      // [E][7] η of the last application
     int greedy_from;       // az_set_greedy_from: -1 = off
+    bool sym;              // az_set_symmetric_eval: selections write canonical leaves (the SYM kernels)
+    bool sym_sel;          // ... and the last selection did (leaf_mirror describes its leaves)
+    uint8_t *leaf_mirror;  // [E] 1 = the leaf arrays hold the mirror of the leaf the descent reached (allocated with the first az_set_symmetric_eval)
     int64_t bytes;
     int64_t launches;
     unsigned long long *d_tot;   // [16] stats totals (device)
@@ -2253,6 +2311,7 @@ static int32_t run_sims_impl(az_engine *h, int32_t num_sims, int32_t eval_kind, 
     if (h->sims_done + num_sims > h->cfg.num_simulations)
         return fail(h, AZ_E_INVALID, "%s", "az_run_simulations: more simulations on these roots than the arena holds (1 + 7*num_simulations nodes per tree)");
     if (eval_kind != AZ_EVAL_UNIFORM && eval_kind != AZ_EVAL_HASH) return fail(h, AZ_E_INVALID, "%s", "az_run_simulations: unknown evaluator");
+    if (h->sym) return fail(h, AZ_E_STATE, "%s", "az_run_simulations: the fused built-in path has no symmetric evaluation (az_set_symmetric_eval)");
     if (num_sims == 0) return AZ_OK;
     if (int rc = set_device(h)) return rc;
     const int n = h->n_active;
@@ -2339,20 +2398,27 @@ int32_t az_select_leaves(az_engine *h, void *stream) {
     const int tpb = 2 * (32 / h->G);
     const bool lat = latency_variant(h, blocks_for(n, tpb));
     const bool cache = cache_active(h);
-#define AZ_SEL(TPW_)                                                                                                  \
-    do {                                                                                                              \
-        if (cache) {                                                                                                  \
-            if (lat) k_select<TPW_, true, true><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct);    \
-            else k_select<TPW_, false, true><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct);       \
-        } else {                                                                                                      \
-            if (lat) k_select<TPW_, true, false><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct);   \
-            else k_select<TPW_, false, false><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct);      \
-        }                                                                                                             \
+    const bool sym = h->sym;
+#define AZ_SEL2(TPW_, SYM_)                                                                                                 \
+    do {                                                                                                                    \
+        if (cache) {                                                                                                        \
+            if (lat) k_select<TPW_, true, true, SYM_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror);    \
+            else k_select<TPW_, false, true, SYM_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror);       \
+        } else {                                                                                                            \
+            if (lat) k_select<TPW_, true, false, SYM_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror);   \
+            else k_select<TPW_, false, false, SYM_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror);      \
+        }                                                                                                                   \
+    } while (0)
+#define AZ_SEL(TPW_)                      \
+    do {                                  \
+        if (sym) AZ_SEL2(TPW_, true);     \
+        else AZ_SEL2(TPW_, false);        \
     } while (0)
     if (h->G == 32) AZ_SEL(1);
     else if (h->G == 16) AZ_SEL(2);
     else AZ_SEL(4);
 #undef AZ_SEL
+#undef AZ_SEL2
     AZ_LAUNCH_CHECK(h, "k_select");
     h->compact_valid = h->compact != 0;
     if (h->compact) {
@@ -2363,6 +2429,7 @@ int32_t az_select_leaves(az_engine *h, void *stream) {
     h->sims_done += 1;
     h->sel_pending = true;
     h->cache_sel = cache;
+    h->sym_sel = sym;
     return AZ_OK;
 }
 
@@ -2382,15 +2449,22 @@ int32_t az_expand_backup(az_engine *h, const float *policy, const float *values,
     if (int rc = set_device(h)) return rc;
     const int n = h->n_active;
     const bool cache = h->sel_pending && h->cache_sel;  // SERVED leaves and claims exist only after a cached selection
-#define AZ_EB(TPW_)                                                                                                   \
-    do {                                                                                                              \
-        if (cache) k_expand_backup<TPW_, true><<<blocks_for(n, 2 * TPW_), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind);  \
-        else k_expand_backup<TPW_, false><<<blocks_for(n, 2 * TPW_), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind);  \
+    const bool sym = h->sel_pending && h->sym_sel;      // mirrored leaves exist only after a symmetric selection
+#define AZ_EB2(TPW_, SYM_)                                                                                                          \
+    do {                                                                                                                            \
+        if (cache) k_expand_backup<TPW_, true, SYM_><<<blocks_for(n, 2 * TPW_), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->leaf_mirror);  \
+        else k_expand_backup<TPW_, false, SYM_><<<blocks_for(n, 2 * TPW_), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->leaf_mirror);  \
+    } while (0)
+#define AZ_EB(TPW_)                      \
+    do {                                 \
+        if (sym) AZ_EB2(TPW_, true);     \
+        else AZ_EB2(TPW_, false);        \
     } while (0)
     if (h->G == 32) AZ_EB(1);
     else if (h->G == 16) AZ_EB(2);
     else AZ_EB(4);
 #undef AZ_EB
+#undef AZ_EB2
     AZ_LAUNCH_CHECK(h, "k_expand_backup");
     h->compact_valid = false;  // the leaves are consumed
     h->sel_pending = false;
@@ -2413,10 +2487,16 @@ int32_t az_expand_backup_select(az_engine *h, const float *policy, const float *
     const bool cache = cache_active(h);
     if (h->sel_pending && h->cache_sel != cache)
         return fail(h, AZ_E_STATE, "%s", "az_expand_backup_select: the evaluation cache or leaf compaction changed between a selection and its expansion");
-#define AZ_ES2(TPW_, LAT_, CMP_)                                                                                                      \
+    const bool sym = h->sym;  // az_set_symmetric_eval refuses while a selection is pending: the expansion matches its selection
+#define AZ_ES3(TPW_, LAT_, CMP_, SYM_)                                                                                                      \
     do {                                                                                                                              \
-        if (cache) k_expand_select<TPW_, LAT_, CMP_, true><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct);  \
-        else k_expand_select<TPW_, LAT_, CMP_, false><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct);  \
+        if (cache) k_expand_select<TPW_, LAT_, CMP_, true, SYM_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct, h->leaf_mirror);  \
+        else k_expand_select<TPW_, LAT_, CMP_, false, SYM_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct, h->leaf_mirror);  \
+    } while (0)
+#define AZ_ES2(TPW_, LAT_, CMP_)                     \
+    do {                                             \
+        if (sym) AZ_ES3(TPW_, LAT_, CMP_, true);     \
+        else AZ_ES3(TPW_, LAT_, CMP_, false);        \
     } while (0)
 #define AZ_ES(TPW_)                               \
     do {                                          \
@@ -2433,6 +2513,7 @@ int32_t az_expand_backup_select(az_engine *h, const float *policy, const float *
     else AZ_ES(4);
 #undef AZ_ES
 #undef AZ_ES2
+#undef AZ_ES3
     AZ_LAUNCH_CHECK(h, "k_expand_select");
     h->compact_valid = h->compact != 0;
     if (h->compact == 1) {
@@ -2443,6 +2524,7 @@ int32_t az_expand_backup_select(az_engine *h, const float *policy, const float *
     h->sims_done += 1;
     h->sel_pending = true;
     h->cache_sel = cache;
+    h->sym_sel = sym;
     return AZ_OK;
 }
 
@@ -2773,6 +2855,46 @@ int32_t az_reset_stats(az_engine *h, void *stream) {
     k_zero_u32<<<148, 256, 0, S(stream)>>>(h->a.tstats, (long long)h->a.E * NSTAT);
     AZ_LAUNCH_CHECK(h, "k_zero_u32");
     memset(h->acc_tot, 0, sizeof h->acc_tot);
+    return AZ_OK;
+}
+
+int32_t az_set_symmetric_eval(az_engine *h, int32_t on) {
+    if (!h) return AZ_E_INVALID;
+    if (h->sel_pending) return fail(h, AZ_E_STATE, "%s", "az_set_symmetric_eval: a selection's leaves wait for their expansion");
+    if (on && !h->leaf_mirror) {
+        if (int rc = set_device(h)) return rc;
+        if (int rc = dev_alloc(h, &h->leaf_mirror, h->a.E)) return rc;
+        AZ_CUDA(h, cudaMemset(h->leaf_mirror, 0, (size_t)h->a.E));
+    }
+    h->sym = on != 0;
+    return AZ_OK;
+}
+
+int32_t az_leaf_mirror(az_engine *h, const uint8_t **mirrored) {
+    if (!h || !mirrored) return AZ_E_INVALID;
+    *mirrored = h->sym_sel ? h->leaf_mirror : nullptr;
+    return AZ_OK;
+}
+
+int32_t az_mirror_states(az_engine *h, const uint64_t *bb0, const uint64_t *bb1, const uint8_t *flags, int64_t n, uint64_t *out_bb0,
+                         uint64_t *out_bb1, void *stream) {
+    if (!h) return AZ_E_INVALID;
+    if (n < 0 || (n > 0 && (!bb0 || !bb1 || !out_bb0 || !out_bb1))) return fail(h, AZ_E_INVALID, "%s", "az_mirror_states: null argument");
+    if (n == 0) return AZ_OK;
+    if (int rc = set_device(h)) return rc;
+    const void *ptrs[] = {bb0, bb1, out_bb0, out_bb1};
+    bool vec = !flags || (reinterpret_cast<uintptr_t>(flags) & 3u) == 0;
+    for (const void *p : ptrs) vec = vec && (reinterpret_cast<uintptr_t>(p) & 15u) == 0;
+    const long long quads = vec ? n / 4 : 0, head = quads * 4;
+    if (quads) {
+        k_mirror_states<<<blocks_for(quads, 256), 256, 0, S(stream)>>>(bb0, bb1, flags, n, out_bb0, out_bb1, 1);
+        AZ_LAUNCH_CHECK(h, "k_mirror_states");
+    }
+    if (head < n) {
+        k_mirror_states<<<blocks_for(n - head, 256), 256, 0, S(stream)>>>(bb0 + head, bb1 + head, flags ? flags + head : nullptr, n - head,
+                                                                      out_bb0 + head, out_bb1 + head, 0);
+        AZ_LAUNCH_CHECK(h, "k_mirror_states");
+    }
     return AZ_OK;
 }
 

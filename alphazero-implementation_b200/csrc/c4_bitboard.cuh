@@ -73,6 +73,29 @@ C4_HD int nth_legal_column(uint32_t legal, int idx) {
     return col;
 }
 
+// Left-right mirror of one player's stones: column c's 7 bits (bit 7c + r) move to column 6 - c.  A position and its mirror
+// have the same value, and their policies are the same with the columns reversed; the side to move does not change.
+C4_HD uint64_t mirror(uint64_t b) {
+    constexpr uint64_t C0 = 0x7Full, C1 = C0 << 7, C2 = C0 << 14, C3 = C0 << 21;
+    return (b & C3) | ((b & C0) << 42) | ((b >> 42) & C0) | ((b & C1) << 28) | ((b >> 28) & C1) | ((b & C2) << 14) |
+           ((b >> 14) & C2);
+}
+
+// Canonical form of a position: the smaller of (b0, b1) and (mirror(b0), mirror(b1)) as unsigned 64-bit values, b0 first.
+// `mirrored` is set only when the mirror was taken; a palindrome (its own mirror) is its own canonical form.
+struct Canonical {
+    uint64_t b0, b1;
+    bool mirrored;
+};
+C4_HD Canonical canonical(uint64_t b0, uint64_t b1) {
+    const uint64_t m0 = mirror(b0), m1 = mirror(b1);
+    Canonical r;
+    r.mirrored = m0 < b0 || (m0 == b0 && m1 < b1);
+    r.b0 = r.mirrored ? m0 : b0;
+    r.b1 = r.mirrored ? m1 : b1;
+    return r;
+}
+
 // has_ended / reward of an arbitrary position (root states handed in by the caller):
 // winner = whoever owns a 4-in-line (player 0 tested first), else draw iff board full.
 struct Terminal {

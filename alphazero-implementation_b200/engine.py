@@ -97,6 +97,7 @@ class Engine:
         self.eval_cache_log2 = 0
         self.root_noise = None  # (alpha, fraction, seed, slot_offset) while noise is configured
         self.greedy_from = -1
+        self.symmetric_eval = False
         self.tree_capacity = self.lib.az_tree_capacity(self.h)
 
     # -- plumbing --------------------------------------------------------------------------------
@@ -155,6 +156,18 @@ class Engine:
         self._check(self.lib.az_state_info(self.h, _ptr(bb0), _ptr(bb1), None, n, _ptr(out["legal"]), _ptr(out["ended"]),
                                            _ptr(out["reward"]), _stream()), "az_state_info")
         return out
+
+    def mirror_states(self, bb0, bb1, flags=None, out: tuple[torch.Tensor, torch.Tensor] | None = None):
+        """Left-right mirror of the positions (`az_mirror_states`): column c goes to column 6 - c in both bitboards; with `flags`
+        (u8 per position) only the rows whose flag is non-zero, the others are copied.  `out` = (bb0, bb1) int64 device tensors,
+        which may be the inputs themselves.  -> (bb0, bb1)"""
+        bb0 = self._dev(bb0, torch.int64); bb1 = self._dev(bb1, torch.int64)
+        flags = None if flags is None else self._dev(flags, torch.uint8)
+        n = bb0.numel()
+        o0, o1 = out if out is not None else (self.empty(n, torch.int64), self.empty(n, torch.int64))
+        self._check(self.lib.az_mirror_states(self.h, _ptr(bb0), _ptr(bb1), _ptr(flags), n, _ptr(o0), _ptr(o1), _stream()),
+                    "az_mirror_states")
+        return o0, o1
 
     def masked_softmax(self, logits: torch.Tensor, legal) -> torch.Tensor:
         logits = self._dev(logits, torch.float32).reshape(-1, 7)
@@ -243,6 +256,27 @@ class Engine:
         plies = -1 if plies is None or plies < 0 else int(plies)
         self._check(self.lib.az_set_greedy_from(self.h, plies), "az_set_greedy_from")
         self.greedy_from = plies
+
+    def set_symmetric_eval(self, on: bool):
+        """Symmetric leaf evaluation (`az_set_symmetric_eval`): every non-terminal leaf is evaluated in its canonical orientation
+        (the smaller of it and its left-right mirror) and a mirrored leaf's priors are stored with the columns reversed.  Network and
+        `predict` evaluators only; call it before a CUDA graph of the search is captured."""
+        self._check(self.lib.az_set_symmetric_eval(self.h, 1 if on else 0), "az_set_symmetric_eval")
+        self.symmetric_eval = bool(on)
+
+    def leaf_mirror(self) -> torch.Tensor | None:
+        """u8 [num_games] view of the engine's flags: 1 where the last selection's leaf is the mirror of the position reached;
+        None when that selection ran with symmetric evaluation off."""
+        p = C.c_void_p()
+        self._check(self.lib.az_leaf_mirror(self.h, C.byref(p)), "az_leaf_mirror")
+        if not p.value:
+            return None
+
+        class _Raw:
+            def __init__(self, ptr, n):
+                self.__cuda_array_interface__ = dict(shape=(n,), typestr="|u1", data=(ptr, False), version=2)
+
+        return torch.as_tensor(_Raw(p.value, self.num_games), device=self.device)
 
     def run_simulations(self, num_sims: int, eval_kind: int):
         self._check(self.lib.az_run_simulations(self.h, int(num_sims), int(eval_kind), _stream()), "az_run_simulations")

@@ -48,6 +48,32 @@ def bitboards_to_grid(bb0: int, bb1: int) -> np.ndarray:
     return g
 
 
+_COL = np.uint64(0x7F)
+
+
+def _mirror(b: np.ndarray) -> np.ndarray:
+    out = b & (_COL << np.uint64(21))
+    for c in range(3):  # columns c and 6 - c trade places; column 3 stays
+        s, lo = np.uint64(7 * (6 - 2 * c)), _COL << np.uint64(7 * c)
+        out |= ((b & lo) << s) | ((b >> s) & lo)
+    return out
+
+
+def mirror_bitboards(bb0, bb1) -> tuple[np.ndarray, np.ndarray]:
+    """Left-right mirror of positions (what `az_mirror_states` computes on the device): column c's 7 bits (bit 7c + r) move to
+    column 6 - c, in both bitboards; the side to move does not change."""
+    return _mirror(np.asarray(bb0, np.uint64)), _mirror(np.asarray(bb1, np.uint64))
+
+
+def canonical_bitboards(bb0, bb1) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """Canonical form of positions under the mirror: the smaller of (bb0, bb1) and its mirror as unsigned 64-bit values, bb0
+    first -> (bb0, bb1, mirrored).  A palindrome (its own mirror) is its own canonical form and is not marked mirrored."""
+    b0, b1 = np.asarray(bb0, np.uint64), np.asarray(bb1, np.uint64)
+    m0, m1 = mirror_bitboards(b0, b1)
+    mirrored = (m0 < b0) | ((m0 == b0) & (m1 < b1))
+    return np.where(mirrored, m0, b0), np.where(mirrored, m1, b1), mirrored
+
+
 class Config:
     """`Config(6, 7, 4)` (scripts/train.py:12).  Only that configuration has kernels."""
 

@@ -50,7 +50,8 @@ class AlphaZeroPlayer(Player):
     """MCTS agent with the reference's constructor and temperature semantics (ui/cli/player.py:18-76).  The reference builds a new
     `AlphaZeroSearch` (a deep copy of the model) for every move; here the search - and its engine, packed weights and CUDA graph -
     is built once and kept.  (`agent.run` returns `(policy, value)`; the reference's `play` indexes that tuple as if it were the
-    policy, ui/cli/player.py:64 - the intended behaviour is implemented.)"""
+    policy, ui/cli/player.py:64 - the intended behaviour is implemented.)  `search_kwargs` go to `AlphaZeroSearch` (for example
+    `symmetric=True`), and an `Arena` plays through its agents' searches."""
 
     def __init__(self, model, *, mcts_simulation: int = 100, temperature: float = 1.0, **search_kwargs) -> None:
         self.model = model

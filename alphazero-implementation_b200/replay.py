@@ -114,14 +114,21 @@ class ReplayBuffer:
         n = ep_len.shape[0]
         return EpisodeBatch(np.full(n, -1, np.int32), np.zeros(n, np.int32), ep_len, off, outcome, bb0, bb1, pl, counts)
 
-    def batches(self, layout: int, batch_size: int = 32, shuffle: bool = True, generator: torch.Generator | None = None):
-        """Yield (x, policy_target, value_target) minibatches on the device (DataLoader(batch 32, shuffle), datamodule.py:124-130)."""
+    def batches(self, layout: int, batch_size: int = 32, shuffle: bool = True, generator: torch.Generator | None = None,
+                mirror: bool = False):
+        """Yield (x, policy_target, value_target) minibatches on the device (DataLoader(batch 32, shuffle), datamodule.py:124-130).
+        `mirror`: one Bernoulli(1/2) flag per sample, drawn after the permutation from `generator`; flagged samples come as their
+        left-right mirror image (bitboards through `az_mirror_states`, policy target columns reversed)."""
         bb0, bb1, pl, policy, value = self.tensors()
         n = bb0.numel()
         perm = torch.randperm(n, generator=generator).to(self.device) if shuffle else torch.arange(n, device=self.device)
         # one gather per epoch instead of five per minibatch: the shuffled set is materialised once, minibatches are views
         bb0, bb1, pl, policy, value = bb0[perm], bb1[perm], pl[perm], policy[perm], value[perm]
         eng = rules_engine()
+        if mirror:
+            flip = torch.randint(0, 2, (n,), generator=generator, dtype=torch.uint8).to(self.device)
+            bb0, bb1 = eng.mirror_states(bb0, bb1, flip, out=(bb0, bb1))
+            policy = torch.where(flip.bool().unsqueeze(1), policy.flip(1), policy)
         for i in range(0, n, batch_size):
             x = eng.encode_states(bb0[i:i + batch_size], bb1[i:i + batch_size], pl[i:i + batch_size], layout)
             yield x, policy[i:i + batch_size], value[i:i + batch_size]

@@ -199,12 +199,16 @@ class AlphaZeroSearch:
     def __init__(self, *, model, num_simulations: int, exploration_weight: float = 1.0, device: int | None = None,
                  lanes_per_tree: int = 0, inference_dtype: torch.dtype | None = None, use_cuda_graph: bool = True,
                  use_tensor_core_kernels: bool = True, trunk_variant: int | None = None, eval_cache: bool | int = True,
-                 root_noise: RootNoise | None = None):
+                 root_noise: RootNoise | None = None, symmetric: bool = False):
         """`eval_cache`: serve repeated leaf positions from the engine's evaluation cache (`Engine.set_eval_cache`) when the
         evaluator's outputs depend on the position alone (`InferenceNet.position_only_outputs`); same results, fewer evaluator rows.
         True = a table sized for the engine, False = off, an int = log2 of its entry count.
         `root_noise`: every search runs one simulation, mixes Dirichlet noise into the root priors (`RootNoise`), then runs the
-        other num_simulations - 1; None (default) = no noise."""
+        other num_simulations - 1; None (default) = no noise.
+        `symmetric`: evaluate every leaf in its canonical orientation under Connect4's left-right mirror (`Engine.set_symmetric_eval`):
+        a position and its mirror get the same value and mirrored priors, and share one evaluator row and one cache entry.  Network
+        and `predict` evaluators only (ValueError for the built-in ones); off (default) = the reference's search, bit for bit."""
+        self.symmetric = bool(symmetric)
         self.inference_model = model.get_inference_clone()
         self.eval_cache = eval_cache
         self.root_noise = root_noise
@@ -254,6 +258,9 @@ class AlphaZeroSearch:
             torch.cuda.current_stream(dev).synchronize()
         else:
             self._mode, self._net, self._graphed = "predict", None, None
+        if self.symmetric and self._mode == "builtin":
+            raise ValueError("symmetric=True needs a network or predict() evaluator: the built-in evaluators run in the fused "
+                             "k_run_sims path, which has no symmetric variant (and the uniform one is symmetric already)")
         if self._engine is not None:
             self._engine.bump_eval_epoch()  # other weights or another evaluator: what the cache holds no longer applies
             torch.cuda.current_stream(self._engine.device).synchronize()
@@ -297,6 +304,13 @@ class AlphaZeroSearch:
         elif engine.root_noise != (float(rn.alpha), float(rn.fraction), int(rn.seed), int(rn.slot_offset)):
             engine.set_root_noise(rn.alpha, rn.fraction, rn.seed, rn.slot_offset)
 
+    def _configure_symmetry(self, engine: Engine):
+        """before any selection of this search and any capture of its CUDA graph (launches bake the kernel choice in)"""
+        if engine.symmetric_eval != self.symmetric:
+            engine.set_symmetric_eval(self.symmetric)
+            if self._graphed is not None and self._graphed.engine is engine:
+                self._graphed = None
+
     def close(self):
         if self._engine is not None:
             self._engine.close()
@@ -313,6 +327,7 @@ class AlphaZeroSearch:
             self._engine = Engine(num_games=n, num_simulations=self.num_simulations, c_puct=float(self.exploration_weight),
                                   device=self.device_index, lanes_per_tree=self.lanes_per_tree)
             self._graphed = None
+        self._configure_symmetry(self._engine)
         return self._engine
 
     def simulate(self, engine: Engine, num_simulations: int | None = None, evaluator_events: list | None = None):
@@ -320,6 +335,7 @@ class AlphaZeroSearch:
         is mixed into the root priors after the first.  `evaluator_events` (network evaluators only): run the steps un-graphed and
         collect a CUDA-event pair around every evaluator call."""
         S = self.num_simulations if num_simulations is None else num_simulations
+        self._configure_symmetry(engine)
         self._configure_noise(engine)
         runs = self._search_runs(S)
         for i, n in enumerate(runs):

@@ -32,11 +32,15 @@ class _GraphedTraining:
     eagerly on the training stream (they ARE training steps; cuDNN / cuBLAS pick algorithms and the optimiser state is
     created there), the capture only records.  The replay set is copied into static buffers every iteration, so one capture
     serves the whole training run (a buffer that has to grow drops the graph; the next iteration captures again).
+    `mirror_augment`: every epoch draws one Bernoulli(1/2) flag per sample (next to the permutation, from the same generator);
+    a flagged sample is trained in its left-right mirror image - bitboards mirrored by `az_mirror_states` before the encoding,
+    policy target columns reversed.  The flags are device data read by the step, so the graph still takes no host arguments.
     """
 
     MIN_REPLAYS = 4  # fewer full-size steps than 3 eager + this: not worth a capture
 
-    def __init__(self, model, opt, batch_size: int, precision: str, device: torch.device, channels_last: bool = True):
+    def __init__(self, model, opt, batch_size: int, precision: str, device: torch.device, channels_last: bool = True,
+                 mirror_augment: bool = False):
         from .game import rules_engine
 
         self.model, self.opt, self.B, self.precision, self.device = model, opt, int(batch_size), precision, device
@@ -51,16 +55,25 @@ class _GraphedTraining:
         self.ctr = torch.zeros(1, dtype=torch.int64, device=device)
         self.loss_sum = torch.zeros((), dtype=torch.float32, device=device)
         self.replays = 0  # graph replays so far (reported by Trainer.history)
-        self.cap, self.data, self.perm, self.graph = 0, None, None, None
+        self.mirror_augment = bool(mirror_augment)
+        self.cap, self.data, self.perm, self.flip, self.graph = 0, None, None, None, None
 
     def _step_on(self, j):
         bb0, bb1, pl, policy, value = self.data
-        x = self.eng.encode_states(bb0.index_select(0, j), bb1.index_select(0, j), pl.index_select(0, j), self.model.input_layout)
+        if self.mirror_augment:
+            f = self.flip.index_select(0, j)
+            b0, b1 = self.eng.mirror_states(bb0.index_select(0, j), bb1.index_select(0, j), f)
+            x = self.eng.encode_states(b0, b1, pl.index_select(0, j), self.model.input_layout)
+            pol = policy.index_select(0, j)
+            pol = torch.where(f.bool().unsqueeze(1), pol.flip(1), pol)
+        else:
+            x = self.eng.encode_states(bb0.index_select(0, j), bb1.index_select(0, j), pl.index_select(0, j), self.model.input_layout)
+            pol = policy.index_select(0, j)
         if self.channels_last and x.dim() == 4:
             x = x.contiguous(memory_format=torch.channels_last)
         self.opt.zero_grad(set_to_none=True)
         with torch.autocast("cuda", dtype=torch.bfloat16, enabled=self.precision == "bf16-mixed"):
-            loss = self.model.training_step((x, policy.index_select(0, j), value.index_select(0, j)), 0)
+            loss = self.model.training_step((x, pol, value.index_select(0, j)), 0)
         loss.backward()
         self.opt.step()
         self.loss_sum += loss.detach().float()
@@ -77,6 +90,7 @@ class _GraphedTraining:
             self.cap = max(2 * n, 1 << 16)
             self.data = tuple(torch.empty((self.cap,) + tuple(t.shape[1:]), dtype=t.dtype, device=self.device) for t in fresh)
             self.perm = torch.zeros(self.cap, dtype=torch.int64, device=self.device)
+            self.flip = torch.zeros(self.cap, dtype=torch.uint8, device=self.device) if self.mirror_augment else None
             self.graph = None
         for dst, src in zip(self.data, fresh):
             dst[:n].copy_(src)
@@ -92,6 +106,8 @@ class _GraphedTraining:
             self.loss_sum.zero_()
             for _ in range(epochs):
                 self.perm[:n].copy_(torch.randperm(n, generator=generator))
+                if self.mirror_augment:
+                    self.flip[:n].copy_(torch.randint(0, 2, (n,), generator=generator, dtype=torch.uint8))
                 self.ctr.zero_()
                 done = 0
                 if use_graph and self.graph is None and full >= 3 + self.MIN_REPLAYS:
@@ -133,7 +149,7 @@ class Trainer:
               initial_state, buffer_size: int, save_every_n_iterations: int = 0, batch_size: int = 32, seed: int = 0,
               overlap: bool = True, inference_dtype: torch.dtype | None = None, precision: str = "32-true",
               cuda_graph: bool = True, trainer_share: float | None = None, save_dir: str | None = None, root_noise=None,
-              sampling_moves: int | None = None):
+              sampling_moves: int | None = None, symmetric: bool = False, mirror_augment: bool = False):
         """`overlap=True` reproduces the reference's pipeline (datamodule.py:89-101): the self-play of iteration k+1 runs on a
         background thread (own CUDA stream, weights as of the end of iteration k-1's training) while iteration k trains.
         `precision`: "32-true" (the reference's Lightning default) or "bf16-mixed" (forward / backward under bf16 autocast,
@@ -146,7 +162,10 @@ class Trainer:
         `ModelCheckpoint(every_n_epochs=...)`, trainer.py:66-70; read back with `Model.load_from_checkpoint`, scripts/play.py:19).
         `root_noise` (`search.RootNoise`) and `sampling_moves` (`EpisodeGenerator`): AlphaZero's self-play exploration, off by
         default.  Each rank's noise is keyed by the global index of its games (`slot_offset` = the first slot of its shard), so
-        the draws do not depend on how the games are sharded."""
+        the draws do not depend on how the games are sharded.
+        `symmetric`: self-play evaluates every leaf in its canonical orientation under the left-right mirror
+        (`AlphaZeroSearch(symmetric=True)`).  `mirror_augment`: each epoch trains a random half of the samples in their mirror
+        image (`_GraphedTraining`).  Both off by default."""
         import threading
 
         world = dist.get_world_size() if dist.is_initialized() else 1
@@ -162,6 +181,8 @@ class Trainer:
         kw = {} if inference_dtype is None else dict(inference_dtype=inference_dtype)
         if root_noise is not None:
             kw["root_noise"] = dataclasses.replace(root_noise, slot_offset=lo)
+        if symmetric:
+            kw["symmetric"] = True
         gen = EpisodeGenerator(model=model, num_simulations=simulations_per_episode, num_episodes=hi - lo,
                                game_initial_state=initial_state, device=self.device_index, sampling_moves=sampling_moves, **kw)
         replay = ReplayBuffer(buffer_size, simulations_per_episode, self.device)
@@ -169,7 +190,7 @@ class Trainer:
         for group in opt.param_groups:  # Adam's step counter on the device, so that optimiser steps can be captured
             group["capturable"] = True
         g = torch.Generator().manual_seed(seed)
-        steps = _GraphedTraining(model, opt, batch_size, precision, self.device)
+        steps = _GraphedTraining(model, opt, batch_size, precision, self.device, mirror_augment=mirror_augment)
         play_stream = torch.cuda.Stream(device=self.device)
         box: dict = {}
 

@@ -13,7 +13,7 @@ __version__ = "0.1.0"
 from ._lib import LIB_PATH, build_library, library_available  # noqa: E402,F401
 from .engine import Engine, EpisodeBatch  # noqa: E402,F401
 from .evaluators import HashEvaluator, UniformEvaluator  # noqa: E402,F401
-from .game import Action, Config, State  # noqa: E402,F401
+from .game import Action, Config, State, canonical_bitboards, mirror_bitboards  # noqa: E402,F401
 from .episode import Episode, Sample  # noqa: E402,F401
 from .search import AlphaZeroSearch, Node, RootNoise  # noqa: E402,F401
 from .episode_generator import EpisodeGenerator  # noqa: E402,F401

@@ -156,12 +156,14 @@ int32_t az_expand_backup(az_engine *h, const float *policy /*[E][7]*/, const flo
 /* az_expand_backup followed by az_select_leaves in one launch (same results): the only tree kernel between two evaluator
  * calls of the simulation loop (search.py:66-91). */
 int32_t az_expand_backup_select(az_engine *h, const float *policy, const float *values, int32_t policy_kind, void *stream);
-/* the leaves chosen by the last az_select_leaves (for evaluators that want positions, not planes) */
+/* the leaves chosen by the last az_select_leaves (for evaluators that want positions, not planes); with symmetric evaluation on
+ * (az_set_symmetric_eval), every non-terminal leaf in its canonical orientation and the legal mask of that orientation */
 int32_t az_leaf_info(az_engine *h, uint64_t *out_bb0, uint64_t *out_bb1, uint8_t *out_player, uint8_t *out_legal,
                      uint8_t *out_status, void *stream);
 
 /* engine-owned device arrays describing the leaves of the last az_select_leaves (borrowed; valid until az_destroy):
- * lets another kernel consume the leaves without a gather launch (see az_mlp_forward_leaves) */
+ * lets another kernel consume the leaves without a gather launch (see az_mlp_forward_leaves).  With symmetric evaluation on,
+ * non-terminal leaves are in their canonical orientation (az_leaf_mirror tells which were mirrored). */
 int32_t az_leaf_arrays(az_engine *h, const uint64_t **bb0, const uint64_t **bb1, const uint8_t **status, int32_t *n_active);
 int32_t az_leaf_players(az_engine *h, const uint8_t **player);
 /* Leaf compaction.  Terminal leaves (search.py:75-77, ~15 % of the simulations of a running self-play loop) need no evaluation.
@@ -197,6 +199,27 @@ typedef struct az_eval_cache_stats {
 } az_eval_cache_stats;
 /* totals since az_create / az_reset_stats (az_stats.evaluations = rows + hits + followers).  Synchronises. */
 int32_t az_get_eval_cache_stats(az_engine *h, az_eval_cache_stats *out_host, void *stream);
+
+/* ---- left-right mirror symmetry of Connect4 (off by default; with it off every result is unchanged) ----
+ * mirror(b) moves column c's 7 bits (bit 7c + r) to column 6 - c, in both bitboards; the side to move does not change.  The
+ * canonical form of a position is the smaller of it and its mirror, comparing (bb0, bb1) as unsigned 64-bit values, bb0 first;
+ * a palindrome (its own mirror) is its own canonical form and is not mirrored.
+ * az_set_symmetric_eval(h, 1): the network-in-the-loop search evaluates f_sym(x) = f(canon(x)) with the policy columns reversed
+ * when canon(x) is the mirror of x.  Each selection writes the canonical form of every non-terminal leaf to the leaf arrays (what
+ * az_gather_leaves, az_leaf_info, az_leaf_arrays and every evaluator read) and probes the evaluation cache with it; the expansion
+ * stores canonical column c's prior at actual column 6 - c of a mirrored leaf.  The tree, root statistics, root noise and the
+ * episode ring stay in the actual orientation.  f_sym is a pure function of the position, so the cache stays exact; its entries
+ * hold plain rows f(y) keyed by y and stay valid when the mode changes.  Adds no launch.  AZ_E_STATE while a selection's leaves
+ * wait for their expansion; call it before capturing a CUDA graph of the search (launches bake the kernel choice in).  The fused
+ * built-in path (az_run_simulations, az_run_move_step) has no symmetric variant: it returns AZ_E_STATE while the mode is on. */
+int32_t az_set_symmetric_eval(az_engine *h, int32_t on);
+/* [E] u8 device array (borrowed; valid until az_destroy): 1 where the last selection's leaf is the mirror of the position the
+ * descent reached (0 for palindromes, terminal and idle slots); NULL when the last selection ran with the mode off */
+int32_t az_leaf_mirror(az_engine *h, const uint8_t **mirrored);
+/* out = mirror(in) for the n positions (device arrays), or, with flags (u8 [n], may be NULL = every row), only for the rows
+ * whose flag is non-zero (the others are copied).  The output may be the input. */
+int32_t az_mirror_states(az_engine *h, const uint64_t *bb0, const uint64_t *bb1, const uint8_t *flags, int64_t n, uint64_t *out_bb0,
+                         uint64_t *out_bb1, void *stream);
 
 /* ---- results ---- */
 /* root statistics of every active tree, per column (0 on illegal columns):
