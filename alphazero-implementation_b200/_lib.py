@@ -92,6 +92,10 @@ class AzRootNoise(C.Structure):
     _fields_ = [("alpha", C.c_double), ("fraction", C.c_float), ("seed", C.c_uint64), ("slot_offset", C.c_int64)]
 
 
+class AzReuseStats(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in ("retained", "fresh", "dropped", "nodes", "visits")]
+
+
 class AzResnetDesc(C.Structure):
     _fields_ = [
         ("num_blocks", C.c_int32), ("num_channels", C.c_int32), ("operand_format", C.c_int32), ("variant", C.c_int32),
@@ -165,6 +169,9 @@ SIGNATURES = {
     "az_root_noise_values": (I32, [P, P, P]),
     "az_set_greedy_from": (I32, [P, I32]),
     "az_set_symmetric_eval": (I32, [P, I32]),
+    "az_set_subtree_reuse": (I32, [P, I32]),
+    "az_advance_roots": (I32, [P, P, P, P]),
+    "az_get_reuse_stats": (I32, [P, C.POINTER(AzReuseStats), P]),
     "az_leaf_mirror": (I32, [P, C.POINTER(P)]),
     "az_mirror_states": (I32, [P, P, P, P, I64, P, P, P]),
     "az_trunk_weight_bytes": (I64, [I32]),

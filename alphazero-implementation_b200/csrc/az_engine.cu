@@ -1,7 +1,7 @@
 // B200-native AlphaZero self-play engine: MCTS tree arena + Connect4 rules + leaf gather.
 // C ABI in include/az_engine.h.  Built for sm_100a only; there is no CPU path.
 //
-// Data layout in HBM (structure of arrays, tree-major, `cap` = roundup8(1 + 7*S) nodes per tree):
+// Data layout in HBM (structure of arrays, tree-major, `cap` = roundup8(1 + 7*S) nodes per tree, 1 + 7*V with subtree reuse):
 //   W[E][cap] f64     value_sum (node.py:14); fp64 because the reference sums Python floats
 //   M[E][cap] uint4   {visit_count u32 (node.py:13), prior f32 bits (node.py:15), first-child index u32, 0}
 //                     one 16-byte vector load per child; children of a node are contiguous in ascending
@@ -1572,11 +1572,16 @@ k_leaf_info(Arena a, int n, uint64_t *o0, uint64_t *o1, uint8_t *opl, uint8_t *o
 // Returns through copy_len / copy_dst the finished game's samples still to be copied into the ring.
 // GREEDY (az_set_greedy_from): from ply `greedy_from` of the game on, the move is the most visited root child, the lowest
 // column on ties (select_action of deepmind_alphazero_pseudocode.py past num_sampling_moves); earlier plies are sampled.
-template <bool GREEDY>
+// REUSE (az_set_subtree_reuse): a game that goes on records the played child's node index in reroot[t] for k_reroot instead of
+// resetting the tree; every other slot gets REROOT_NONE.
+constexpr uint32_t REROOT_NONE = 0u;  // node 0 is the root, never a played child
+
+template <bool GREEDY, bool REUSE>
 __device__ __forceinline__ void sample_move_slot(const Arena &a, int t, const double *__restrict__ uniforms, uint8_t *finished, int step,
                                                  uint64_t init0, uint64_t init1, int initpl, int greedy_from, int &copy_len,
-                                                 long long &copy_dst) {
+                                                 long long &copy_dst, uint32_t *reroot) {
     if (finished) finished[t] = 0;
+    if (REUSE) reroot[t] = REROOT_NONE;
     if (a.tree_err[t]) return;
     const size_t base = (size_t)t * a.cap;
     const uint4 rootm = a.M[base];
@@ -1673,21 +1678,24 @@ __device__ __forceinline__ void sample_move_slot(const Arena &a, int t, const do
         a.g_len[t] = 0;
         if (finished) finished[t] = 1;
     }
-    reset_tree(a, t);  // no subtree reuse: the new root has no children (node.py:37-41)
+    if (REUSE && !ended) reroot[t] = cb + (uint32_t)__popc(legal & ((1u << col) - 1u));
+    else reset_tree(a, t);  // no subtree reuse: the new root has no children (node.py:37-41)
 }
 
 // self-play move step (episode_generator.py:53-78, node.py:23-42): one thread per slot for the move itself; the samples of
 // games that ended (up to 42 x 45 bytes each, cold in L2 / HBM) are then copied into the ring by the whole warp, one
 // lane per sample, so the few threads with a finished game do not serialise dozens of dependent loads.
-template <bool GREEDY>
+// `reroot` is a trailing argument read by the REUSE builds only, so the REUSE = false builds keep the parameter layout.
+template <bool GREEDY, bool REUSE>
 __global__ void __launch_bounds__(128)
 k_sample_moves(Arena a, int n, const double *__restrict__ uniforms, uint8_t *finished, int step, uint64_t init0,
-               uint64_t init1, int initpl, int greedy_from) {
+               uint64_t init1, int initpl, int greedy_from, uint32_t *reroot) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
     int copy_len = 0;
     long long copy_dst = 0;
-    if (t < n) sample_move_slot<GREEDY>(a, t, uniforms, finished, step, init0, init1, initpl, greedy_from, copy_len, copy_dst);
+    if (t < n)
+        sample_move_slot<GREEDY, REUSE>(a, t, uniforms, finished, step, init0, init1, initpl, greedy_from, copy_len, copy_dst, reroot);
     __syncwarp();  // the sample recorded by this step is visible to the lanes that copy it
     unsigned todo = __ballot_sync(FULL, copy_len > 0);
     while (todo) {
@@ -1703,6 +1711,159 @@ k_sample_moves(Arena a, int n, const double *__restrict__ uniforms, uint8_t *fin
         }
         for (int i = lane; i < len * 7; i += 32) a.s_counts[dst * 7 + i] = a.g_counts[g0 * 7 + i];
     }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Subtree reuse (az_set_subtree_reuse / az_advance_roots): after the move to child c, the subtree of c becomes the tree when c is
+// expanded and N(c) + S <= V (max_root_visits), so that the next S simulations keep every visit count <= V and the tree within
+// 1 + 7 V nodes.  Otherwise the tree is a fresh root (c never expanded: "fresh"; over the bound: "dropped").
+// Per-slot counters of the outcomes, kept apart from tstats: [E][RS_N] u64.
+enum { RS_RETAINED, RS_FRESH, RS_DROPPED, RS_NODES, RS_VISITS, RS_N };
+constexpr int AZ_MAX_ROOT_VISITS = 1 << 16;  // k_reroot's two bitmaps of 1 + 7 V bits stay within one block's shared memory (115 KB)
+
+// One warp per tree compacts the subtree of c in place.  A node's children always lie above it (first_child > i) and a children
+// block is contiguous, so one ascending pass marks the subtree and the retained nodes move down in ascending order (each destination
+// is <= its source and below every source not yet read): children blocks stay contiguous and in column order, c becomes node 0
+// with {N(c), prior 0, first child remapped} and W(c).  Shared memory: two bitmaps of `words` 32-bit words - the block starts
+// (first_child values of every node; a block ends at the next start, at most 7 nodes on, or at `used`), reused for the retained
+// count below each word once the subtree is marked, and the subtree membership.
+__global__ void __launch_bounds__(32)
+k_reroot(Arena a, int n, int S, int V, const uint32_t *__restrict__ reroot, unsigned long long *__restrict__ rstats, int words) {
+    extern __shared__ uint32_t smw[];
+    uint32_t *start = smw;
+    uint32_t *member = smw + words;
+    const int t = blockIdx.x;
+    const int lane = threadIdx.x;
+    if (t >= n) return;
+    const uint32_t c = reroot[t];
+    if (c == REROOT_NONE) return;
+    const size_t base = (size_t)t * a.cap;
+    double *__restrict__ W = a.W + base;
+    uint4 *__restrict__ M = a.M + base;
+    const uint4 mc = M[c];
+    unsigned long long *st = rstats + (size_t)t * RS_N;
+    if (mc.z == 0 || mc.x + (uint32_t)S > (uint32_t)V) {
+        if (lane == 0) {
+            reset_tree(a, t);
+            st[mc.z == 0 ? RS_FRESH : RS_DROPPED] += 1ull;
+        }
+        return;
+    }
+    const uint32_t used = a.used[t];
+    for (int w = lane; w < words; w += 32) {
+        start[w] = 0u;
+        member[w] = 0u;
+    }
+    __syncwarp();
+    for (uint32_t i = lane; i < used; i += 32) {
+        const uint32_t cb = reinterpret_cast<const uint32_t *>(M + i)[2];
+        if (cb) atomicOr(&start[cb >> 5], 1u << (cb & 31));
+    }
+    if (lane == 0) atomicOr(&member[c >> 5], 1u << (c & 31));
+    __syncwarp();
+    // mark: a chunk of 32 nodes may hold a node and its children (then the loop goes round again for them)
+    for (uint32_t i0 = c & ~31u; i0 < used; i0 += 32) {
+        const uint32_t i = i0 + lane;
+        const bool in = i >= c && i < used;
+        const uint32_t cb = in ? reinterpret_cast<const uint32_t *>(M + i)[2] : 0u;
+        bool done = false;
+        for (;;) {
+            const bool m = in && ((member[i0 >> 5] >> lane) & 1u);
+            if (m && !done && cb) {
+                const uint32_t wi = cb >> 5;
+                uint64_t win = start[wi];
+                if (wi + 1 < (uint32_t)words) win |= (uint64_t)start[wi + 1] << 32;
+                const uint64_t after = (win >> (cb & 31)) >> 1;  // block starts at cb + 1, cb + 2, ...
+                uint32_t k = after ? (uint32_t)__ffsll((long long)after) : 7u;
+                k = k < 7u ? k : 7u;
+                k = cb + k <= used ? k : used - cb;
+                const uint64_t bits = ((1ull << k) - 1ull) << (cb & 31);
+                atomicOr(&member[wi], (uint32_t)bits);
+                if (bits >> 32) atomicOr(&member[wi + 1], (uint32_t)(bits >> 32));
+            }
+            done = done || m;
+            __syncwarp();
+            if (!__any_sync(FULL, in && !done && ((member[i0 >> 5] >> lane) & 1u))) break;
+        }
+    }
+    __syncwarp();
+    // start[w] := retained nodes in words below w (words below c's hold none)
+    uint32_t carry = 0;
+    const uint32_t wend = (used + 31) >> 5;
+    for (uint32_t wb = c >> 5; wb < wend; wb += 32) {
+        const uint32_t w = wb + lane;
+        const uint32_t cnt = w < wend ? (uint32_t)__popc(member[w]) : 0u;
+        uint32_t incl = cnt;
+#pragma unroll
+        for (int off = 1; off < 32; off <<= 1) {
+            const uint32_t o = __shfl_up_sync(FULL, incl, off);
+            incl += lane >= off ? o : 0u;
+        }
+        if (w < wend) start[w] = carry + incl - cnt;
+        carry += __shfl_sync(FULL, incl, 31);
+    }
+    __syncwarp();
+    // move: node i goes to its rank among the retained nodes
+    for (uint32_t i0 = c & ~31u; i0 < used; i0 += 32) {
+        const uint32_t i = i0 + lane;
+        const uint32_t mw = member[i0 >> 5];
+        const bool m = i < used && ((mw >> lane) & 1u);
+        double w = 0.0;
+        uint4 rec = make_uint4(0u, 0u, 0u, 0u);
+        if (m) {
+            w = W[i];
+            rec = M[i];
+            if (rec.z) rec.z = start[rec.z >> 5] + (uint32_t)__popc(member[rec.z >> 5] & ((1u << (rec.z & 31)) - 1u));
+            if (i == c) rec.y = 0u;  // the root's prior
+        }
+        const uint32_t dst = start[i0 >> 5] + (uint32_t)__popc(mw & ((1u << lane) - 1u));
+        __syncwarp();  // every source of this chunk is read before any destination of it is written
+        if (m) {
+            W[dst] = w;
+            M[dst] = rec;
+        }
+    }
+    if (lane == 0) {
+        a.used[t] = carry;
+        st[RS_RETAINED] += 1ull;
+        st[RS_NODES] += carry;
+        st[RS_VISITS] += mc.x;
+    }
+}
+
+// az_advance_roots: plays cols[t] on every active root.  An illegal column (or a root in error) leaves the slot untouched; a move
+// that ends the game makes that position the root of a fresh tree flagged AZ_TREE_ROOT_ENDED; otherwise k_reroot applies the
+// retention rule to the played child (an unexpanded root just gets the new position).  Game logs are not touched.
+__global__ void __launch_bounds__(256)
+k_advance_roots(Arena a, int n, const uint8_t *__restrict__ cols, uint8_t *__restrict__ status, uint32_t *__restrict__ reroot) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    reroot[t] = REROOT_NONE;
+    uint64_t b0 = a.root_bb0[t], b1 = a.root_bb1[t];
+    const int pl = a.root_player[t];
+    const uint32_t legal = a.tree_err[t] ? 0u : c4::legal_mask(b0 | b1);
+    const int col = cols[t];
+    if (col >= c4::W || !((legal >> col) & 1u)) {
+        status[t] = 1;
+        return;
+    }
+    status[t] = 0;
+    const uint32_t cb = a.M[(size_t)t * a.cap].z;
+    const uint64_t bit = c4::drop_bit(b0 | b1, col);
+    if (pl == 0) b0 |= bit; else b1 |= bit;
+    const bool ended = c4::has4(pl ? b1 : b0) || c4::is_full(b0 | b1);
+    a.root_bb0[t] = b0;
+    a.root_bb1[t] = b1;
+    a.root_player[t] = (uint8_t)(pl ^ 1);
+    a.leaf_status[t] = AZ_LEAF_IDLE;
+    if (ended) a.tree_err[t] = AZ_TREE_ROOT_ENDED;
+    if (ended || cb == 0) reset_tree(a, t);
+    else reroot[t] = cb + (uint32_t)__popc(legal & ((1u << col) - 1u));
+}
+
+__global__ void __launch_bounds__(256) k_reset_trees(Arena a, int n) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < n) reset_tree(a, t);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1892,6 +2053,9 @@ struct az_engine {
     bool sym;              // az_set_symmetric_eval: selections write canonical leaves (the SYM kernels)
     bool sym_sel;          // ... and the last selection did (leaf_mirror describes its leaves)
     uint8_t *leaf_mirror;  // [E] 1 = the leaf arrays hold the mirror of the leaf the descent reached (allocated with the first az_set_symmetric_eval)
+    int reuse_v;               // az_set_subtree_reuse: max_root_visits V, 0 = off (the arena and the tables are sized for V, else for S)
+    uint32_t *reroot;          // [E] played child for k_reroot (REROOT_NONE = nothing to keep); allocated with the first az_set_subtree_reuse
+    unsigned long long *rstats;  // [E][RS_N] k_reroot's counters
     int64_t bytes;
     int64_t launches;
     unsigned long long *d_tot;   // [16] stats totals (device)
@@ -1943,6 +2107,17 @@ int dev_alloc(az_engine *h, T **p, size_t count) {
     return AZ_OK;
 }
 
+// releases an allocation of dev_alloc (`bytes` = what it took)
+void dev_free(az_engine *h, void *p, size_t bytes) {
+    for (int i = 0; i < h->n_allocs; ++i)
+        if (h->allocs[i] == p) {
+            cudaFree(p);
+            h->allocs[i] = h->allocs[--h->n_allocs];
+            h->bytes -= (int64_t)bytes;
+            return;
+        }
+}
+
 void use_ring(az_engine *h, int r) {
     const RingPtrs &g = h->rings[r];
     Arena &a = h->a;
@@ -1978,6 +2153,16 @@ int launch_encode(az_engine *h, const uint64_t *bb0, const uint64_t *bb1, const 
         default: k_encode<AZ_LAYOUT_PLANES_BF16_NHWC><<<blocks, B, smem, st>>>(bb0, bb1, player, status, n, o); break;
     }
     AZ_LAUNCH_CHECK(h, "k_encode");
+    return AZ_OK;
+}
+
+// k_reroot over the first n slots, after k_sample_moves<REUSE> or k_advance_roots wrote h->reroot
+int launch_reroot(az_engine *h, int n, cudaStream_t st) {
+    const int words = (h->a.cap + 31) / 32;
+    const size_t smem = (size_t)2 * words * sizeof(uint32_t);
+    if (smem > 48 * 1024) AZ_CUDA(h, cudaFuncSetAttribute(k_reroot, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_reroot<<<n, 32, smem, st>>>(h->a, n, h->cfg.num_simulations, h->reuse_v, h->reroot, h->rstats, words);
+    AZ_LAUNCH_CHECK(h, "k_reroot");
     return AZ_OK;
 }
 }  // namespace
@@ -2292,7 +2477,8 @@ int32_t az_run_move_step(az_engine *h, int32_t num_sims, int32_t eval_kind, cons
     if (!uniforms) return fail(h, AZ_E_INVALID, "%s", "az_run_move_step: null uniforms");
     if (!h->have_init) return fail(h, AZ_E_STATE, "%s", "az_run_move_step: call az_reset_games first");
     if (num_sims < 1) return fail(h, AZ_E_INVALID, "%s", "az_run_move_step: num_sims < 1");
-    if (h->greedy_from >= 0) {  // the greedy rule lives in k_sample_moves only: the search, then the move, as two launches
+    // the greedy rule and subtree reuse live in k_sample_moves (+ k_reroot) only: the search (its hot prefix written back), then the move
+    if (h->greedy_from >= 0 || h->reuse_v > 0) {
         const int32_t rc = run_sims_impl(h, num_sims, eval_kind, nullptr, nullptr, false, stream);
         if (rc != AZ_OK) return rc;
         return az_sample_moves(h, uniforms, finished, stream);
@@ -2602,13 +2788,25 @@ int32_t az_sample_moves(az_engine *h, const double *uniforms, uint8_t *finished,
     if (!h->have_init) return fail(h, AZ_E_STATE, "%s", "az_sample_moves: call az_reset_games first");
     if (int rc = set_device(h)) return rc;
     const int n = h->n_active;
-    if (h->greedy_from >= 0)
-        k_sample_moves<true><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0, h->init1,
-                                                                       h->initpl, h->greedy_from);
-    else
-        k_sample_moves<false><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0, h->init1,
-                                                                        h->initpl, -1);
+    const bool reuse = h->reuse_v > 0;
+    if (h->greedy_from >= 0) {
+        if (reuse)
+            k_sample_moves<true, true><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0,
+                                                                                 h->init1, h->initpl, h->greedy_from, h->reroot);
+        else
+            k_sample_moves<true, false><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0,
+                                                                                  h->init1, h->initpl, h->greedy_from, nullptr);
+    } else {
+        if (reuse)
+            k_sample_moves<false, true><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0,
+                                                                                  h->init1, h->initpl, -1, h->reroot);
+        else
+            k_sample_moves<false, false><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0,
+                                                                                   h->init1, h->initpl, -1, nullptr);
+    }
     AZ_LAUNCH_CHECK(h, "k_sample_moves");
+    if (reuse)
+        if (int rc = launch_reroot(h, n, S(stream))) return rc;
     h->step++;
     h->sims_done = 0;
     h->noise_applied = false;
@@ -2855,6 +3053,119 @@ int32_t az_reset_stats(az_engine *h, void *stream) {
     k_zero_u32<<<148, 256, 0, S(stream)>>>(h->a.tstats, (long long)h->a.E * NSTAT);
     AZ_LAUNCH_CHECK(h, "k_zero_u32");
     memset(h->acc_tot, 0, sizeof h->acc_tot);
+    if (h->rstats) AZ_CUDA(h, cudaMemsetAsync(h->rstats, 0, (size_t)h->a.E * RS_N * sizeof(unsigned long long), S(stream)));
+    return AZ_OK;
+}
+
+int32_t az_set_subtree_reuse(az_engine *h, int32_t max_root_visits) {
+    if (!h) return AZ_E_INVALID;
+    const int S_ = h->cfg.num_simulations;
+    if (max_root_visits != 0 && (max_root_visits < S_ || max_root_visits > AZ_MAX_ROOT_VISITS))
+        return fail(h, AZ_E_INVALID, "%s", "az_set_subtree_reuse: max_root_visits must be 0 (off) or in [num_simulations, 65536]");
+    if (h->sel_pending) return fail(h, AZ_E_STATE, "%s", "az_set_subtree_reuse: a selection's leaves wait for their expansion");
+    if (int rc = set_device(h)) return rc;
+    Arena &a = h->a;
+    const int E = a.E;
+    const int V = max_root_visits ? max_root_visits : S_;
+    const int cap = ((1 + 7 * V) + 7) & ~7;
+    const int tab_n = V + 8;
+    // everything new is allocated before anything old is released: on AZ_E_NOMEM the engine is as it was
+    double *W = nullptr;
+    uint4 *M = nullptr;
+    double *rcp = nullptr, *sqt = nullptr;
+    double2 *t2 = nullptr;
+    int rc = AZ_OK;
+    if (cap != a.cap) {
+        rc = dev_alloc(h, &W, (size_t)E * cap);
+        if (rc == AZ_OK) rc = dev_alloc(h, &M, (size_t)E * cap);
+    }
+    if (rc == AZ_OK && tab_n != a.tab_n) {
+        rc = dev_alloc(h, &rcp, tab_n);
+        if (rc == AZ_OK) rc = dev_alloc(h, &sqt, tab_n);
+        if (rc == AZ_OK) rc = dev_alloc(h, &t2, tab_n);
+    }
+    if (rc == AZ_OK && max_root_visits && !h->reroot) rc = dev_alloc(h, &h->reroot, E);
+    if (rc == AZ_OK && max_root_visits && !h->rstats) {
+        unsigned long long *p = nullptr;
+        rc = dev_alloc(h, &p, (size_t)E * RS_N);
+        if (rc == AZ_OK) {
+            AZ_CUDA(h, cudaMemset(p, 0, (size_t)E * RS_N * sizeof(unsigned long long)));
+            h->rstats = p;
+        }
+    }
+    if (rc != AZ_OK) {
+        void *fresh[] = {W, M, rcp, sqt, t2};
+        const size_t sz[] = {(size_t)E * cap * sizeof(double), (size_t)E * cap * sizeof(uint4), tab_n * sizeof(double),
+                             tab_n * sizeof(double), tab_n * sizeof(double2)};
+        for (int i = 0; i < 5; ++i)
+            if (fresh[i]) dev_free(h, fresh[i], sz[i]);
+        return rc;
+    }
+    AZ_CUDA(h, cudaDeviceSynchronize());  // no launch may still use what is released below
+    if (W) {
+        dev_free(h, a.W, (size_t)E * a.cap * sizeof(double));
+        dev_free(h, a.M, (size_t)E * a.cap * sizeof(uint4));
+        a.W = W;
+        a.M = M;
+        a.cap = cap;
+    }
+    if (rcp) {
+        dev_free(h, const_cast<double *>(a.rcp), a.tab_n * sizeof(double));
+        dev_free(h, const_cast<double *>(a.sqt), a.tab_n * sizeof(double));
+        dev_free(h, const_cast<double2 *>(a.t2), a.tab_n * sizeof(double2));
+        k_init_tables<<<blocks_for(tab_n, 256), 256>>>(rcp, sqt, t2, tab_n);
+        AZ_LAUNCH_CHECK(h, "k_init_tables");
+        a.rcp = rcp;
+        a.sqt = sqt;
+        a.t2 = t2;
+        a.tab_n = tab_n;
+    }
+    k_reset_trees<<<blocks_for(E, 256), 256>>>(a, E);
+    AZ_LAUNCH_CHECK(h, "k_reset_trees");
+    AZ_CUDA(h, cudaDeviceSynchronize());
+    h->reuse_v = max_root_visits;
+    h->sims_done = 0;
+    h->noise_applied = false;
+    return AZ_OK;
+}
+
+int32_t az_advance_roots(az_engine *h, const uint8_t *cols, uint8_t *out_status, void *stream) {
+    if (!h) return AZ_E_INVALID;
+    if (!cols || !out_status) return fail(h, AZ_E_INVALID, "%s", "az_advance_roots: null argument");
+    if (h->reuse_v == 0) return fail(h, AZ_E_STATE, "%s", "az_advance_roots: subtree reuse is off (az_set_subtree_reuse)");
+    if (h->sel_pending) return fail(h, AZ_E_STATE, "%s", "az_advance_roots: a selection's leaves wait for their expansion");
+    if (int rc = set_device(h)) return rc;
+    const int n = h->n_active;
+    k_advance_roots<<<blocks_for(n, 256), 256, 0, S(stream)>>>(h->a, n, cols, out_status, h->reroot);
+    AZ_LAUNCH_CHECK(h, "k_advance_roots");
+    if (int rc = launch_reroot(h, n, S(stream))) return rc;
+    h->sims_done = 0;
+    h->noise_applied = false;
+    return AZ_OK;
+}
+
+int32_t az_get_reuse_stats(az_engine *h, az_reuse_stats *out, void *stream) {
+    if (!h || !out) return AZ_E_INVALID;
+    memset(out, 0, sizeof *out);
+    if (!h->rstats) return AZ_OK;
+    if (int rc = set_device(h)) return rc;
+    const size_t n = (size_t)h->a.E * RS_N;
+    unsigned long long *buf = (unsigned long long *)malloc(n * sizeof(unsigned long long));
+    if (!buf) return fail(h, AZ_E_NOMEM, "%s", "az_get_reuse_stats: host allocation failed");
+    cudaError_t e = cudaMemcpyAsync(buf, h->rstats, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, S(stream));
+    if (e == cudaSuccess) e = cudaStreamSynchronize(S(stream));
+    if (e != cudaSuccess) {
+        free(buf);
+        return fail(h, AZ_E_CUDA, "az_get_reuse_stats: %s", cudaGetErrorString(e));
+    }
+    unsigned long long tot[RS_N] = {};
+    for (size_t i = 0; i < n; ++i) tot[i % RS_N] += buf[i];
+    free(buf);
+    out->retained = tot[RS_RETAINED];
+    out->fresh = tot[RS_FRESH];
+    out->dropped = tot[RS_DROPPED];
+    out->nodes = tot[RS_NODES];
+    out->visits = tot[RS_VISITS];
     return AZ_OK;
 }
 

@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import AzConfig, AzEvalCacheStats, AzRootNoise, AzStats
+from ._lib import AzConfig, AzEvalCacheStats, AzReuseStats, AzRootNoise, AzStats
 
 EVAL_UNIFORM = 1
 EVAL_HASH = 2
@@ -49,7 +49,8 @@ class EpisodeBatch:
     """Finished games as flat host arrays (the device ring drained once).
 
     Episode i owns samples [ep_offset[i], ep_offset[i] + ep_len[i]).  Policy target of a sample =
-    s_counts / (S - 1) (`Node.improved_policy`, node.py:23-29); value target = ep_outcome of its episode
+    s_counts / (root visits - 1) = s_counts over their sum (`Node.improved_policy`, node.py:23-29; S - 1 unless the root kept
+    its subtree, `Engine.set_subtree_reuse`); value target = ep_outcome of its episode
     (`Episode.backpropagate_outcome`, episode.py:52-54).  Sorted in the reference's yield order (step, slot).
     """
 
@@ -98,6 +99,7 @@ class Engine:
         self.root_noise = None  # (alpha, fraction, seed, slot_offset) while noise is configured
         self.greedy_from = -1
         self.symmetric_eval = False
+        self.subtree_reuse = 0  # max_root_visits, 0 = off
         self.tree_capacity = self.lib.az_tree_capacity(self.h)
 
     # -- plumbing --------------------------------------------------------------------------------
@@ -277,6 +279,35 @@ class Engine:
                 self.__cuda_array_interface__ = dict(shape=(n,), typestr="|u1", data=(ptr, False), version=2)
 
         return torch.as_tensor(_Raw(p.value, self.num_games), device=self.device)
+
+    def set_subtree_reuse(self, max_root_visits: int | None):
+        """Subtree reuse (`az_set_subtree_reuse`): after each self-play move (and `advance_roots`) the played child becomes the root
+        and keeps its subtree with all its statistics when it is expanded and N(child) + num_simulations <= max_root_visits; every
+        search still runs num_simulations new simulations.  None / 0 = off (the default).  Sizes the trees for 1 + 7 max_root_visits
+        nodes (`tree_capacity`) and resets every tree to a fresh root (positions and game logs are kept).  Call it before a CUDA
+        graph of the search is captured."""
+        v = 0 if max_root_visits is None else int(max_root_visits)
+        self._check(self.lib.az_set_subtree_reuse(self.h, v), "az_set_subtree_reuse")
+        self.subtree_reuse = v
+        self.tree_capacity = self.lib.az_tree_capacity(self.h)
+
+    def advance_roots(self, cols) -> torch.Tensor:
+        """Play column `cols[t]` on every active root and keep that child's subtree under the reuse rule (`az_advance_roots`; subtree
+        reuse must be on).  -> u8 status per root: 0 played, 1 illegal column (the slot is left as it was).  A move that ends the game
+        leaves that position as a finished root (`TREE_ROOT_ENDED`)."""
+        cols = self._dev(cols, torch.uint8)
+        assert cols.numel() >= self.n_active
+        status = self.empty(self.n_active, torch.uint8)
+        self._check(self.lib.az_advance_roots(self.h, _ptr(cols), _ptr(status), _stream()), "az_advance_roots")
+        return status
+
+    def reuse_stats(self) -> dict:
+        """Moves whose played child's subtree was retained, that went to a never-expanded child (fresh) or were dropped
+        (N(child) + num_simulations > max_root_visits), and the retained nodes and root visits - totals since creation /
+        `reset_stats`."""
+        st = AzReuseStats()
+        self._check(self.lib.az_get_reuse_stats(self.h, C.byref(st), _stream()), "az_get_reuse_stats")
+        return {n: int(getattr(st, n)) for n, _ in AzReuseStats._fields_}
 
     def run_simulations(self, num_sims: int, eval_kind: int):
         self._check(self.lib.az_run_simulations(self.h, int(num_sims), int(eval_kind), _stream()), "az_run_simulations")

@@ -65,12 +65,14 @@ class Episode:
 def episodes_from_batch(batch, num_simulations: int) -> list[Episode]:
     """Materialise an `EpisodeBatch` (flat arrays from the device ring) as reference-style objects.
 
-    policy[a] = child visits / (S - 1) as a Python float (int / int true division, node.py:27);
+    policy[a] = child visits / (root visits - 1) as a Python float (int / int true division, node.py:27), where root visits - 1
+    is the sample's count sum: S - 1 for a search on a fresh root (the first simulation expands the root, every later one passes
+    through a child), N(c) + S - 1 on a root that kept its subtree (`AlphaZeroSearch(subtree_reuse=...)`).  `num_simulations` is
+    kept for the signature; the row sum gives the same denominator for fresh roots.
     value = outcome list shared by every sample of the episode (episode.py:52-54).
     """
     from .game import DEFAULT_CONFIG, rules_engine
 
-    denom = num_simulations - 1
     out = []
     if batch.num_samples == 0:
         return out
@@ -82,6 +84,7 @@ def episodes_from_batch(batch, num_simulations: int) -> list[Episode]:
         ep = Episode()
         for i in range(o, o + n):
             counts = batch.s_counts[i]
+            denom = int(counts.sum())
             bb0, bb1 = int(batch.s_bb0[i]), int(batch.s_bb1[i])
             legal = int(legal_all[i])
             st = State(DEFAULT_CONFIG, bb0, bb1, int(batch.s_player[i]), legal=legal, ended=False, reward=(0, 0))

@@ -46,9 +46,13 @@ class _Chunk:
 
 
 class ReplayBuffer:
-    def __init__(self, buffer_size: int, num_simulations: int, device: torch.device | str = "cuda"):
+    def __init__(self, buffer_size: int, num_simulations: int, device: torch.device | str = "cuda", *, subtree_reuse: bool = False):
+        """`subtree_reuse`: the samples come from searches whose roots may have kept their subtree (`AlphaZeroSearch(subtree_reuse=)`),
+        so a root holds N(c) + S visits: policy targets are the counts over each row's own sum (root visits - 1) instead of over
+        S - 1.  Rows of fresh roots sum to S - 1 and get the same bits either way."""
         self.buffer_size = int(buffer_size)
         self.num_simulations = int(num_simulations)
+        self.subtree_reuse = bool(subtree_reuse)
         self.device = torch.device(device)
         self.chunks: deque[_Chunk] = deque()
 
@@ -93,6 +97,11 @@ class ReplayBuffer:
         pl = torch.cat([c.s_player[c.first_sample:] for c in cs])
         counts = torch.cat([c.s_counts[c.first_sample:] for c in cs]).to(torch.float32)
         policy = counts / float(self.num_simulations - 1)  # Node.improved_policy (node.py:27), fp32 like torch.zeros(...)[i, col] = prob
+        if self.subtree_reuse:
+            # counts / (root visits - 1) = over the row's sum, more than S - 1 for a root that kept its subtree.  Rows that sum to
+            # S - 1 keep the scalar division above (on CUDA a multiply by the fp32 reciprocal): the same bits as without reuse
+            rows = counts.sum(1, keepdim=True)
+            policy = torch.where(rows == float(self.num_simulations - 1), policy, counts / rows)
         value = torch.cat([torch.repeat_interleave(c.ep_outcome[c.first:].to(torch.float32), c.ep_len[c.first:], dim=0) for c in cs])
         return bb0, bb1, pl, policy, value
 

@@ -199,7 +199,7 @@ class AlphaZeroSearch:
     def __init__(self, *, model, num_simulations: int, exploration_weight: float = 1.0, device: int | None = None,
                  lanes_per_tree: int = 0, inference_dtype: torch.dtype | None = None, use_cuda_graph: bool = True,
                  use_tensor_core_kernels: bool = True, trunk_variant: int | None = None, eval_cache: bool | int = True,
-                 root_noise: RootNoise | None = None, symmetric: bool = False):
+                 root_noise: RootNoise | None = None, symmetric: bool = False, subtree_reuse: bool | int = False):
         """`eval_cache`: serve repeated leaf positions from the engine's evaluation cache (`Engine.set_eval_cache`) when the
         evaluator's outputs depend on the position alone (`InferenceNet.position_only_outputs`); same results, fewer evaluator rows.
         True = a table sized for the engine, False = off, an int = log2 of its entry count.
@@ -207,8 +207,14 @@ class AlphaZeroSearch:
         other num_simulations - 1; None (default) = no noise.
         `symmetric`: evaluate every leaf in its canonical orientation under Connect4's left-right mirror (`Engine.set_symmetric_eval`):
         a position and its mirror get the same value and mirrored priors, and share one evaluator row and one cache entry.  Network
-        and `predict` evaluators only (ValueError for the built-in ones); off (default) = the reference's search, bit for bit."""
+        and `predict` evaluators only (ValueError for the built-in ones); off (default) = the reference's search, bit for bit.
+        `subtree_reuse`: in the self-play move step (`simulate_and_move`) the played child becomes the next root and keeps its subtree
+        with all its statistics (AlphaGo Zero), as long as N(child) + num_simulations <= max_root_visits (`Engine.set_subtree_reuse`);
+        each search still runs num_simulations new simulations, so a root then holds more visits.  True = max_root_visits of
+        4 num_simulations, an int = max_root_visits, False (default) = every move step starts from a fresh root, as the reference
+        does.  `run_simulations(nodes)` always starts from the given fresh roots."""
         self.symmetric = bool(symmetric)
+        self.subtree_reuse = subtree_reuse
         self.inference_model = model.get_inference_clone()
         self.eval_cache = eval_cache
         self.root_noise = root_noise
@@ -278,20 +284,29 @@ class AlphaZeroSearch:
         """A search of S simulations as runs of consecutive simulations: with root noise, one simulation, the noise, the rest."""
         return [1, S - 1] if self.root_noise is not None and S > 0 else [S]
 
+    @property
+    def max_root_visits(self) -> int:
+        """max_root_visits of the self-play engine's subtree reuse: 0 = off"""
+        r = self.subtree_reuse
+        if r is True:
+            return 4 * self.num_simulations
+        return 0 if r is False or r is None else int(r)
+
     def launches_per_move_step(self) -> int:
         """Kernels of libaz_engine.so per self-play move step (`simulate_and_move`)."""
         S = self.num_simulations
         runs = [n for n in self._search_runs(S) if n > 0]
         noise = 1 if self.root_noise is not None else 0
         greedy = self._engine is not None and self._engine.greedy_from >= 0
+        reuse = 1 if self.max_root_visits else 0  # k_reroot after k_sample_moves
         if self._mode == "builtin":
-            # one k_run_sims per run, the last one with the move fused in - unless the greedy cutoff (or a search of one simulation
-            # with noise) leaves the move to k_sample_moves
-            return len(runs) + noise + (1 if greedy or noise and S == 1 else 0)
+            # one k_run_sims per run, the last one with the move fused in - unless the greedy cutoff, subtree reuse (or a search of one
+            # simulation with noise) leaves the move to k_sample_moves
+            return len(runs) + noise + (1 if greedy or reuse or noise and S == 1 else 0) + reuse
         # per run of n: k_select; n - 1 x (evaluator or gather, k_expand_select); evaluator, k_expand_backup.  Then k_root_noise
         # between the runs and k_sample_moves.  When the evaluator walks the compacted leaf list: one k_compact_leaves after
         # every k_select (the later lists come out of k_expand_select) or, AZ_COMPACT_FUSED=0, one per selection
-        n = sum(2 * r + 1 for r in runs) + noise + 1
+        n = sum(2 * r + 1 for r in runs) + noise + 1 + reuse
         if not getattr(self._net, "wants_leaf_compaction", False):
             return n
         return n + (len(runs) if os.environ.get("AZ_COMPACT_FUSED", "1") != "0" else S)
@@ -308,6 +323,15 @@ class AlphaZeroSearch:
         """before any selection of this search and any capture of its CUDA graph (launches bake the kernel choice in)"""
         if engine.symmetric_eval != self.symmetric:
             engine.set_symmetric_eval(self.symmetric)
+            if self._graphed is not None and self._graphed.engine is engine:
+                self._graphed = None
+
+    def _configure_reuse(self, engine: Engine):
+        """before the move step's search and any capture of its CUDA graph (launches bake the tree arena in); a change resets every
+        tree to a fresh root"""
+        v = self.max_root_visits
+        if engine.subtree_reuse != v:
+            engine.set_subtree_reuse(v)
             if self._graphed is not None and self._graphed.engine is engine:
                 self._graphed = None
 
@@ -357,7 +381,9 @@ class AlphaZeroSearch:
 
     def simulate_and_move(self, engine: Engine, uniforms: torch.Tensor, finished: torch.Tensor | None = None):
         """One self-play move step: `simulate` then `Engine.sample_moves(uniforms)`.  With a built-in evaluator both run in
-        one launch (`az_run_move_step`), with identical results."""
+        one launch (`az_run_move_step`), with identical results.  With `subtree_reuse`, the move keeps the played child's subtree
+        (`k_reroot`) for the next step's search."""
+        self._configure_reuse(engine)
         if self._mode == "builtin":
             kind = self.inference_model.az_builtin_eval_kind
             self._configure_noise(engine)

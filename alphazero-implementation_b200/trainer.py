@@ -149,7 +149,8 @@ class Trainer:
               initial_state, buffer_size: int, save_every_n_iterations: int = 0, batch_size: int = 32, seed: int = 0,
               overlap: bool = True, inference_dtype: torch.dtype | None = None, precision: str = "32-true",
               cuda_graph: bool = True, trainer_share: float | None = None, save_dir: str | None = None, root_noise=None,
-              sampling_moves: int | None = None, symmetric: bool = False, mirror_augment: bool = False):
+              sampling_moves: int | None = None, symmetric: bool = False, mirror_augment: bool = False,
+              subtree_reuse: bool | int = False):
         """`overlap=True` reproduces the reference's pipeline (datamodule.py:89-101): the self-play of iteration k+1 runs on a
         background thread (own CUDA stream, weights as of the end of iteration k-1's training) while iteration k trains.
         `precision`: "32-true" (the reference's Lightning default) or "bf16-mixed" (forward / backward under bf16 autocast,
@@ -165,7 +166,10 @@ class Trainer:
         the draws do not depend on how the games are sharded.
         `symmetric`: self-play evaluates every leaf in its canonical orientation under the left-right mirror
         (`AlphaZeroSearch(symmetric=True)`).  `mirror_augment`: each epoch trains a random half of the samples in their mirror
-        image (`_GraphedTraining`).  Both off by default."""
+        image (`_GraphedTraining`).  Both off by default.
+        `subtree_reuse`: each self-play move keeps the played child's subtree for the next search (`AlphaZeroSearch(subtree_reuse=)`:
+        True = max_root_visits of 4 simulations_per_episode, an int = max_root_visits); off by default.  The replay buffer then divides
+        each sample's visit counts by their sum (`ReplayBuffer(subtree_reuse=True)`)."""
         import threading
 
         world = dist.get_world_size() if dist.is_initialized() else 1
@@ -183,9 +187,11 @@ class Trainer:
             kw["root_noise"] = dataclasses.replace(root_noise, slot_offset=lo)
         if symmetric:
             kw["symmetric"] = True
+        if subtree_reuse:
+            kw["subtree_reuse"] = subtree_reuse
         gen = EpisodeGenerator(model=model, num_simulations=simulations_per_episode, num_episodes=hi - lo,
                                game_initial_state=initial_state, device=self.device_index, sampling_moves=sampling_moves, **kw)
-        replay = ReplayBuffer(buffer_size, simulations_per_episode, self.device)
+        replay = ReplayBuffer(buffer_size, simulations_per_episode, self.device, subtree_reuse="subtree_reuse" in kw)
         opt = model.configure_optimizers()
         for group in opt.param_groups:  # Adam's step counter on the device, so that optimiser steps can be captured
             group["capturable"] = True

@@ -238,14 +238,15 @@ int32_t az_export_tree(az_engine *h, int32_t slot, double *W, uint32_t *N, float
 /* ---- self-play (episode_generator.py:53-78) ---- */
 /* For every slot in slot order semantics: record the sample (root position, child visit counts),
  * draw the move with the supplied uniform exactly as np.random.choice(k, p=N_c/(N-1)) would
- * (node.py:31-35), advance the root (no subtree reuse, node.py:37-41); if the successor is terminal,
+ * (node.py:31-35), advance the root (no subtree reuse unless az_set_subtree_reuse, node.py:37-41); if the successor is terminal,
  * finish the episode (outcome = successor reward, episode.py:52-54), move it to the episode ring and
  * recycle the slot to the initial state.  finished[slot] (may be NULL) = 1 where an episode finished.
  * Increments the move-step counter. */
 int32_t az_sample_moves(az_engine *h, const double *uniforms /*[E]*/, uint8_t *finished, void *stream);
 /* One whole move step of the self-play loop (episode_generator.py:53-78) with a built-in deterministic evaluator in ONE
  * launch: az_run_simulations(num_sims, evaluator_kind) followed by az_sample_moves(uniforms, finished), same results.
- * The root's child statistics never leave the registers and the discarded tree is not written back. */
+ * The root's child statistics never leave the registers and the discarded tree is not written back (no subtree reuse unless
+ * az_set_subtree_reuse: then it runs as az_run_simulations + az_sample_moves, whose k_reroot keeps the played child's subtree). */
 int32_t az_run_move_step(az_engine *h, int32_t num_sims, int32_t evaluator_kind, const double *uniforms /*[E]*/, uint8_t *finished,
                          void *stream);
 /* ---- self-play exploration (absent from the reference, which ships DeepMind's pseudocode for them only; both off by default,
@@ -278,6 +279,37 @@ int32_t az_root_noise_values(az_engine *h, float *eta, void *stream);
  * With the cutoff on, az_run_move_step runs as az_run_simulations + az_sample_moves (two launches, same results). */
 int32_t az_set_greedy_from(az_engine *h, int32_t plies);
 
+/* ---- subtree reuse (AlphaGo Zero: the child of the played move becomes the new root and keeps its subtree with all its
+ * statistics; off by default, and with it off every result is unchanged) ----
+ * Each search still runs num_simulations = S new simulations.  After a move to child c of a root:
+ *   - c is expanded and N(c) + S <= max_root_visits (= V): the subtree of c becomes the tree (retained).  Its nodes keep their
+ *     relative order, so every children block stays contiguous and in column order; c becomes node 0 with {N(c), W(c), prior 0};
+ *   - c was never expanded: a fresh root (N = W = 0, no children);
+ *   - N(c) + S > V: a fresh root as well (dropped);
+ *   - a game that ended is recycled as before.
+ * A subtree of N(c) visits has at most 1 + 7 N(c) nodes, so trees stay within 1 + 7 V nodes and visit counts within V.
+ * az_set_subtree_reuse: V = 0 (off, the default) or S <= V <= 65536, else AZ_E_INVALID.  Sizes the arena for 1 + 7 V nodes per tree
+ * (az_tree_capacity) and the PUCT tables for counts up to V (AZ_E_NOMEM, and the engine unchanged, if that fails) and resets every
+ * tree to a fresh root; root positions and game logs are kept.  V = S never retains a subtree (same results as off).  AZ_E_STATE
+ * while a selection's leaves wait for their expansion.  Call it before capturing a CUDA graph of the search: launches bake the
+ * arena (tree arrays, tables, capacity) in.  While reuse is on, az_sample_moves runs k_sample_moves then k_reroot, and
+ * az_run_move_step runs as az_run_simulations + az_sample_moves. */
+int32_t az_set_subtree_reuse(az_engine *h, int32_t max_root_visits);
+/* "Play this move, keep the tree": plays cols[t] (u8, device) on every active root under the rule above.  out_status[t] (u8,
+ * device) = 0 when played; 1 for an illegal column (or a root in error), which leaves the slot untouched.  A move that ends the game
+ * makes that position the root of a fresh tree flagged AZ_TREE_ROOT_ENDED, as az_set_roots would.  Game logs are not touched.
+ * AZ_E_STATE while reuse is off or a selection's leaves wait for their expansion. */
+int32_t az_advance_roots(az_engine *h, const uint8_t *cols, uint8_t *out_status, void *stream);
+typedef struct az_reuse_stats {
+    uint64_t retained; /* moves whose played child's subtree was kept */
+    uint64_t fresh;    /* moves to a child that was never expanded */
+    uint64_t dropped;  /* moves to an expanded child with N(c) + S > V */
+    uint64_t nodes;    /* nodes of the retained subtrees */
+    uint64_t visits;   /* root visits of the retained subtrees, N(c) */
+} az_reuse_stats;
+/* totals since az_create / az_reset_stats over moves from a searched root that did not end the game.  Synchronises. */
+int32_t az_get_reuse_stats(az_engine *h, az_reuse_stats *out_host, void *stream);
+
 /* number of finished episodes / samples waiting in the ring.  Synchronises on `stream`. */
 int32_t az_episode_counts(az_engine *h, int64_t *n_episodes_host, int64_t *n_samples_host, void *stream);
 /* copy the ring out (device buffers sized from az_episode_counts) and empty it.  Episodes appear in
@@ -306,7 +338,8 @@ int32_t az_read_episode_ring(az_engine *h, int32_t ring, int64_t n_episodes, int
 int32_t az_get_stats(az_engine *h, az_stats *out_host, void *stream); /* synchronises */
 int32_t az_reset_stats(az_engine *h, void *stream);
 /* checks the table-based fp64 division used by the PUCT score against IEEE division on n pseudo-random
- * (x, d) pairs, d an integer below num_simulations + 2; *mismatches_host must come back 0.  Synchronises. */
+ * (x, d) pairs, d an integer below num_simulations + 2 (max_root_visits + 2 with az_set_subtree_reuse); *mismatches_host must
+ * come back 0.  Synchronises. */
 int32_t az_selftest_division(az_engine *h, int64_t n, uint64_t seed, int64_t *mismatches_host);
 /* number of kernels this engine has launched since az_create */
 int64_t az_launch_count(const az_engine *h);
