@@ -96,6 +96,15 @@ class AzReuseStats(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in ("retained", "fresh", "dropped", "nodes", "visits")]
 
 
+class AzPlayoutCap(C.Structure):
+    _fields_ = [("fast_sims", C.c_int32), ("p_full", C.c_float), ("seed", C.c_uint64), ("slot_offset", C.c_int64),
+                ("visit_budget", C.c_int32)]
+
+
+class AzCapStats(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in ("full_searches", "fast_searches", "samples_recorded", "samples_dropped", "simulations")]
+
+
 class AzResnetDesc(C.Structure):
     _fields_ = [
         ("num_blocks", C.c_int32), ("num_channels", C.c_int32), ("operand_format", C.c_int32), ("variant", C.c_int32),
@@ -172,6 +181,9 @@ SIGNATURES = {
     "az_set_subtree_reuse": (I32, [P, I32]),
     "az_advance_roots": (I32, [P, P, P, P]),
     "az_get_reuse_stats": (I32, [P, C.POINTER(AzReuseStats), P]),
+    "az_set_playout_cap": (I32, [P, C.POINTER(AzPlayoutCap)]),
+    "az_search_budgets": (I32, [P, P, P, P]),
+    "az_get_cap_stats": (I32, [P, C.POINTER(AzCapStats), P]),
     "az_leaf_mirror": (I32, [P, C.POINTER(P)]),
     "az_mirror_states": (I32, [P, P, P, P, I64, P, P, P]),
     "az_trunk_weight_bytes": (I64, [I32]),

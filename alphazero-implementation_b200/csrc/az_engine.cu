@@ -439,8 +439,11 @@ struct MoveArgs {
 };
 
 // TSM: the tables live in shared memory (a compile-time fact, so that the loads are LDS, not generic loads)
-template <int TPW, int EVAL, bool LAT, bool MOVE, bool TSM>
-__global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, double c_puct, int K, MoveArgs mv) {
+// BUDGET (az_set_playout_cap; MOVE = false only): a tree takes part in a simulation only while its root has fewer visits than
+// budget[t] (a trailing argument, so that the other builds keep their parameter layout); the other trees of the warp go on, and a
+// warp whose trees have all reached their budget leaves the loop
+template <int TPW, int EVAL, bool LAT, bool MOVE, bool TSM, bool BUDGET>
+__global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, double c_puct, int K, MoveArgs mv, const uint32_t *budget) {
     constexpr int TREES = 2 * TPW;  // per 64-thread block
     constexpr int NL = 32 / TPW;    // lanes per tree
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -488,6 +491,7 @@ __global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, d
     const int rpl = a.root_player[tt];
     uint32_t used = a.used[tt];
     uint32_t levels = 0, evals = 0, children = 0, scanned = 0;
+    const uint32_t bud = BUDGET ? budget[tt] : 0u;
     double mv_u = 0.0;
     int mv_len = 0;
     if (MOVE && alive) {
@@ -522,6 +526,7 @@ __global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, d
         root_n = rm.x;
         root_cb = rm.z;
     }
+    const uint32_t n0 = root_n;  // BUDGET: every simulation adds one root visit, so the simulations run are root_n - n0 at the end
     const bool r_can = (c < c4::W) && !(((rb0 | rb1) >> (c4::STRIDE * c + 5)) & 1ull);
     const unsigned r_legal = (__ballot_sync(FULL, r_can) >> sub) & 0x7Fu;
     const int r_j = __popc(r_legal & ((1u << c) - 1u));
@@ -535,8 +540,11 @@ __global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, d
     long long racc[4] = {0, 0, 0, 0};
 #endif
     for (int s = 0; s < S; ++s) {
+        // the tree's part in this simulation: `live` stands for `alive` everywhere in the loop
+        const bool live = BUDGET ? alive && root_n < bud : alive;
+        if (BUDGET && !__any_sync(FULL, live)) break;
         RCLK(c0);
-        Leaf L = descend<LAT>(tm, tb, rb0, rb1, rpl, c_puct, root_cb, root_sq, r_legal, rch, alive, writer, path, levels, scanned);
+        Leaf L = descend<LAT>(tm, tb, rb0, rb1, rpl, c_puct, root_cb, root_sq, r_legal, rch, live, writer, path, levels, scanned);
         RCLK(c1);
         RACC(0, c1, c0);
         // Straight-line from here on as well (the four trees of a warp end in different cases).
@@ -544,7 +552,7 @@ __global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, d
         // is expanded by this simulation is visited for the first time (N = 0, W = 0: a node is expanded on its first
         // visit), so it needs no load.
         __syncwarp();  // path[] (written by the tree's first lane) is visible to its other lanes
-        const bool own = alive && lit <= L.depth;
+        const bool own = live && lit <= L.depth;
         const bool fresh = lit == L.depth && !L.term;
         const uint32_t my_idx = own ? path[lit] : 0u;
         const bool my_hot = my_idx < tm.K;
@@ -571,7 +579,7 @@ __global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, d
             const float v0 = azeval::hash_value0(h);
             val = L.pl == 0 ? v0 : -v0;
         }
-        const bool expand = alive && !L.term;
+        const bool expand = live && !L.term;
         if (expand && can && first_q) store_new_child(tm, used + j, prior);
         if (expand && writer) set_first_child(tm, L.node, used);
         // the root itself was expanded: its children enter the registers; depth 1: the chosen root child got children
@@ -591,9 +599,9 @@ __global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, d
         RCLK(c2);
         RACC(1, c2, c1);
         // Backup, part 2.  Registers: root and the chosen root child; memory: every node on the path.
-        root_n += (uint32_t)alive;
+        root_n += (uint32_t)live;
         root_sq = tb.t2[root_n].y;  // next simulation's sqrt(N_root) and the root child's table entries: loaded behind the backup
-        rch.n += (uint32_t)(alive && mine);
+        rch.n += (uint32_t)(live && mine);
         if (LAT) {
             const double2 e = tb.t2[rch.n];
             rch.r1 = e.x;
@@ -603,7 +611,7 @@ __global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, d
             rch.d1 = (double)(1u + rch.n);
             rch.d0 = (double)rch.n;
         }
-        rch.w = __dadd_rn(rch.w, (alive && mine) ? backup_sign(v, L.depth, 1, L.term) : 0.0);  // + 0.0: value sums are never -0.0
+        rch.w = __dadd_rn(rch.w, (live && mine) ? backup_sign(v, L.depth, 1, L.term) : 0.0);  // + 0.0: value sums are never -0.0
         if (own) {
             const double w_new = __dadd_rn(w_old, backup_sign(v, L.depth, lit, L.term));
             if (my_hot) {
@@ -614,7 +622,7 @@ __global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, d
                 reinterpret_cast<uint32_t *>(tm.gM + my_idx)[0] = n_old + 1u;
             }
         }
-        if (alive)
+        if (live)
             for (int i = lit + NL; i <= L.depth; i += NL) visit_node(tm, path[i], backup_sign(v, L.depth, i, L.term));
         __syncwarp();
         RCLK(c3);
@@ -735,7 +743,7 @@ __global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, d
     if (writer) {
         a.used[t] = used;
         uint32_t *st = a.tstats + (size_t)t * NSTAT;
-        st[0] += (uint32_t)S;
+        st[0] += BUDGET ? root_n - n0 : (uint32_t)S;
         st[1] += evals;
         st[2] += levels;
         st[3] += children;
@@ -903,9 +911,12 @@ __device__ __forceinline__ void cache_publish(const Arena &a, uint32_t claim, in
 // SYM: a non-terminal leaf is written (and probed) in its canonical form, leaf_mirror[t] = 1 when that is its mirror (the array
 // is a trailing kernel argument rather than an Arena member, so that the other kernels' parameter layout stays as it was); every
 // evaluator then evaluates the canonical position, so the search runs with f_sym(x) = unmirror_if_flagged(f(canon(x)))
-template <int TPW, bool LAT, bool CACHE, bool SYM>
+// BUDGET (az_set_playout_cap): a tree whose root has reached its visit budget (budget[t], a trailing kernel argument like
+// leaf_mirror) has finished its search of this move step and is idle, as a tree in error is: every simulation adds exactly one
+// visit to the root, so the root's N counts the simulations done
+template <int TPW, bool LAT, bool CACHE, bool SYM, bool BUDGET>
 __device__ __forceinline__ bool select_body(const Arena &a, int n_active, double c_puct, uint32_t launch, uint32_t epoch,
-                                            uint8_t *leaf_mirror) {
+                                            uint8_t *leaf_mirror, const uint32_t *budget) {
     constexpr int TREES = 2 * TPW;
     constexpr int NL = 32 / TPW;
     const int lane = threadIdx.x & 31;
@@ -923,12 +934,13 @@ __device__ __forceinline__ bool select_body(const Arena &a, int n_active, double
     tm.sH = nullptr;
     tm.K = 0;
     AZ_SET_CAP(tm, a.cap);
-    // first round of loads, all independent: error flag, root position, root record
+    // first round of loads, all independent: error flag, root position, root record (and the visit budget)
     const int32_t err = a.tree_err[tt];
     const uint64_t rb0 = a.root_bb0[tt], rb1 = a.root_bb1[tt];
     const int rpl = a.root_player[tt];
     const uint4 rm = tm.gM[0];
-    const bool alive = in_range && err == 0;
+    const uint32_t bud = BUDGET ? budget[tt] : 0u;
+    const bool alive = in_range && err == 0 && (!BUDGET || rm.x < bud);
     const int lit = lane & (NL - 1);
     if (in_range && !alive && lit == 0) {
         a.leaf_status[t] = AZ_LEAF_IDLE;
@@ -977,11 +989,11 @@ __device__ __forceinline__ bool select_body(const Arena &a, int n_active, double
 }
 
 // split path, step 3: search.py:87-91 with the evaluator's outputs
-template <int TPW, bool LAT, bool CACHE, bool SYM>
-__global__ void __launch_bounds__(64) k_select(Arena a, int n_active, double c_puct, uint8_t *leaf_mirror) {
+template <int TPW, bool LAT, bool CACHE, bool SYM, bool BUDGET>
+__global__ void __launch_bounds__(64) k_select(Arena a, int n_active, double c_puct, uint8_t *leaf_mirror, const uint32_t *budget) {
     uint32_t launch = 0, epoch = 0;
     if (CACHE) load_cache_ctl(a, launch, epoch);
-    select_body<TPW, LAT, CACHE, SYM>(a, n_active, c_puct, launch, epoch, leaf_mirror);
+    select_body<TPW, LAT, CACHE, SYM, BUDGET>(a, n_active, c_puct, launch, epoch, leaf_mirror, budget);
 }
 
 // split path, step 3: search.py:87-91 with the evaluator's outputs
@@ -1113,15 +1125,15 @@ k_expand_backup(Arena a, int n_active, const float *__restrict__ policy, const f
 // outputs to the slots' rows and a position's outputs do not depend on the batch it falls into, so the search is unchanged.
 // CACHE: both halves use the evaluation cache; with COMPACT the last warp also advances the launch number (the ticket atomic is then
 // acq_rel, so that every warp's read of the number at its start precedes the advance).
-template <int TPW, bool LAT, bool COMPACT, bool CACHE, bool SYM>
+template <int TPW, bool LAT, bool COMPACT, bool CACHE, bool SYM, bool BUDGET>
 __global__ void __launch_bounds__(64)
 k_expand_select(Arena a, int n_active, const float *__restrict__ policy, const float *__restrict__ values, int policy_kind, double c_puct,
-                uint8_t *leaf_mirror) {
+                uint8_t *leaf_mirror, const uint32_t *budget) {
     uint32_t launch = 0, epoch = 0;
     if (CACHE) load_cache_ctl(a, launch, epoch);
     expand_backup_body<TPW, CACHE, SYM>(a, n_active, policy, values, policy_kind, launch, leaf_mirror);
     __syncwarp();
-    const bool wants = select_body<TPW, LAT, CACHE, SYM>(a, n_active, c_puct, launch, epoch, leaf_mirror);
+    const bool wants = select_body<TPW, LAT, CACHE, SYM, BUDGET>(a, n_active, c_puct, launch, epoch, leaf_mirror, budget);
     if (COMPACT) {
         const int lane = threadIdx.x & 31;
         const unsigned m = __ballot_sync(FULL, wants);
@@ -1514,6 +1526,68 @@ k_masked_softmax_tile(const float4 *__restrict__ logits, const uint8_t *__restri
 }
 
 // ------------------------------------------------------------------------------------------------
+// Counter-based random numbers of the self-play options: Philox4x32-10 (root noise, playout cap randomization)
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
+        c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+        k.x += 0x9E3779B9u;
+        k.y += 0xBB67AE85u;
+    }
+    return c;
+}
+
+__device__ __forceinline__ double u01_open(uint32_t x) { return ((double)x + 0.5) * 0x1p-32; }  // (0, 1)
+
+// Playout cap randomization (az_set_playout_cap; KataGo): each search of a self-play move step is "full" with probability p_full,
+// else "fast".  A full search runs S new simulations, a fast one fast_sims; with visit_budget the search tops the root up to that
+// many visits instead, at least one new simulation (n = max(S_t - N_start, 1)).  budget[t] = N_start + n is the root visit count at
+// which tree t stops: the BUDGET builds of the selection kernels and of k_run_sims leave it idle from there on.  Only full searches
+// become training samples.  The flag of (slot, move step) is a pure function of (seed, global slot, step): Philox keyed by the
+// seed, counter {global slot lo, hi, step, CAP_TAG}, full iff u01_open(x) < p_full in fp64 - root noise's counters end in
+// column << 24 | attempt < 7 << 24, so the two never share a counter.
+constexpr uint32_t CAP_TAG = 0xC0000000u;
+// Per-slot counters of the mode, [E][CS_N] u64.
+enum { CS_FULL, CS_FAST, CS_RECORDED, CS_DROPPED, CS_N };
+
+struct CapArgs {
+    uint32_t *budget;             // [E] absolute root visit count at which the tree stops
+    uint8_t *full;                // [E] 1 = the current search is full
+    uint8_t *g_full;              // [E][42] the flag of every ply in the game log
+    unsigned long long *cstats;   // [E][CS_N]
+    unsigned long long seed;
+    long long slot_offset;
+    double p_full;
+    int S, fast, visit_budget;
+};
+
+__device__ __forceinline__ bool cap_draw_full(const CapArgs &cp, int t, uint32_t step) {
+    const unsigned long long g = (unsigned long long)(cp.slot_offset + t);
+    const uint4 r = philox4x32_10(make_uint4((uint32_t)g, (uint32_t)(g >> 32), step, CAP_TAG),
+                                  make_uint2((uint32_t)cp.seed, (uint32_t)(cp.seed >> 32)));
+    return u01_open(r.x) < cp.p_full;
+}
+
+// the flag and the budget of the search that starts from a root with n_start visits
+__device__ __forceinline__ void cap_set(const CapArgs &cp, int t, bool full, uint32_t n_start) {
+    const uint32_t st = (uint32_t)(full ? cp.S : cp.fast);
+    const uint32_t n = !cp.visit_budget ? st : (st > n_start + 1u ? st - n_start : 1u);
+    cp.full[t] = full ? 1 : 0;
+    cp.budget[t] = n_start + n;
+}
+
+// the draw of move step `step` for every slot < n from the roots as they are (all_full: every search full with S new simulations,
+// for az_set_roots and az_advance_roots, which are not self-play)
+__global__ void __launch_bounds__(256) k_cap_draw(Arena a, int n, CapArgs cp, uint32_t step, int all_full) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    if (all_full) cp.visit_budget = 0;  // S new simulations, as without the mode, also on a root that kept its subtree
+    cap_set(cp, t, all_full || cap_draw_full(cp, t, step), a.M[(size_t)t * a.cap].x);
+}
+
+// ------------------------------------------------------------------------------------------------
 // roots / results
 __global__ void __launch_bounds__(256)
 k_set_roots(Arena a, const uint64_t *bb0, const uint64_t *bb1, const uint8_t *player, uint64_t c0, uint64_t c1,
@@ -1576,10 +1650,12 @@ k_leaf_info(Arena a, int n, uint64_t *o0, uint64_t *o1, uint8_t *opl, uint8_t *o
 // resetting the tree; every other slot gets REROOT_NONE.
 constexpr uint32_t REROOT_NONE = 0u;  // node 0 is the root, never a played child
 
-template <bool GREEDY, bool REUSE>
+// BUDGET (az_set_playout_cap): the ply's flag goes into the game log next to the sample, and a finished game emits only the samples
+// of its full searches (ep_len = their number, possibly 0); copy_len stays the number of plies, the copy skips the fast ones.
+template <bool GREEDY, bool REUSE, bool BUDGET>
 __device__ __forceinline__ void sample_move_slot(const Arena &a, int t, const double *__restrict__ uniforms, uint8_t *finished, int step,
                                                  uint64_t init0, uint64_t init1, int initpl, int greedy_from, int &copy_len,
-                                                 long long &copy_dst, uint32_t *reroot) {
+                                                 long long &copy_dst, uint32_t *reroot, const CapArgs &cp) {
     if (finished) finished[t] = 0;
     if (REUSE) reroot[t] = REROOT_NONE;
     if (a.tree_err[t]) return;
@@ -1620,8 +1696,10 @@ __device__ __forceinline__ void sample_move_slot(const Arena &a, int t, const do
         a.g_player[o] = (uint8_t)pl;
 #pragma unroll
         for (int c = 0; c < 7; ++c) a.g_counts[o * 7 + c] = cnt[c];
+        if (BUDGET) cp.g_full[o] = cp.full[t];
     }
     const int new_len = len + 1;
+    if (BUDGET) cp.cstats[(size_t)t * CS_N + (cp.full[t] ? CS_FULL : CS_FAST)] += 1ull;
     int col;
     if (GREEDY && len >= greedy_from) {
         int32_t best = -1;
@@ -1657,19 +1735,28 @@ __device__ __forceinline__ void sample_move_slot(const Arena &a, int t, const do
     } else {
         // outcome to every sample (episode.py:52-54); emit; recycle the slot (episode_generator.py:71-78)
         const int8_t r0 = win ? (pl == 0 ? 1 : -1) : 0;
+        int rec = new_len;  // samples the game emits: with the playout cap, its full plies
+        if (BUDGET) {
+            rec = 0;
+            for (int q = 0; q < new_len && q < MAX_PLIES; ++q) rec += cp.g_full[(size_t)t * MAX_PLIES + q];
+        }
         const unsigned long long e = atomicAdd(&a.ring[0], 1ull);
-        const unsigned long long o = atomicAdd(&a.ring[1], (unsigned long long)new_len);
-        if ((long long)e < a.ep_cap && (long long)(o + new_len) <= a.s_cap) {
+        const unsigned long long o = atomicAdd(&a.ring[1], (unsigned long long)rec);
+        if ((long long)e < a.ep_cap && (long long)(o + rec) <= a.s_cap) {
             a.ep_slot[e] = t;
             a.ep_step[e] = step;
-            a.ep_len[e] = new_len;
+            a.ep_len[e] = rec;
             a.ep_offset[e] = (int64_t)o;
             a.ep_outcome[2 * e] = r0;
             a.ep_outcome[2 * e + 1] = (int8_t)-r0;
-            copy_len = new_len;  // the samples are copied by the whole warp below
+            copy_len = BUDGET && rec == 0 ? 0 : new_len;  // the samples are copied by the whole warp below
             copy_dst = (long long)o;
         } else {
             atomicAdd(&a.ring[2], 1ull);
+        }
+        if (BUDGET) {
+            cp.cstats[(size_t)t * CS_N + CS_RECORDED] += (unsigned long long)rec;
+            cp.cstats[(size_t)t * CS_N + CS_DROPPED] += (unsigned long long)(new_len - rec);
         }
         st[5] += 1u;
         a.root_bb0[t] = init0;
@@ -1685,20 +1772,47 @@ __device__ __forceinline__ void sample_move_slot(const Arena &a, int t, const do
 // self-play move step (episode_generator.py:53-78, node.py:23-42): one thread per slot for the move itself; the samples of
 // games that ended (up to 42 x 45 bytes each, cold in L2 / HBM) are then copied into the ring by the whole warp, one
 // lane per sample, so the few threads with a finished game do not serialise dozens of dependent loads.
-// `reroot` is a trailing argument read by the REUSE builds only, so the REUSE = false builds keep the parameter layout.
-template <bool GREEDY, bool REUSE>
+// `reroot` and `cp` are trailing arguments read by the REUSE / BUDGET builds only, so the other builds keep the parameter layout.
+// BUDGET without REUSE also draws the flag of the slot's next search (step + 1) and writes its budget; with REUSE k_cap_draw does
+// that after k_reroot has fixed the new root's visit count.
+template <bool GREEDY, bool REUSE, bool BUDGET>
 __global__ void __launch_bounds__(128)
 k_sample_moves(Arena a, int n, const double *__restrict__ uniforms, uint8_t *finished, int step, uint64_t init0,
-               uint64_t init1, int initpl, int greedy_from, uint32_t *reroot) {
+               uint64_t init1, int initpl, int greedy_from, uint32_t *reroot, CapArgs cp) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
     int copy_len = 0;
     long long copy_dst = 0;
-    if (t < n)
-        sample_move_slot<GREEDY, REUSE>(a, t, uniforms, finished, step, init0, init1, initpl, greedy_from, copy_len, copy_dst, reroot);
+    if (t < n) {
+        sample_move_slot<GREEDY, REUSE, BUDGET>(a, t, uniforms, finished, step, init0, init1, initpl, greedy_from, copy_len, copy_dst,
+                                                reroot, cp);
+        if (BUDGET && !REUSE) cap_set(cp, t, cap_draw_full(cp, t, (uint32_t)step + 1u), a.M[(size_t)t * a.cap].x);
+    }
     __syncwarp();  // the sample recorded by this step is visible to the lanes that copy it
     unsigned todo = __ballot_sync(FULL, copy_len > 0);
-    while (todo) {
+    while (BUDGET && todo) {  // the full plies only, in order: a ballot over the flags, then the ranks
+        const int src_lane = __ffs(todo) - 1;
+        todo &= todo - 1;
+        const int len = __shfl_sync(FULL, copy_len, src_lane);
+        const long long dst = __shfl_sync(FULL, copy_dst, src_lane);
+        const size_t g0 = (size_t)(t - lane + src_lane) * MAX_PLIES;
+        long long rank = dst;
+        for (int q0 = 0; q0 < len; q0 += 32) {
+            const int q = q0 + lane;
+            const bool f = q < len && cp.g_full[g0 + q] != 0;
+            const unsigned m = __ballot_sync(FULL, f);
+            if (f) {
+                const long long d = rank + __popc(m & ((1u << lane) - 1u));
+                a.s_bb0[d] = a.g_bb0[g0 + q];
+                a.s_bb1[d] = a.g_bb1[g0 + q];
+                a.s_player[d] = a.g_player[g0 + q];
+#pragma unroll
+                for (int i = 0; i < 7; ++i) a.s_counts[d * 7 + i] = a.g_counts[(g0 + q) * 7 + i];
+            }
+            rank += __popc(m);
+        }
+    }
+    while (!BUDGET && todo) {
         const int src_lane = __ffs(todo) - 1;
         todo &= todo - 1;
         const int len = __shfl_sync(FULL, copy_len, src_lane);
@@ -1875,20 +1989,6 @@ __global__ void __launch_bounds__(256) k_reset_trees(Arena a, int n) {
 // underflow every component to 0.
 constexpr int NOISE_MAX_ATTEMPTS = 1 << 16;  // acceptance is >= 95 % per attempt: never reached in practice
 
-__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
-        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
-        c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
-        k.x += 0x9E3779B9u;
-        k.y += 0xBB67AE85u;
-    }
-    return c;
-}
-
-__device__ __forceinline__ double u01_open(uint32_t x) { return ((double)x + 0.5) * 0x1p-32; }  // (0, 1)
-
 // log of a Gamma(alpha, 1) variate
 __device__ double log_gamma_variate(double alpha, uint2 key, uint4 ctr) {
     const bool boost = alpha < 1.0;
@@ -1912,15 +2012,17 @@ __device__ double log_gamma_variate(double alpha, uint2 key, uint4 ctr) {
 
 // eight lanes per tree, lane c < 7 = column c.  Trees in error or without children (the first simulation did not expand the
 // root) are left alone; their η rows, and those of inactive slots, are 0.
+// BUDGET (az_set_playout_cap): fast searches (full[t] == 0, a trailing argument) get no noise either.
+template <bool BUDGET>
 __global__ void __launch_bounds__(256)
 k_root_noise(Arena a, int n_active, double alpha, float fraction, unsigned long long seed, long long slot_offset, uint32_t draw,
-             float *__restrict__ eta) {
+             float *__restrict__ eta, const uint8_t *full) {
     const int t = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 3);
     const int c = threadIdx.x & 7;
     const int tt = t < a.E ? t : 0;
     const size_t base = (size_t)tt * a.cap;
     const uint32_t cb = a.M[base].z;
-    const bool act = t < n_active && a.tree_err[tt] == 0 && cb != 0;
+    const bool act = t < n_active && a.tree_err[tt] == 0 && cb != 0 && (!BUDGET || full[tt] != 0);
     const uint32_t legal = act ? c4::legal_mask(a.root_bb0[tt] | a.root_bb1[tt]) : 0u;
     const bool mine = c < 7 && ((legal >> c) & 1u);
     double lg = -INFINITY;
@@ -2056,6 +2158,8 @@ struct az_engine {
     int reuse_v;               // az_set_subtree_reuse: max_root_visits V, 0 = off (the arena and the tables are sized for V, else for S)
     uint32_t *reroot;          // [E] played child for k_reroot (REROOT_NONE = nothing to keep); allocated with the first az_set_subtree_reuse
     unsigned long long *rstats;  // [E][RS_N] k_reroot's counters
+    bool cap_on;                 // az_set_playout_cap: self-play searches run to per-tree budgets (the BUDGET kernels)
+    CapArgs cap;                 // its arrays (allocated with the first az_set_playout_cap) and configuration, as the kernels take them
     int64_t bytes;
     int64_t launches;
     unsigned long long *d_tot;   // [16] stats totals (device)
@@ -2153,6 +2257,13 @@ int launch_encode(az_engine *h, const uint64_t *bb0, const uint64_t *bb1, const 
         default: k_encode<AZ_LAYOUT_PLANES_BF16_NHWC><<<blocks, B, smem, st>>>(bb0, bb1, player, status, n, o); break;
     }
     AZ_LAUNCH_CHECK(h, "k_encode");
+    return AZ_OK;
+}
+
+// the playout cap's flags and budgets of every slot for move step `step`, from the roots as they are (all_full: every search full)
+int launch_cap_draw(az_engine *h, uint32_t step, bool all_full, cudaStream_t st) {
+    k_cap_draw<<<blocks_for(h->a.E, 256), 256, 0, st>>>(h->a, h->a.E, h->cap, step, all_full ? 1 : 0);
+    AZ_LAUNCH_CHECK(h, "k_cap_draw");
     return AZ_OK;
 }
 
@@ -2414,6 +2525,8 @@ int32_t az_reset_games(az_engine *h, uint64_t init_bb0, uint64_t init_bb1, int32
     k_set_roots<<<blocks_for(E, 256), 256, 0, S(stream)>>>(h->a, nullptr, nullptr, nullptr, init_bb0, init_bb1, init_player,
                                                           E, 1);
     AZ_LAUNCH_CHECK(h, "k_set_roots");
+    if (h->cap_on)
+        if (int rc = launch_cap_draw(h, 0u, false, S(stream))) return rc;
     AZ_CUDA(h, cudaMemsetAsync(h->rings[0].ring, 0, 4 * sizeof(unsigned long long), S(stream)));
     AZ_CUDA(h, cudaMemsetAsync(h->rings[1].ring, 0, 4 * sizeof(unsigned long long), S(stream)));
     h->init0 = init_bb0;
@@ -2435,6 +2548,8 @@ int32_t az_set_roots(az_engine *h, const uint64_t *bb0, const uint64_t *bb1, con
     if (int rc = set_device(h)) return rc;
     k_set_roots<<<blocks_for(n, 256), 256, 0, S(stream)>>>(h->a, bb0, bb1, player, 0ull, 0ull, 0, n, 0);
     AZ_LAUNCH_CHECK(h, "k_set_roots");
+    if (h->cap_on)  // not a self-play move step: every search is full
+        if (int rc = launch_cap_draw(h, 0u, true, S(stream))) return rc;
     h->n_active = n;
     h->sims_done = 0;
     h->noise_applied = false;
@@ -2477,8 +2592,9 @@ int32_t az_run_move_step(az_engine *h, int32_t num_sims, int32_t eval_kind, cons
     if (!uniforms) return fail(h, AZ_E_INVALID, "%s", "az_run_move_step: null uniforms");
     if (!h->have_init) return fail(h, AZ_E_STATE, "%s", "az_run_move_step: call az_reset_games first");
     if (num_sims < 1) return fail(h, AZ_E_INVALID, "%s", "az_run_move_step: num_sims < 1");
-    // the greedy rule and subtree reuse live in k_sample_moves (+ k_reroot) only: the search (its hot prefix written back), then the move
-    if (h->greedy_from >= 0 || h->reuse_v > 0) {
+    // the greedy rule, subtree reuse and the playout cap live in k_sample_moves (+ k_reroot) only: the search (its hot prefix written
+    // back), then the move
+    if (h->greedy_from >= 0 || h->reuse_v > 0 || h->cap_on) {
         const int32_t rc = run_sims_impl(h, num_sims, eval_kind, nullptr, nullptr, false, stream);
         if (rc != AZ_OK) return rc;
         return az_sample_moves(h, uniforms, finished, stream);
@@ -2534,20 +2650,22 @@ static int32_t run_sims_impl(az_engine *h, int32_t num_sims, int32_t eval_kind, 
     mv.init1 = h->init1;
     mv.step = h->step;
     mv.initpl = h->initpl;
-#define AZ_RUN3(TPW_, EV_, LAT_, MOVE_, TSM_)                                                                                               \
-    do {                                                                                                                                    \
-        AZ_CUDA(h, cudaFuncSetAttribute(k_run_sims<TPW_, EV_, LAT_, MOVE_, TSM_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        k_run_sims<TPW_, EV_, LAT_, MOVE_, TSM_><<<blocks, 64, smem, S(stream)>>>(h->a, n, num_sims, c, K, mv);                             \
+    const bool budget = h->cap_on;  // never with `move`: az_run_move_step leaves the move to k_sample_moves then
+#define AZ_RUN3(TPW_, EV_, LAT_, MOVE_, TSM_, BUD_)                                                                                               \
+    do {                                                                                                                                          \
+        AZ_CUDA(h, cudaFuncSetAttribute(k_run_sims<TPW_, EV_, LAT_, MOVE_, TSM_, BUD_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+        k_run_sims<TPW_, EV_, LAT_, MOVE_, TSM_, BUD_><<<blocks, 64, smem, S(stream)>>>(h->a, n, num_sims, c, K, mv, h->cap.budget);            \
     } while (0)
-#define AZ_RUN2(TPW_, EV_, LAT_, MOVE_)                       \
-    do {                                                      \
-        if (tabs_in_smem) AZ_RUN3(TPW_, EV_, LAT_, MOVE_, true); \
-        else AZ_RUN3(TPW_, EV_, LAT_, MOVE_, false);          \
+#define AZ_RUN2(TPW_, EV_, LAT_, MOVE_, BUD_)                       \
+    do {                                                            \
+        if (tabs_in_smem) AZ_RUN3(TPW_, EV_, LAT_, MOVE_, true, BUD_); \
+        else AZ_RUN3(TPW_, EV_, LAT_, MOVE_, false, BUD_);          \
     } while (0)
-#define AZ_RUN1(TPW_, EV_, LAT_)                  \
-    do {                                          \
-        if (move) AZ_RUN2(TPW_, EV_, LAT_, true); \
-        else AZ_RUN2(TPW_, EV_, LAT_, false);     \
+#define AZ_RUN1(TPW_, EV_, LAT_)                           \
+    do {                                                   \
+        if (move) AZ_RUN2(TPW_, EV_, LAT_, true, false);   \
+        else if (budget) AZ_RUN2(TPW_, EV_, LAT_, false, true); \
+        else AZ_RUN2(TPW_, EV_, LAT_, false, false);       \
     } while (0)
 #define AZ_RUN(TPW_, EV_)                  \
     do {                                   \
@@ -2585,15 +2703,21 @@ int32_t az_select_leaves(az_engine *h, void *stream) {
     const bool lat = latency_variant(h, blocks_for(n, tpb));
     const bool cache = cache_active(h);
     const bool sym = h->sym;
-#define AZ_SEL2(TPW_, SYM_)                                                                                                 \
-    do {                                                                                                                    \
-        if (cache) {                                                                                                        \
-            if (lat) k_select<TPW_, true, true, SYM_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror);    \
-            else k_select<TPW_, false, true, SYM_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror);       \
-        } else {                                                                                                            \
-            if (lat) k_select<TPW_, true, false, SYM_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror);   \
-            else k_select<TPW_, false, false, SYM_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror);      \
-        }                                                                                                                   \
+    const bool budget = h->cap_on;
+#define AZ_SEL3(TPW_, SYM_, BUD_)                                                                                                        \
+    do {                                                                                                                                 \
+        if (cache) {                                                                                                                     \
+            if (lat) k_select<TPW_, true, true, SYM_, BUD_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);  \
+            else k_select<TPW_, false, true, SYM_, BUD_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);     \
+        } else {                                                                                                                         \
+            if (lat) k_select<TPW_, true, false, SYM_, BUD_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror, h->cap.budget); \
+            else k_select<TPW_, false, false, SYM_, BUD_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);    \
+        }                                                                                                                                \
+    } while (0)
+#define AZ_SEL2(TPW_, SYM_)                        \
+    do {                                           \
+        if (budget) AZ_SEL3(TPW_, SYM_, true);     \
+        else AZ_SEL3(TPW_, SYM_, false);           \
     } while (0)
 #define AZ_SEL(TPW_)                      \
     do {                                  \
@@ -2605,6 +2729,7 @@ int32_t az_select_leaves(az_engine *h, void *stream) {
     else AZ_SEL(4);
 #undef AZ_SEL
 #undef AZ_SEL2
+#undef AZ_SEL3
     AZ_LAUNCH_CHECK(h, "k_select");
     h->compact_valid = h->compact != 0;
     if (h->compact) {
@@ -2674,10 +2799,16 @@ int32_t az_expand_backup_select(az_engine *h, const float *policy, const float *
     if (h->sel_pending && h->cache_sel != cache)
         return fail(h, AZ_E_STATE, "%s", "az_expand_backup_select: the evaluation cache or leaf compaction changed between a selection and its expansion");
     const bool sym = h->sym;  // az_set_symmetric_eval refuses while a selection is pending: the expansion matches its selection
-#define AZ_ES3(TPW_, LAT_, CMP_, SYM_)                                                                                                      \
+    const bool budget = h->cap_on;
+#define AZ_ES4(TPW_, LAT_, CMP_, SYM_, BUD_)                                                                                                \
     do {                                                                                                                              \
-        if (cache) k_expand_select<TPW_, LAT_, CMP_, true, SYM_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct, h->leaf_mirror);  \
-        else k_expand_select<TPW_, LAT_, CMP_, false, SYM_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct, h->leaf_mirror);  \
+        if (cache) k_expand_select<TPW_, LAT_, CMP_, true, SYM_, BUD_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);  \
+        else k_expand_select<TPW_, LAT_, CMP_, false, SYM_, BUD_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);  \
+    } while (0)
+#define AZ_ES3(TPW_, LAT_, CMP_, SYM_)                   \
+    do {                                                 \
+        if (budget) AZ_ES4(TPW_, LAT_, CMP_, SYM_, true); \
+        else AZ_ES4(TPW_, LAT_, CMP_, SYM_, false);      \
     } while (0)
 #define AZ_ES2(TPW_, LAT_, CMP_)                     \
     do {                                             \
@@ -2700,6 +2831,7 @@ int32_t az_expand_backup_select(az_engine *h, const float *policy, const float *
 #undef AZ_ES
 #undef AZ_ES2
 #undef AZ_ES3
+#undef AZ_ES4
     AZ_LAUNCH_CHECK(h, "k_expand_select");
     h->compact_valid = h->compact != 0;
     if (h->compact == 1) {
@@ -2789,24 +2921,30 @@ int32_t az_sample_moves(az_engine *h, const double *uniforms, uint8_t *finished,
     if (int rc = set_device(h)) return rc;
     const int n = h->n_active;
     const bool reuse = h->reuse_v > 0;
+    const bool budget = h->cap_on;
+#define AZ_SM2(G_, R_, B_)                                                                                                         \
+    k_sample_moves<G_, R_, B_><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0, h->init1, \
+                                                                        h->initpl, G_ ? h->greedy_from : -1, R_ ? h->reroot : nullptr, h->cap)
+#define AZ_SM(G_, R_)                  \
+    do {                               \
+        if (budget) AZ_SM2(G_, R_, true); \
+        else AZ_SM2(G_, R_, false);    \
+    } while (0)
     if (h->greedy_from >= 0) {
-        if (reuse)
-            k_sample_moves<true, true><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0,
-                                                                                 h->init1, h->initpl, h->greedy_from, h->reroot);
-        else
-            k_sample_moves<true, false><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0,
-                                                                                  h->init1, h->initpl, h->greedy_from, nullptr);
+        if (reuse) AZ_SM(true, true);
+        else AZ_SM(true, false);
     } else {
-        if (reuse)
-            k_sample_moves<false, true><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0,
-                                                                                  h->init1, h->initpl, -1, h->reroot);
-        else
-            k_sample_moves<false, false><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0,
-                                                                                   h->init1, h->initpl, -1, nullptr);
+        if (reuse) AZ_SM(false, true);
+        else AZ_SM(false, false);
     }
+#undef AZ_SM
+#undef AZ_SM2
     AZ_LAUNCH_CHECK(h, "k_sample_moves");
-    if (reuse)
+    if (reuse) {
         if (int rc = launch_reroot(h, n, S(stream))) return rc;
+        if (budget)  // the next search's budget counts from the visits the new root kept
+            if (int rc = launch_cap_draw(h, (uint32_t)h->step + 1u, false, S(stream))) return rc;
+    }
     h->step++;
     h->sims_done = 0;
     h->noise_applied = false;
@@ -2850,9 +2988,14 @@ int32_t az_apply_root_noise(az_engine *h, void *stream) {
     if (cap != cudaStreamCaptureStatusNone)
         return fail(h, AZ_E_STATE, "%s", "az_apply_root_noise: not inside a CUDA graph capture (the draw number is a launch argument)");
     const int E = h->a.E;
-    k_root_noise<<<blocks_for((long long)E * 8, 256), 256, 0, S(stream)>>>(h->a, h->n_active, h->noise_alpha, h->noise_fraction,
-                                                                          h->noise_seed, h->noise_slot_offset, h->noise_draws,
-                                                                          h->noise_eta);
+    if (h->cap_on)
+        k_root_noise<true><<<blocks_for((long long)E * 8, 256), 256, 0, S(stream)>>>(h->a, h->n_active, h->noise_alpha, h->noise_fraction,
+                                                                                    h->noise_seed, h->noise_slot_offset, h->noise_draws,
+                                                                                    h->noise_eta, h->cap.full);
+    else
+        k_root_noise<false><<<blocks_for((long long)E * 8, 256), 256, 0, S(stream)>>>(h->a, h->n_active, h->noise_alpha, h->noise_fraction,
+                                                                                     h->noise_seed, h->noise_slot_offset, h->noise_draws,
+                                                                                     h->noise_eta, nullptr);
     AZ_LAUNCH_CHECK(h, "k_root_noise");
     h->noise_draws++;
     h->noise_applied = true;
@@ -3054,6 +3197,7 @@ int32_t az_reset_stats(az_engine *h, void *stream) {
     AZ_LAUNCH_CHECK(h, "k_zero_u32");
     memset(h->acc_tot, 0, sizeof h->acc_tot);
     if (h->rstats) AZ_CUDA(h, cudaMemsetAsync(h->rstats, 0, (size_t)h->a.E * RS_N * sizeof(unsigned long long), S(stream)));
+    if (h->cap.cstats) AZ_CUDA(h, cudaMemsetAsync(h->cap.cstats, 0, (size_t)h->a.E * CS_N * sizeof(unsigned long long), S(stream)));
     return AZ_OK;
 }
 
@@ -3122,6 +3266,8 @@ int32_t az_set_subtree_reuse(az_engine *h, int32_t max_root_visits) {
     }
     k_reset_trees<<<blocks_for(E, 256), 256>>>(a, E);
     AZ_LAUNCH_CHECK(h, "k_reset_trees");
+    if (h->cap_on)  // the budgets of the current step count from the reset roots
+        if (int rc2 = launch_cap_draw(h, (uint32_t)h->step, false, nullptr)) return rc2;
     AZ_CUDA(h, cudaDeviceSynchronize());
     h->reuse_v = max_root_visits;
     h->sims_done = 0;
@@ -3139,6 +3285,8 @@ int32_t az_advance_roots(az_engine *h, const uint8_t *cols, uint8_t *out_status,
     k_advance_roots<<<blocks_for(n, 256), 256, 0, S(stream)>>>(h->a, n, cols, out_status, h->reroot);
     AZ_LAUNCH_CHECK(h, "k_advance_roots");
     if (int rc = launch_reroot(h, n, S(stream))) return rc;
+    if (h->cap_on)  // not a self-play move step: every search is full
+        if (int rc = launch_cap_draw(h, 0u, true, S(stream))) return rc;
     h->sims_done = 0;
     h->noise_applied = false;
     return AZ_OK;
@@ -3166,6 +3314,93 @@ int32_t az_get_reuse_stats(az_engine *h, az_reuse_stats *out, void *stream) {
     out->dropped = tot[RS_DROPPED];
     out->nodes = tot[RS_NODES];
     out->visits = tot[RS_VISITS];
+    return AZ_OK;
+}
+
+int32_t az_set_playout_cap(az_engine *h, const az_playout_cap *cfg) {
+    if (!h) return AZ_E_INVALID;
+    if (h->sel_pending) return fail(h, AZ_E_STATE, "%s", "az_set_playout_cap: a selection's leaves wait for their expansion");
+    if (!cfg) {
+        h->cap_on = false;
+        return AZ_OK;
+    }
+    const int S_ = h->cfg.num_simulations;
+    if (cfg->fast_sims < 1 || cfg->fast_sims > S_)
+        return fail(h, AZ_E_INVALID, "%s", "az_set_playout_cap: fast_sims must be in [1, num_simulations]");
+    if (!(cfg->p_full >= 0.0f && cfg->p_full <= 1.0f)) return fail(h, AZ_E_INVALID, "%s", "az_set_playout_cap: p_full must be in [0, 1]");
+    if (cfg->slot_offset < 0 || cfg->slot_offset > ((int64_t)1 << 62))
+        return fail(h, AZ_E_INVALID, "%s", "az_set_playout_cap: slot_offset must be in [0, 2^62]");
+    if (cfg->visit_budget != 0 && cfg->visit_budget != 1) return fail(h, AZ_E_INVALID, "%s", "az_set_playout_cap: visit_budget must be 0 or 1");
+    if (int rc = set_device(h)) return rc;
+    const int E = h->a.E;
+    CapArgs &cp = h->cap;
+    if (!cp.budget) {
+        uint32_t *budget = nullptr;
+        uint8_t *full = nullptr, *g_full = nullptr;
+        unsigned long long *cstats = nullptr;
+        int rc = dev_alloc(h, &budget, E);
+        if (rc == AZ_OK) rc = dev_alloc(h, &full, E);
+        if (rc == AZ_OK) rc = dev_alloc(h, &g_full, (size_t)E * MAX_PLIES);
+        if (rc == AZ_OK) rc = dev_alloc(h, &cstats, (size_t)E * CS_N);
+        if (rc != AZ_OK) {
+            if (budget) dev_free(h, budget, (size_t)E * sizeof(uint32_t));
+            if (full) dev_free(h, full, (size_t)E);
+            if (g_full) dev_free(h, g_full, (size_t)E * MAX_PLIES);
+            return rc;
+        }
+        AZ_CUDA(h, cudaMemset(cstats, 0, (size_t)E * CS_N * sizeof(unsigned long long)));
+        cp.budget = budget;
+        cp.full = full;
+        cp.g_full = g_full;
+        cp.cstats = cstats;
+    }
+    // the flags apply only while the mode is on: every ply already in the logs counts as full (az_engine.h)
+    if (!h->cap_on) AZ_CUDA(h, cudaMemset(cp.g_full, 1, (size_t)E * MAX_PLIES));
+    cp.seed = cfg->seed;
+    cp.slot_offset = cfg->slot_offset;
+    cp.p_full = (double)cfg->p_full;
+    cp.S = S_;
+    cp.fast = cfg->fast_sims;
+    cp.visit_budget = cfg->visit_budget;
+    h->cap_on = true;
+    if (int rc = launch_cap_draw(h, (uint32_t)h->step, false, nullptr)) return rc;
+    AZ_CUDA(h, cudaDeviceSynchronize());
+    return AZ_OK;
+}
+
+int32_t az_search_budgets(az_engine *h, uint32_t *budget, uint8_t *full, void *stream) {
+    if (!h) return AZ_E_INVALID;
+    if (!h->cap.budget) return fail(h, AZ_E_STATE, "%s", "az_search_budgets: no playout cap configured (az_set_playout_cap)");
+    if (int rc = set_device(h)) return rc;
+    const size_t E = (size_t)h->a.E;
+    if (budget) AZ_CUDA(h, cudaMemcpyAsync(budget, h->cap.budget, E * sizeof(uint32_t), cudaMemcpyDefault, S(stream)));
+    if (full) AZ_CUDA(h, cudaMemcpyAsync(full, h->cap.full, E, cudaMemcpyDefault, S(stream)));
+    return AZ_OK;
+}
+
+int32_t az_get_cap_stats(az_engine *h, az_cap_stats *out, void *stream) {
+    if (!h || !out) return AZ_E_INVALID;
+    memset(out, 0, sizeof *out);
+    unsigned long long r[NSTAT];
+    if (int rc = sum_stats(h, r, S(stream))) return rc;
+    out->simulations = r[0];
+    if (!h->cap.cstats) return AZ_OK;
+    const size_t n = (size_t)h->a.E * CS_N;
+    unsigned long long *buf = (unsigned long long *)malloc(n * sizeof(unsigned long long));
+    if (!buf) return fail(h, AZ_E_NOMEM, "%s", "az_get_cap_stats: host allocation failed");
+    cudaError_t e = cudaMemcpyAsync(buf, h->cap.cstats, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, S(stream));
+    if (e == cudaSuccess) e = cudaStreamSynchronize(S(stream));
+    if (e != cudaSuccess) {
+        free(buf);
+        return fail(h, AZ_E_CUDA, "az_get_cap_stats: %s", cudaGetErrorString(e));
+    }
+    unsigned long long tot[CS_N] = {};
+    for (size_t i = 0; i < n; ++i) tot[i % CS_N] += buf[i];
+    free(buf);
+    out->full_searches = tot[CS_FULL];
+    out->fast_searches = tot[CS_FAST];
+    out->samples_recorded = tot[CS_RECORDED];
+    out->samples_dropped = tot[CS_DROPPED];
     return AZ_OK;
 }
 

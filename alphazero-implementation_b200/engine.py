@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import AzConfig, AzEvalCacheStats, AzReuseStats, AzRootNoise, AzStats
+from ._lib import AzCapStats, AzConfig, AzEvalCacheStats, AzPlayoutCap, AzReuseStats, AzRootNoise, AzStats
 
 EVAL_UNIFORM = 1
 EVAL_HASH = 2
@@ -100,6 +100,7 @@ class Engine:
         self.greedy_from = -1
         self.symmetric_eval = False
         self.subtree_reuse = 0  # max_root_visits, 0 = off
+        self.playout_cap = None  # (fast_sims, p_full, seed, slot_offset, visit_budget) while the playout cap is on
         self.tree_capacity = self.lib.az_tree_capacity(self.h)
 
     # -- plumbing --------------------------------------------------------------------------------
@@ -308,6 +309,37 @@ class Engine:
         st = AzReuseStats()
         self._check(self.lib.az_get_reuse_stats(self.h, C.byref(st), _stream()), "az_get_reuse_stats")
         return {n: int(getattr(st, n)) for n, _ in AzReuseStats._fields_}
+
+    def set_playout_cap(self, fast_sims: int | None, p_full: float = 0.25, seed: int = 0, slot_offset: int = 0,
+                        visit_budget: bool = False):
+        """Playout cap randomization (`az_set_playout_cap`, KataGo): each self-play search (after `reset_games` and every
+        `sample_moves`) is full with probability `p_full` (num_simulations new simulations) or fast (`fast_sims`); a tree that has run
+        its share is idle for the rest of the move step.  Only full searches become samples of the finished games (an episode may
+        then have none).  Fast searches get no root noise.  `visit_budget`: a search tops the root up to that many visits instead
+        (at least one new simulation; for subtree reuse).  The draw is a function of (seed, slot_offset + slot, move step) alone.
+        `fast_sims=None` = off (the default).  Call it before a CUDA graph of the search is captured."""
+        if fast_sims is None:
+            self._check(self.lib.az_set_playout_cap(self.h, None), "az_set_playout_cap")
+            self.playout_cap = None
+            return
+        cfg = AzPlayoutCap(int(fast_sims), float(p_full), int(seed) & (2**64 - 1), int(slot_offset), 1 if visit_budget else 0)
+        self._check(self.lib.az_set_playout_cap(self.h, C.byref(cfg)), "az_set_playout_cap")
+        self.playout_cap = (int(fast_sims), float(p_full), int(seed), int(slot_offset), bool(visit_budget))
+
+    def search_budgets(self) -> tuple[torch.Tensor, torch.Tensor]:
+        """The playout cap's current draw -> (budget int64 [num_games]: the root visit count at which each tree stops, full u8
+        [num_games]: 1 = full search)."""
+        b = self.empty(self.num_games, torch.int32)
+        f = self.empty(self.num_games, torch.uint8)
+        self._check(self.lib.az_search_budgets(self.h, _ptr(b), _ptr(f), _stream()), "az_search_budgets")
+        return b.to(torch.int64) & 0xFFFFFFFF, f
+
+    def cap_stats(self) -> dict:
+        """Self-play searches by kind (full / fast), samples of finished games recorded / dropped, and the new simulations run -
+        totals since creation / `reset_stats`."""
+        st = AzCapStats()
+        self._check(self.lib.az_get_cap_stats(self.h, C.byref(st), _stream()), "az_get_cap_stats")
+        return {n: int(getattr(st, n)) for n, _ in AzCapStats._fields_}
 
     def run_simulations(self, num_sims: int, eval_kind: int):
         self._check(self.lib.az_run_simulations(self.h, int(num_sims), int(eval_kind), _stream()), "az_run_simulations")

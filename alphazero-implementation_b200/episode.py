@@ -74,10 +74,11 @@ def episodes_from_batch(batch, num_simulations: int) -> list[Episode]:
     from .game import DEFAULT_CONFIG, rules_engine
 
     out = []
-    if batch.num_samples == 0:
+    if len(batch) == 0:
         return out
-    # State.actions of every sample position from the rules kernel, one call for the whole batch
-    legal_all = rules_engine().state_info(batch.s_bb0, batch.s_bb1)["legal"].cpu().numpy()
+    # State.actions of every sample position from the rules kernel, one call for the whole batch (an episode of a game whose
+    # searches were all fast under `AlphaZeroSearch(playout_cap=)` has no samples: it is still an episode)
+    legal_all = rules_engine().state_info(batch.s_bb0, batch.s_bb1)["legal"].cpu().numpy() if batch.num_samples else None
     for e in range(len(batch)):
         o, n = int(batch.ep_offset[e]), int(batch.ep_len[e])
         value = [float(batch.ep_outcome[e, 0]), float(batch.ep_outcome[e, 1])]

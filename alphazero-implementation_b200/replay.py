@@ -65,7 +65,8 @@ class ReplayBuffer:
 
     def extend(self, batch: EpisodeBatch | dict):
         """Append finished episodes in order (`buffer.append(episode)`, datamodule.py:29-30); the deque keeps the last
-        `buffer_size` of them.  Episodes must be stored with their samples back to back in episode order."""
+        `buffer_size` of them.  Episodes must be stored with their samples back to back in episode order.  `buffer_size` counts
+        episodes, empty ones included (an episode of `AlphaZeroSearch(playout_cap=)` self-play may have no samples)."""
         if isinstance(batch, EpisodeBatch):
             d = dict(ep_len=batch.ep_len, ep_offset=batch.ep_offset, ep_outcome=batch.ep_outcome, s_bb0=batch.s_bb0.view(np.int64),
                      s_bb1=batch.s_bb1.view(np.int64), s_player=batch.s_player, s_counts=batch.s_counts)

@@ -92,6 +92,22 @@ class RootNoise:
     slot_offset: int = 0
 
 
+@dataclass(frozen=True)
+class PlayoutCap:
+    """Playout cap randomization of the self-play searches (KataGo; `Engine.set_playout_cap`): each search of a move step is full
+    with probability `full_probability` (num_simulations new simulations) or fast (`fast_simulations`).  Every move is played, but
+    only the full searches become training samples, so a game costs fewer simulations while the policy targets keep the full
+    search's depth.  Fast searches get no root noise.  `visit_budget` (with subtree reuse): a search tops the root up to that many
+    visits instead of adding them, at least one new simulation.  The draws are a function of (seed, slot_offset + slot, move step)
+    only.  Off (None) by default."""
+
+    fast_simulations: int
+    full_probability: float = 0.25
+    seed: int = 0
+    slot_offset: int = 0
+    visit_budget: bool = False
+
+
 class _GraphedStep:
     """The simulation loop of the network-in-the-loop path, optionally replayed as a CUDA graph.
 
@@ -199,7 +215,8 @@ class AlphaZeroSearch:
     def __init__(self, *, model, num_simulations: int, exploration_weight: float = 1.0, device: int | None = None,
                  lanes_per_tree: int = 0, inference_dtype: torch.dtype | None = None, use_cuda_graph: bool = True,
                  use_tensor_core_kernels: bool = True, trunk_variant: int | None = None, eval_cache: bool | int = True,
-                 root_noise: RootNoise | None = None, symmetric: bool = False, subtree_reuse: bool | int = False):
+                 root_noise: RootNoise | None = None, symmetric: bool = False, subtree_reuse: bool | int = False,
+                 playout_cap: PlayoutCap | None = None):
         """`eval_cache`: serve repeated leaf positions from the engine's evaluation cache (`Engine.set_eval_cache`) when the
         evaluator's outputs depend on the position alone (`InferenceNet.position_only_outputs`); same results, fewer evaluator rows.
         True = a table sized for the engine, False = off, an int = log2 of its entry count.
@@ -212,8 +229,11 @@ class AlphaZeroSearch:
         with all its statistics (AlphaGo Zero), as long as N(child) + num_simulations <= max_root_visits (`Engine.set_subtree_reuse`);
         each search still runs num_simulations new simulations, so a root then holds more visits.  True = max_root_visits of
         4 num_simulations, an int = max_root_visits, False (default) = every move step starts from a fresh root, as the reference
-        does.  `run_simulations(nodes)` always starts from the given fresh roots."""
+        does.  `run_simulations(nodes)` always starts from the given fresh roots.
+        `playout_cap`: the self-play move steps run full or fast searches (`PlayoutCap`) and record only the full ones as samples;
+        None (default) = every search is full.  `run_simulations(nodes)` always runs full searches."""
         self.symmetric = bool(symmetric)
+        self.playout_cap = playout_cap
         self.subtree_reuse = subtree_reuse
         self.inference_model = model.get_inference_clone()
         self.eval_cache = eval_cache
@@ -299,14 +319,16 @@ class AlphaZeroSearch:
         noise = 1 if self.root_noise is not None else 0
         greedy = self._engine is not None and self._engine.greedy_from >= 0
         reuse = 1 if self.max_root_visits else 0  # k_reroot after k_sample_moves
+        cap = self.playout_cap is not None
+        redraw = 1 if cap and reuse else 0  # k_cap_draw after k_reroot (without reuse k_sample_moves draws the next budgets itself)
         if self._mode == "builtin":
-            # one k_run_sims per run, the last one with the move fused in - unless the greedy cutoff, subtree reuse (or a search of one
-            # simulation with noise) leaves the move to k_sample_moves
-            return len(runs) + noise + (1 if greedy or reuse or noise and S == 1 else 0) + reuse
+            # one k_run_sims per run, the last one with the move fused in - unless the greedy cutoff, subtree reuse, the playout cap (or
+            # a search of one simulation with noise) leaves the move to k_sample_moves
+            return len(runs) + noise + (1 if greedy or reuse or cap or noise and S == 1 else 0) + reuse + redraw
         # per run of n: k_select; n - 1 x (evaluator or gather, k_expand_select); evaluator, k_expand_backup.  Then k_root_noise
         # between the runs and k_sample_moves.  When the evaluator walks the compacted leaf list: one k_compact_leaves after
         # every k_select (the later lists come out of k_expand_select) or, AZ_COMPACT_FUSED=0, one per selection
-        n = sum(2 * r + 1 for r in runs) + noise + 1 + reuse
+        n = sum(2 * r + 1 for r in runs) + noise + 1 + reuse + redraw
         if not getattr(self._net, "wants_leaf_compaction", False):
             return n
         return n + (len(runs) if os.environ.get("AZ_COMPACT_FUSED", "1") != "0" else S)
@@ -334,6 +356,21 @@ class AlphaZeroSearch:
             engine.set_subtree_reuse(v)
             if self._graphed is not None and self._graphed.engine is engine:
                 self._graphed = None
+
+    def _configure_cap(self, engine: Engine):
+        """before the move step's search and any capture of its CUDA graph (switching the cap on or off changes the kernels)"""
+        pc = self.playout_cap
+        want = None if pc is None else (int(pc.fast_simulations), float(pc.full_probability), int(pc.seed), int(pc.slot_offset),
+                                        bool(pc.visit_budget))
+        if engine.playout_cap == want:
+            return
+        switched = (engine.playout_cap is None) != (want is None)
+        if want is None:
+            engine.set_playout_cap(None)
+        else:
+            engine.set_playout_cap(*want)
+        if switched and self._graphed is not None and self._graphed.engine is engine:
+            self._graphed = None
 
     def close(self):
         if self._engine is not None:
@@ -384,6 +421,7 @@ class AlphaZeroSearch:
         one launch (`az_run_move_step`), with identical results.  With `subtree_reuse`, the move keeps the played child's subtree
         (`k_reroot`) for the next step's search."""
         self._configure_reuse(engine)
+        self._configure_cap(engine)
         if self._mode == "builtin":
             kind = self.inference_model.az_builtin_eval_kind
             self._configure_noise(engine)

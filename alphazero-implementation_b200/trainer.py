@@ -150,7 +150,7 @@ class Trainer:
               overlap: bool = True, inference_dtype: torch.dtype | None = None, precision: str = "32-true",
               cuda_graph: bool = True, trainer_share: float | None = None, save_dir: str | None = None, root_noise=None,
               sampling_moves: int | None = None, symmetric: bool = False, mirror_augment: bool = False,
-              subtree_reuse: bool | int = False):
+              subtree_reuse: bool | int = False, playout_cap=None):
         """`overlap=True` reproduces the reference's pipeline (datamodule.py:89-101): the self-play of iteration k+1 runs on a
         background thread (own CUDA stream, weights as of the end of iteration k-1's training) while iteration k trains.
         `precision`: "32-true" (the reference's Lightning default) or "bf16-mixed" (forward / backward under bf16 autocast,
@@ -169,7 +169,9 @@ class Trainer:
         image (`_GraphedTraining`).  Both off by default.
         `subtree_reuse`: each self-play move keeps the played child's subtree for the next search (`AlphaZeroSearch(subtree_reuse=)`:
         True = max_root_visits of 4 simulations_per_episode, an int = max_root_visits); off by default.  The replay buffer then divides
-        each sample's visit counts by their sum (`ReplayBuffer(subtree_reuse=True)`)."""
+        each sample's visit counts by their sum (`ReplayBuffer(subtree_reuse=True)`).
+        `playout_cap` (`search.PlayoutCap`): most self-play moves get a fast search and only the full searches become samples
+        (`AlphaZeroSearch(playout_cap=)`); off by default.  Like `root_noise`, its `slot_offset` is set to the rank's first game."""
         import threading
 
         world = dist.get_world_size() if dist.is_initialized() else 1
@@ -189,6 +191,8 @@ class Trainer:
             kw["symmetric"] = True
         if subtree_reuse:
             kw["subtree_reuse"] = subtree_reuse
+        if playout_cap is not None:
+            kw["playout_cap"] = dataclasses.replace(playout_cap, slot_offset=lo)
         gen = EpisodeGenerator(model=model, num_simulations=simulations_per_episode, num_episodes=hi - lo,
                                game_initial_state=initial_state, device=self.device_index, sampling_moves=sampling_moves, **kw)
         replay = ReplayBuffer(buffer_size, simulations_per_episode, self.device, subtree_reuse="subtree_reuse" in kw)

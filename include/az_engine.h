@@ -310,6 +310,44 @@ typedef struct az_reuse_stats {
 /* totals since az_create / az_reset_stats over moves from a searched root that did not end the game.  Synchronises. */
 int32_t az_get_reuse_stats(az_engine *h, az_reuse_stats *out_host, void *stream);
 
+/* Playout cap randomization (KataGo): the searches of the self-play move steps (after az_reset_games and after every
+ * az_sample_moves) are each "full" with probability p_full, else "fast".  A full search runs num_simulations new simulations,
+ * a fast one fast_sims; a tree that has run its share is idle for the rest of the move step (no leaf, no evaluator row, no cache
+ * probe), so a step costs fewer evaluator rows.  Every move is played and logged as before, but a finished game emits only the
+ * samples of its full searches, in order: ep_len counts them and may be 0 (the episode is still emitted, with its outcome).
+ * Fast searches get no root noise (their η row is 0).
+ *   visit_budget = 1 (for subtree reuse): a search tops the root up to num_simulations (fast_sims) visits instead, at least one
+ *   new simulation: n = max(S_t - N_start, 1).  With reuse off N_start = 0 and this is the plain cap.
+ * The flag of (slot, move step) is a function of (seed, slot_offset + slot, step) alone: Philox4x32-10 keyed by the seed, counter
+ * {global slot lo, hi, step, 0xC0000000}, full iff (x + 0.5) / 2^32 < p_full in fp64 - sharded self-play draws what the
+ * unsharded run draws.  az_set_roots and az_advance_roots make every search full with S new simulations, visit_budget or not:
+ * they are not self-play.  The budgets live in device memory, so a captured simulation graph stays valid from move to move;
+ * switching the mode on or off changes the kernels a launch uses (capture after it).  The flags of the game logs apply only while
+ * the mode is on: with it off a finished game emits every ply, and switching it on counts every ply already in the logs as full -
+ * also a fast ply of an earlier period with the mode on, which its game would have emitted had it ended while the mode was off. */
+typedef struct az_playout_cap {
+    int32_t fast_sims;     /* new simulations of a fast search, 1 .. num_simulations */
+    float p_full;          /* probability of a full search, [0, 1] */
+    uint64_t seed;
+    int64_t slot_offset;   /* global index of this engine's slot 0, [0, 2^62] */
+    int32_t visit_budget;  /* 0 or 1 */
+} az_playout_cap;
+/* cfg NULL = off (the default).  Draws the flags and budgets of the current roots (synchronises).  AZ_E_INVALID for values out
+ * of range, AZ_E_STATE while a selection's leaves wait for their expansion. */
+int32_t az_set_playout_cap(az_engine *h, const az_playout_cap *cfg);
+/* the current draw: budget[num_games] u32 = the root visit count at which each tree stops (N_start + n), full[num_games] u8;
+ * device or pinned host memory, either may be NULL.  AZ_E_STATE before the first az_set_playout_cap. */
+int32_t az_search_budgets(az_engine *h, uint32_t *budget, uint8_t *full, void *stream);
+typedef struct az_cap_stats {
+    uint64_t full_searches;     /* self-play searches that ended in a move, by kind */
+    uint64_t fast_searches;
+    uint64_t samples_recorded;  /* samples of finished games emitted / left out (fast searches) */
+    uint64_t samples_dropped;
+    uint64_t simulations;       /* new simulations actually run (az_stats.simulations) */
+} az_cap_stats;
+/* totals since az_create / az_reset_stats.  Synchronises. */
+int32_t az_get_cap_stats(az_engine *h, az_cap_stats *out_host, void *stream);
+
 /* number of finished episodes / samples waiting in the ring.  Synchronises on `stream`. */
 int32_t az_episode_counts(az_engine *h, int64_t *n_episodes_host, int64_t *n_samples_host, void *stream);
 /* copy the ring out (device buffers sized from az_episode_counts) and empty it.  Episodes appear in
