@@ -37,6 +37,8 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <type_traits>
+
 #include <cuda_bf16.h>
 
 #include "../../include/az_engine.h"
@@ -2233,6 +2235,31 @@ void use_ring(az_engine *h, int r) {
 inline cudaStream_t S(void *s) { return (cudaStream_t)s; }
 inline int blocks_for(long long n, int per_block) { return (int)((n + per_block - 1) / per_block); }
 
+// Host dispatch of a kernel's template variants: f gets each runtime value as a compile-time constant, so one launch line in a
+// generic lambda covers every variant.  f takes its parameters by value (`auto`): in C++17 a reference parameter is not a constant
+// expression.  An excluded combination is an `if constexpr` inside f.
+// with_int<Vs...>(v, f): f(std::integral_constant<int, V>{}) for the V of Vs equal to v, the last of Vs when none is.
+template <int V, int... Vs, typename F>
+auto with_int(int v, F f) {
+    if constexpr (sizeof...(Vs) == 0) return f(std::integral_constant<int, V>{});
+    else if (v == V) return f(std::integral_constant<int, V>{});
+    else return with_int<Vs...>(v, f);
+}
+
+// with_flags(f, b...): f(std::bool_constant<b>{}...)
+template <typename F>
+auto with_flags(F f) { return f(); }
+template <typename F, typename... B>
+auto with_flags(F f, bool b, B... bs) {
+    auto bind = [&](auto c) { return with_flags([&](auto... cs) { return f(c, cs...); }, bs...); };
+    if (b) return bind(std::true_type{});
+    return bind(std::false_type{});
+}
+
+// with_tpw(G, f): f(std::integral_constant<int, TPW>{}), TPW = 32 / G trees per warp for G = 32 / 16 / 8 lanes per tree
+template <typename F>
+auto with_tpw(int G, F f) { return with_int<1, 2, 4>(32 / G, f); }
+
 int set_device(az_engine *h) {
     AZ_CUDA(h, cudaSetDevice(h->cfg.device));
     return AZ_OK;
@@ -2250,12 +2277,9 @@ int launch_encode(az_engine *h, const uint64_t *bb0, const uint64_t *bb1, const 
     const size_t smem = (size_t)B * WP * sizeof(uint32_t);
     const int blocks = blocks_for(n, B);
     uint32_t *o = static_cast<uint32_t *>(out);
-    switch (layout) {
-        case AZ_LAYOUT_GRID_F32: k_encode<AZ_LAYOUT_GRID_F32><<<blocks, B, smem, st>>>(bb0, bb1, player, status, n, o); break;
-        case AZ_LAYOUT_PLANES_F32: k_encode<AZ_LAYOUT_PLANES_F32><<<blocks, B, smem, st>>>(bb0, bb1, player, status, n, o); break;
-        case AZ_LAYOUT_PLANES_BF16: k_encode<AZ_LAYOUT_PLANES_BF16><<<blocks, B, smem, st>>>(bb0, bb1, player, status, n, o); break;
-        default: k_encode<AZ_LAYOUT_PLANES_BF16_NHWC><<<blocks, B, smem, st>>>(bb0, bb1, player, status, n, o); break;
-    }
+    with_int<AZ_LAYOUT_GRID_F32, AZ_LAYOUT_PLANES_F32, AZ_LAYOUT_PLANES_BF16, AZ_LAYOUT_PLANES_BF16_NHWC>(layout, [&](auto LAYOUT) {
+        k_encode<LAYOUT><<<blocks, B, smem, st>>>(bb0, bb1, player, status, n, o);
+    });
     AZ_LAUNCH_CHECK(h, "k_encode");
     return AZ_OK;
 }
@@ -2274,6 +2298,45 @@ int launch_reroot(az_engine *h, int n, cudaStream_t st) {
     if (smem > 48 * 1024) AZ_CUDA(h, cudaFuncSetAttribute(k_reroot, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k_reroot<<<n, 32, smem, st>>>(h->a, n, h->cfg.num_simulations, h->reuse_v, h->reroot, h->rstats, words);
     AZ_LAUNCH_CHECK(h, "k_reroot");
+    return AZ_OK;
+}
+
+// the roots changed: no simulation on them yet, no noise on their priors
+void roots_replaced(az_engine *h) {
+    h->sims_done = 0;
+    h->noise_applied = false;
+}
+
+// the end of a selection launch over n slots: k_compact_leaves when the leaf list is not built by the selection itself
+// (compact_launch), then the state its expansion and az_leaf_compact / az_leaf_mirror read
+int selection_launched(az_engine *h, int n, bool cache, bool sym, bool compact_launch, cudaStream_t st) {
+    h->compact_valid = h->compact != 0;
+    if (compact_launch) {
+        k_compact_leaves<<<1, 1024, 0, st>>>(h->a.leaf_status, n, h->a.eval_list, h->a.eval_count, env_int("AZ_COMPACT_STAGE", 1),
+                                             cache ? h->a.cache_ctl : nullptr);
+        AZ_LAUNCH_CHECK(h, "k_compact_leaves");
+    }
+    h->sims_done += 1;
+    h->sel_pending = true;
+    h->cache_sel = cache;
+    h->sym_sel = sym;
+    return AZ_OK;
+}
+
+// tot[c] += the sum over slots of the device's per-slot counters [E][ncols]; err_fmt ("<caller>: %s") words a failure
+int sum_slot_counters(az_engine *h, const char *err_fmt, const unsigned long long *counters, int ncols, unsigned long long *tot,
+                      cudaStream_t st) {
+    const size_t n = (size_t)h->a.E * ncols;
+    unsigned long long *buf = (unsigned long long *)malloc(n * sizeof(unsigned long long));
+    if (!buf) return fail(h, AZ_E_NOMEM, err_fmt, "host allocation failed");
+    cudaError_t e = cudaMemcpyAsync(buf, counters, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) {
+        free(buf);
+        return fail(h, AZ_E_CUDA, err_fmt, cudaGetErrorString(e));
+    }
+    for (size_t i = 0; i < n; ++i) tot[i % ncols] += buf[i];
+    free(buf);
     return AZ_OK;
 }
 }  // namespace
@@ -2421,19 +2484,13 @@ int32_t az_env_step(az_engine *h, const uint64_t *bb0, const uint64_t *bb1, cons
     for (const void *p : ptrs) vec = vec && p && (reinterpret_cast<uintptr_t>(p) & 15u) == 0;
     const long long quads = vec ? n / 4 : 0, head = quads * 4;
     if (quads) {
-        const int mode = rules_mode();
-#define AZ_ENV_H(M_)                                                                                                                \
-    k_env_step_h<M_><<<blocks_for(quads, 256), 256, 0, S(stream)>>>(                                                                \
-        reinterpret_cast<const uint4 *>(bb0), reinterpret_cast<const uint4 *>(bb1), reinterpret_cast<const uint32_t *>(player),     \
-        reinterpret_cast<const uint32_t *>(col), quads, reinterpret_cast<uint4 *>(o0), reinterpret_cast<uint4 *>(o1),                \
-        reinterpret_cast<uint32_t *>(opl), reinterpret_cast<uint32_t *>(olegal), reinterpret_cast<uint32_t *>(oended),              \
-        reinterpret_cast<uint2 *>(oreward), reinterpret_cast<uint32_t *>(ostatus))
-        if (mode == 0) AZ_ENV_H(0);
-        else if (mode == 2) AZ_ENV_H(2);
-        else if (mode == 3) AZ_ENV_H(3);
-        else if (mode == 1) AZ_ENV_H(1);
-        else AZ_ENV_H(4);
-#undef AZ_ENV_H
+        with_int<0, 1, 2, 3, 4>(rules_mode(), [&](auto MODE) {
+            k_env_step_h<MODE><<<blocks_for(quads, 256), 256, 0, S(stream)>>>(
+                reinterpret_cast<const uint4 *>(bb0), reinterpret_cast<const uint4 *>(bb1), reinterpret_cast<const uint32_t *>(player),
+                reinterpret_cast<const uint32_t *>(col), quads, reinterpret_cast<uint4 *>(o0), reinterpret_cast<uint4 *>(o1),
+                reinterpret_cast<uint32_t *>(opl), reinterpret_cast<uint32_t *>(olegal), reinterpret_cast<uint32_t *>(oended),
+                reinterpret_cast<uint2 *>(oreward), reinterpret_cast<uint32_t *>(ostatus));
+        });
         AZ_LAUNCH_CHECK(h, "k_env_step_h");
     }
     if (head < n) {
@@ -2459,17 +2516,11 @@ int32_t az_state_info(az_engine *h, const uint64_t *bb0, const uint64_t *bb1, co
     for (const void *p : ptrs) vec = vec && p && (reinterpret_cast<uintptr_t>(p) & 15u) == 0;
     const long long quads = vec ? n / 4 : 0, head = quads * 4;
     if (quads) {
-        const int mode = rules_mode();
-#define AZ_INFO_H(M_)                                                                                                                      \
-    k_state_info_h<M_><<<blocks_for(quads, 256), 256, 0, S(stream)>>>(reinterpret_cast<const uint4 *>(bb0), reinterpret_cast<const uint4 *>(bb1), \
-                                                                      quads, reinterpret_cast<uint32_t *>(olegal),                         \
-                                                                      reinterpret_cast<uint32_t *>(oended), reinterpret_cast<uint2 *>(oreward))
-        if (mode == 0) AZ_INFO_H(0);
-        else if (mode == 2) AZ_INFO_H(2);
-        else if (mode == 3) AZ_INFO_H(3);
-        else if (mode == 1) AZ_INFO_H(1);
-        else AZ_INFO_H(4);
-#undef AZ_INFO_H
+        with_int<0, 1, 2, 3, 4>(rules_mode(), [&](auto MODE) {
+            k_state_info_h<MODE><<<blocks_for(quads, 256), 256, 0, S(stream)>>>(
+                reinterpret_cast<const uint4 *>(bb0), reinterpret_cast<const uint4 *>(bb1), quads, reinterpret_cast<uint32_t *>(olegal),
+                reinterpret_cast<uint32_t *>(oended), reinterpret_cast<uint2 *>(oreward));
+        });
         AZ_LAUNCH_CHECK(h, "k_state_info_h");
     }
     if (head < n) {
@@ -2535,8 +2586,7 @@ int32_t az_reset_games(az_engine *h, uint64_t init_bb0, uint64_t init_bb1, int32
     h->have_init = true;
     h->n_active = E;
     h->step = 0;
-    h->sims_done = 0;
-    h->noise_applied = false;
+    roots_replaced(h);
     h->sel_pending = false;
     return AZ_OK;
 }
@@ -2551,8 +2601,7 @@ int32_t az_set_roots(az_engine *h, const uint64_t *bb0, const uint64_t *bb1, con
     if (h->cap_on)  // not a self-play move step: every search is full
         if (int rc = launch_cap_draw(h, 0u, true, S(stream))) return rc;
     h->n_active = n;
-    h->sims_done = 0;
-    h->noise_applied = false;
+    roots_replaced(h);
     h->sel_pending = false;
     return AZ_OK;
 }
@@ -2602,8 +2651,7 @@ int32_t az_run_move_step(az_engine *h, int32_t num_sims, int32_t eval_kind, cons
     const int32_t rc = run_sims_impl(h, num_sims, eval_kind, uniforms, finished, true, stream);
     if (rc != AZ_OK) return rc;
     h->step++;
-    h->sims_done = 0;
-    h->noise_applied = false;
+    roots_replaced(h);
     return AZ_OK;
 }
 
@@ -2650,39 +2698,20 @@ static int32_t run_sims_impl(az_engine *h, int32_t num_sims, int32_t eval_kind, 
     mv.init1 = h->init1;
     mv.step = h->step;
     mv.initpl = h->initpl;
-    const bool budget = h->cap_on;  // never with `move`: az_run_move_step leaves the move to k_sample_moves then
-#define AZ_RUN3(TPW_, EV_, LAT_, MOVE_, TSM_, BUD_)                                                                                               \
-    do {                                                                                                                                          \
-        AZ_CUDA(h, cudaFuncSetAttribute(k_run_sims<TPW_, EV_, LAT_, MOVE_, TSM_, BUD_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        k_run_sims<TPW_, EV_, LAT_, MOVE_, TSM_, BUD_><<<blocks, 64, smem, S(stream)>>>(h->a, n, num_sims, c, K, mv, h->cap.budget);            \
-    } while (0)
-#define AZ_RUN2(TPW_, EV_, LAT_, MOVE_, BUD_)                       \
-    do {                                                            \
-        if (tabs_in_smem) AZ_RUN3(TPW_, EV_, LAT_, MOVE_, true, BUD_); \
-        else AZ_RUN3(TPW_, EV_, LAT_, MOVE_, false, BUD_);          \
-    } while (0)
-#define AZ_RUN1(TPW_, EV_, LAT_)                           \
-    do {                                                   \
-        if (move) AZ_RUN2(TPW_, EV_, LAT_, true, false);   \
-        else if (budget) AZ_RUN2(TPW_, EV_, LAT_, false, true); \
-        else AZ_RUN2(TPW_, EV_, LAT_, false, false);       \
-    } while (0)
-#define AZ_RUN(TPW_, EV_)                  \
-    do {                                   \
-        if (lat) AZ_RUN1(TPW_, EV_, true); \
-        else AZ_RUN1(TPW_, EV_, false);    \
-    } while (0)
-    if (tpw == 1) {
-        if (eval_kind == AZ_EVAL_UNIFORM) AZ_RUN(1, AZ_EVAL_UNIFORM); else AZ_RUN(1, AZ_EVAL_HASH);
-    } else if (tpw == 2) {
-        if (eval_kind == AZ_EVAL_UNIFORM) AZ_RUN(2, AZ_EVAL_UNIFORM); else AZ_RUN(2, AZ_EVAL_HASH);
-    } else {
-        if (eval_kind == AZ_EVAL_UNIFORM) AZ_RUN(4, AZ_EVAL_UNIFORM); else AZ_RUN(4, AZ_EVAL_HASH);
-    }
-#undef AZ_RUN
-#undef AZ_RUN1
-#undef AZ_RUN2
-#undef AZ_RUN3
+    const bool budget = h->cap_on && !move;
+    const int rc = with_tpw(h->G, [&](auto TPW) {
+        return with_int<AZ_EVAL_UNIFORM, AZ_EVAL_HASH>(eval_kind, [&](auto EVAL) {
+            return with_flags([&](auto LAT, auto MOVE, auto TSM, auto BUDGET) -> int {
+                // not built: with a playout cap, az_run_move_step leaves the move to k_sample_moves
+                if constexpr (!(MOVE && BUDGET)) {
+                    AZ_CUDA(h, cudaFuncSetAttribute(k_run_sims<TPW, EVAL, LAT, MOVE, TSM, BUDGET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                    k_run_sims<TPW, EVAL, LAT, MOVE, TSM, BUDGET><<<blocks, 64, smem, S(stream)>>>(h->a, n, num_sims, c, K, mv, h->cap.budget);
+                }
+                return AZ_OK;
+            }, lat, move, tabs_in_smem != 0, budget);
+        });
+    });
+    if (rc != AZ_OK) return rc;
     h->last_hot_nodes = K;
     h->sims_done += num_sims;
     AZ_LAUNCH_CHECK(h, "k_run_sims");
@@ -2703,45 +2732,13 @@ int32_t az_select_leaves(az_engine *h, void *stream) {
     const bool lat = latency_variant(h, blocks_for(n, tpb));
     const bool cache = cache_active(h);
     const bool sym = h->sym;
-    const bool budget = h->cap_on;
-#define AZ_SEL3(TPW_, SYM_, BUD_)                                                                                                        \
-    do {                                                                                                                                 \
-        if (cache) {                                                                                                                     \
-            if (lat) k_select<TPW_, true, true, SYM_, BUD_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);  \
-            else k_select<TPW_, false, true, SYM_, BUD_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);     \
-        } else {                                                                                                                         \
-            if (lat) k_select<TPW_, true, false, SYM_, BUD_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror, h->cap.budget); \
-            else k_select<TPW_, false, false, SYM_, BUD_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);    \
-        }                                                                                                                                \
-    } while (0)
-#define AZ_SEL2(TPW_, SYM_)                        \
-    do {                                           \
-        if (budget) AZ_SEL3(TPW_, SYM_, true);     \
-        else AZ_SEL3(TPW_, SYM_, false);           \
-    } while (0)
-#define AZ_SEL(TPW_)                      \
-    do {                                  \
-        if (sym) AZ_SEL2(TPW_, true);     \
-        else AZ_SEL2(TPW_, false);        \
-    } while (0)
-    if (h->G == 32) AZ_SEL(1);
-    else if (h->G == 16) AZ_SEL(2);
-    else AZ_SEL(4);
-#undef AZ_SEL
-#undef AZ_SEL2
-#undef AZ_SEL3
+    with_tpw(h->G, [&](auto TPW) {
+        with_flags([&](auto LAT, auto CACHE, auto SYM, auto BUDGET) {
+            k_select<TPW, LAT, CACHE, SYM, BUDGET><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);
+        }, lat, cache, sym, h->cap_on);
+    });
     AZ_LAUNCH_CHECK(h, "k_select");
-    h->compact_valid = h->compact != 0;
-    if (h->compact) {
-        k_compact_leaves<<<1, 1024, 0, S(stream)>>>(h->a.leaf_status, n, h->a.eval_list, h->a.eval_count, env_int("AZ_COMPACT_STAGE", 1),
-                                                    cache ? h->a.cache_ctl : nullptr);
-        AZ_LAUNCH_CHECK(h, "k_compact_leaves");
-    }
-    h->sims_done += 1;
-    h->sel_pending = true;
-    h->cache_sel = cache;
-    h->sym_sel = sym;
-    return AZ_OK;
+    return selection_launched(h, n, cache, sym, h->compact != 0, S(stream));
 }
 
 int32_t az_gather_leaves(az_engine *h, void *out, int32_t layout, void *stream) {
@@ -2761,21 +2758,11 @@ int32_t az_expand_backup(az_engine *h, const float *policy, const float *values,
     const int n = h->n_active;
     const bool cache = h->sel_pending && h->cache_sel;  // SERVED leaves and claims exist only after a cached selection
     const bool sym = h->sel_pending && h->sym_sel;      // mirrored leaves exist only after a symmetric selection
-#define AZ_EB2(TPW_, SYM_)                                                                                                          \
-    do {                                                                                                                            \
-        if (cache) k_expand_backup<TPW_, true, SYM_><<<blocks_for(n, 2 * TPW_), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->leaf_mirror);  \
-        else k_expand_backup<TPW_, false, SYM_><<<blocks_for(n, 2 * TPW_), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->leaf_mirror);  \
-    } while (0)
-#define AZ_EB(TPW_)                      \
-    do {                                 \
-        if (sym) AZ_EB2(TPW_, true);     \
-        else AZ_EB2(TPW_, false);        \
-    } while (0)
-    if (h->G == 32) AZ_EB(1);
-    else if (h->G == 16) AZ_EB(2);
-    else AZ_EB(4);
-#undef AZ_EB
-#undef AZ_EB2
+    with_tpw(h->G, [&](auto TPW) {
+        with_flags([&](auto CACHE, auto SYM) {
+            k_expand_backup<TPW, CACHE, SYM><<<blocks_for(n, 2 * TPW), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->leaf_mirror);
+        }, cache, sym);
+    });
     AZ_LAUNCH_CHECK(h, "k_expand_backup");
     h->compact_valid = false;  // the leaves are consumed
     h->sel_pending = false;
@@ -2799,51 +2786,14 @@ int32_t az_expand_backup_select(az_engine *h, const float *policy, const float *
     if (h->sel_pending && h->cache_sel != cache)
         return fail(h, AZ_E_STATE, "%s", "az_expand_backup_select: the evaluation cache or leaf compaction changed between a selection and its expansion");
     const bool sym = h->sym;  // az_set_symmetric_eval refuses while a selection is pending: the expansion matches its selection
-    const bool budget = h->cap_on;
-#define AZ_ES4(TPW_, LAT_, CMP_, SYM_, BUD_)                                                                                                \
-    do {                                                                                                                              \
-        if (cache) k_expand_select<TPW_, LAT_, CMP_, true, SYM_, BUD_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);  \
-        else k_expand_select<TPW_, LAT_, CMP_, false, SYM_, BUD_><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, policy, values, policy_kind, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);  \
-    } while (0)
-#define AZ_ES3(TPW_, LAT_, CMP_, SYM_)                   \
-    do {                                                 \
-        if (budget) AZ_ES4(TPW_, LAT_, CMP_, SYM_, true); \
-        else AZ_ES4(TPW_, LAT_, CMP_, SYM_, false);      \
-    } while (0)
-#define AZ_ES2(TPW_, LAT_, CMP_)                     \
-    do {                                             \
-        if (sym) AZ_ES3(TPW_, LAT_, CMP_, true);     \
-        else AZ_ES3(TPW_, LAT_, CMP_, false);        \
-    } while (0)
-#define AZ_ES(TPW_)                               \
-    do {                                          \
-        if (fused) {                              \
-            if (lat) AZ_ES2(TPW_, true, true);    \
-            else AZ_ES2(TPW_, false, true);       \
-        } else {                                  \
-            if (lat) AZ_ES2(TPW_, true, false);   \
-            else AZ_ES2(TPW_, false, false);      \
-        }                                         \
-    } while (0)
-    if (h->G == 32) AZ_ES(1);
-    else if (h->G == 16) AZ_ES(2);
-    else AZ_ES(4);
-#undef AZ_ES
-#undef AZ_ES2
-#undef AZ_ES3
-#undef AZ_ES4
+    with_tpw(h->G, [&](auto TPW) {
+        with_flags([&](auto LAT, auto COMPACT, auto CACHE, auto SYM, auto BUDGET) {
+            k_expand_select<TPW, LAT, COMPACT, CACHE, SYM, BUDGET><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(
+                h->a, n, policy, values, policy_kind, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);
+        }, lat, fused, cache, sym, h->cap_on);
+    });
     AZ_LAUNCH_CHECK(h, "k_expand_select");
-    h->compact_valid = h->compact != 0;
-    if (h->compact == 1) {
-        k_compact_leaves<<<1, 1024, 0, S(stream)>>>(h->a.leaf_status, n, h->a.eval_list, h->a.eval_count, env_int("AZ_COMPACT_STAGE", 1),
-                                                    cache ? h->a.cache_ctl : nullptr);
-        AZ_LAUNCH_CHECK(h, "k_compact_leaves");
-    }
-    h->sims_done += 1;
-    h->sel_pending = true;
-    h->cache_sel = cache;
-    h->sym_sel = sym;
-    return AZ_OK;
+    return selection_launched(h, n, cache, sym, h->compact == 1, S(stream));
 }
 
 int32_t az_leaf_info(az_engine *h, uint64_t *o0, uint64_t *o1, uint8_t *opl, uint8_t *olegal, uint8_t *ostatus,
@@ -2922,23 +2872,11 @@ int32_t az_sample_moves(az_engine *h, const double *uniforms, uint8_t *finished,
     const int n = h->n_active;
     const bool reuse = h->reuse_v > 0;
     const bool budget = h->cap_on;
-#define AZ_SM2(G_, R_, B_)                                                                                                         \
-    k_sample_moves<G_, R_, B_><<<blocks_for(n, 128), 128, 0, S(stream)>>>(h->a, n, uniforms, finished, h->step, h->init0, h->init1, \
-                                                                        h->initpl, G_ ? h->greedy_from : -1, R_ ? h->reroot : nullptr, h->cap)
-#define AZ_SM(G_, R_)                  \
-    do {                               \
-        if (budget) AZ_SM2(G_, R_, true); \
-        else AZ_SM2(G_, R_, false);    \
-    } while (0)
-    if (h->greedy_from >= 0) {
-        if (reuse) AZ_SM(true, true);
-        else AZ_SM(true, false);
-    } else {
-        if (reuse) AZ_SM(false, true);
-        else AZ_SM(false, false);
-    }
-#undef AZ_SM
-#undef AZ_SM2
+    with_flags([&](auto GREEDY, auto REUSE, auto BUDGET) {
+        k_sample_moves<GREEDY, REUSE, BUDGET><<<blocks_for(n, 128), 128, 0, S(stream)>>>(
+            h->a, n, uniforms, finished, h->step, h->init0, h->init1, h->initpl, GREEDY ? h->greedy_from : -1, REUSE ? h->reroot : nullptr,
+            h->cap);
+    }, h->greedy_from >= 0, reuse, budget);
     AZ_LAUNCH_CHECK(h, "k_sample_moves");
     if (reuse) {
         if (int rc = launch_reroot(h, n, S(stream))) return rc;
@@ -2946,8 +2884,7 @@ int32_t az_sample_moves(az_engine *h, const double *uniforms, uint8_t *finished,
             if (int rc = launch_cap_draw(h, (uint32_t)h->step + 1u, false, S(stream))) return rc;
     }
     h->step++;
-    h->sims_done = 0;
-    h->noise_applied = false;
+    roots_replaced(h);
     return AZ_OK;
 }
 
@@ -2988,14 +2925,11 @@ int32_t az_apply_root_noise(az_engine *h, void *stream) {
     if (cap != cudaStreamCaptureStatusNone)
         return fail(h, AZ_E_STATE, "%s", "az_apply_root_noise: not inside a CUDA graph capture (the draw number is a launch argument)");
     const int E = h->a.E;
-    if (h->cap_on)
-        k_root_noise<true><<<blocks_for((long long)E * 8, 256), 256, 0, S(stream)>>>(h->a, h->n_active, h->noise_alpha, h->noise_fraction,
-                                                                                    h->noise_seed, h->noise_slot_offset, h->noise_draws,
-                                                                                    h->noise_eta, h->cap.full);
-    else
-        k_root_noise<false><<<blocks_for((long long)E * 8, 256), 256, 0, S(stream)>>>(h->a, h->n_active, h->noise_alpha, h->noise_fraction,
-                                                                                     h->noise_seed, h->noise_slot_offset, h->noise_draws,
-                                                                                     h->noise_eta, nullptr);
+    with_flags([&](auto BUDGET) {
+        k_root_noise<BUDGET><<<blocks_for((long long)E * 8, 256), 256, 0, S(stream)>>>(h->a, h->n_active, h->noise_alpha, h->noise_fraction,
+                                                                                      h->noise_seed, h->noise_slot_offset, h->noise_draws,
+                                                                                      h->noise_eta, BUDGET ? h->cap.full : nullptr);
+    }, h->cap_on);
     AZ_LAUNCH_CHECK(h, "k_root_noise");
     h->noise_draws++;
     h->noise_applied = true;
@@ -3270,8 +3204,7 @@ int32_t az_set_subtree_reuse(az_engine *h, int32_t max_root_visits) {
         if (int rc2 = launch_cap_draw(h, (uint32_t)h->step, false, nullptr)) return rc2;
     AZ_CUDA(h, cudaDeviceSynchronize());
     h->reuse_v = max_root_visits;
-    h->sims_done = 0;
-    h->noise_applied = false;
+    roots_replaced(h);
     return AZ_OK;
 }
 
@@ -3287,8 +3220,7 @@ int32_t az_advance_roots(az_engine *h, const uint8_t *cols, uint8_t *out_status,
     if (int rc = launch_reroot(h, n, S(stream))) return rc;
     if (h->cap_on)  // not a self-play move step: every search is full
         if (int rc = launch_cap_draw(h, 0u, true, S(stream))) return rc;
-    h->sims_done = 0;
-    h->noise_applied = false;
+    roots_replaced(h);
     return AZ_OK;
 }
 
@@ -3297,18 +3229,8 @@ int32_t az_get_reuse_stats(az_engine *h, az_reuse_stats *out, void *stream) {
     memset(out, 0, sizeof *out);
     if (!h->rstats) return AZ_OK;
     if (int rc = set_device(h)) return rc;
-    const size_t n = (size_t)h->a.E * RS_N;
-    unsigned long long *buf = (unsigned long long *)malloc(n * sizeof(unsigned long long));
-    if (!buf) return fail(h, AZ_E_NOMEM, "%s", "az_get_reuse_stats: host allocation failed");
-    cudaError_t e = cudaMemcpyAsync(buf, h->rstats, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, S(stream));
-    if (e == cudaSuccess) e = cudaStreamSynchronize(S(stream));
-    if (e != cudaSuccess) {
-        free(buf);
-        return fail(h, AZ_E_CUDA, "az_get_reuse_stats: %s", cudaGetErrorString(e));
-    }
     unsigned long long tot[RS_N] = {};
-    for (size_t i = 0; i < n; ++i) tot[i % RS_N] += buf[i];
-    free(buf);
+    if (int rc = sum_slot_counters(h, "az_get_reuse_stats: %s", h->rstats, RS_N, tot, S(stream))) return rc;
     out->retained = tot[RS_RETAINED];
     out->fresh = tot[RS_FRESH];
     out->dropped = tot[RS_DROPPED];
@@ -3385,18 +3307,8 @@ int32_t az_get_cap_stats(az_engine *h, az_cap_stats *out, void *stream) {
     if (int rc = sum_stats(h, r, S(stream))) return rc;
     out->simulations = r[0];
     if (!h->cap.cstats) return AZ_OK;
-    const size_t n = (size_t)h->a.E * CS_N;
-    unsigned long long *buf = (unsigned long long *)malloc(n * sizeof(unsigned long long));
-    if (!buf) return fail(h, AZ_E_NOMEM, "%s", "az_get_cap_stats: host allocation failed");
-    cudaError_t e = cudaMemcpyAsync(buf, h->cap.cstats, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, S(stream));
-    if (e == cudaSuccess) e = cudaStreamSynchronize(S(stream));
-    if (e != cudaSuccess) {
-        free(buf);
-        return fail(h, AZ_E_CUDA, "az_get_cap_stats: %s", cudaGetErrorString(e));
-    }
     unsigned long long tot[CS_N] = {};
-    for (size_t i = 0; i < n; ++i) tot[i % CS_N] += buf[i];
-    free(buf);
+    if (int rc = sum_slot_counters(h, "az_get_cap_stats: %s", h->cap.cstats, CS_N, tot, S(stream))) return rc;
     out->full_searches = tot[CS_FULL];
     out->fast_searches = tot[CS_FAST];
     out->samples_recorded = tot[CS_RECORDED];
