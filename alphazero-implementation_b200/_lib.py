@@ -105,6 +105,14 @@ class AzCapStats(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in ("full_searches", "fast_searches", "samples_recorded", "samples_dropped", "simulations")]
 
 
+class AzForcedPlayouts(C.Structure):
+    _fields_ = [("k", C.c_double)]
+
+
+class AzForcedStats(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in ("forced_selections", "forced_searches", "visits_pruned", "children_zeroed")]
+
+
 class AzResnetDesc(C.Structure):
     _fields_ = [
         ("num_blocks", C.c_int32), ("num_channels", C.c_int32), ("operand_format", C.c_int32), ("variant", C.c_int32),
@@ -184,6 +192,9 @@ SIGNATURES = {
     "az_set_playout_cap": (I32, [P, C.POINTER(AzPlayoutCap)]),
     "az_search_budgets": (I32, [P, P, P, P]),
     "az_get_cap_stats": (I32, [P, C.POINTER(AzCapStats), P]),
+    "az_set_forced_playouts": (I32, [P, C.POINTER(AzForcedPlayouts)]),
+    "az_policy_targets": (I32, [P, P, P]),
+    "az_get_forced_stats": (I32, [P, C.POINTER(AzForcedStats), P]),
     "az_leaf_mirror": (I32, [P, C.POINTER(P)]),
     "az_mirror_states": (I32, [P, P, P, P, I64, P, P, P]),
     "az_trunk_weight_bytes": (I64, [I32]),

@@ -314,11 +314,17 @@ struct Leaf {
 // LAT = true: the latency-optimised variant, for launches with few warps per SM (a simulation is one long dependent chain
 // and nothing else hides it); LAT = false: fewer shuffles and loads per level, for launches that fill the issue slots.
 // Measured on B200 (sims/s, 200 sims/move): 4096 trees 1.97e9 vs 1.81e9; 16384 trees 3.78e9 vs 4.45e9.
-template <bool LAT>
+// FORCED (az_set_forced_playouts): when `force_tree`, a legal root child with RN(N * N) < RN(RN(k * P) * m), m = N_root - 1, outranks
+// every PUCT score (its score becomes +inf, so the lowest such column wins).  The predicate is computed from the root child record
+// before the level loop and only selects the score at depth 0: the loop stays straight-line.  The writer lane adds 1 to *forced
+// when the rule decided the root selection.
+template <bool LAT, bool FORCED>
 __device__ __forceinline__ Leaf descend(const TreeMem &tm, const Tabs &tb,
                                         uint64_t rb0, uint64_t rb1, int rpl, double c_puct, uint32_t cb,
                                         double sq_parent, unsigned legal, Child ch, bool alive, bool writer,
-                                        uint32_t *path, uint32_t &levels, uint32_t &scanned) {
+                                        uint32_t *path, uint32_t &levels, uint32_t &scanned,
+                                        bool force_tree = false, double k_forced = 0.0, uint32_t m = 0u,
+                                        unsigned long long *forced = nullptr) {
     const int lane = threadIdx.x & 31;
     const int sub = lane & 24;
     const int c = lane & 7;
@@ -332,6 +338,12 @@ __device__ __forceinline__ Leaf descend(const TreeMem &tm, const Tabs &tb,
     L.first_col = 0;
     bool go = alive && cb != 0;
     bool my_legal = (legal >> c) & 1u;
+    bool force = false;  // this lane's root child is forced (cleared after the first level)
+    if (FORCED) {
+        force = force_tree && __dmul_rn((double)ch.n, (double)ch.n) < __dmul_rn(__dmul_rn(k_forced, (double)ch.p), (double)m);
+        const unsigned fm = (__ballot_sync(FULL, go && my_legal && force) >> sub) & 0x7Fu;
+        if (writer && fm) *forced += 1ull;
+    }
     // The loop body is straight-line code: four trees share a warp and an idle eighth lane sits in every tree, so every
     // `if` here would be a divergent branch with its reconvergence barrier on the dependent chain.  Lanes of finished
     // trees keep computing on stale (valid) values and every update of the leaf is masked by `go`.
@@ -345,7 +357,7 @@ __device__ __forceinline__ Leaf descend(const TreeMem &tm, const Tabs &tb,
         const bool fills = ((occ >> (c4::STRIDE * c + 4)) & 3ull) == 1ull;
         const unsigned fill_mask = (__ballot_sync(FULL, fills) >> sub) & 0x7Fu;
         const double s = LAT ? puct_score_pre(ch) : puct_score(ch.n, ch.w, ch.p, sq_parent, c_puct, tb.rcp);
-        const double masked = (go && my_legal) ? s : -INFINITY;
+        const double masked = (go && my_legal) ? (FORCED && force ? INFINITY : s) : -INFINITY;
         const int bc = LAT ? argmax_first(masked, c) : argmax_first_ballot(masked, sub);
         const uint32_t cb_sel = __shfl_sync(FULL, ch.cb, sub + bc);
         if (LAT) sq_parent = __shfl_sync(FULL, ch.sq, sub + bc);
@@ -378,6 +390,7 @@ __device__ __forceinline__ Leaf descend(const TreeMem &tm, const Tabs &tb,
         legal = lg;
         my_legal = can;
         ch = nxt;
+        if (FORCED) force = false;
     }
     // Node.is_terminal of the leaf (node.py:61-63).  Interior nodes are never terminal (a terminal
     // node is never expanded), so only the last mover's stones need the line test.
@@ -440,12 +453,25 @@ struct MoveArgs {
     int step, initpl;
 };
 
+// Forced playouts and policy target pruning (az_set_forced_playouts; KataGo).  Per-slot counters of the mode, [E][FS_N] u64: root
+// selections the rule decided, forced searches that ended in a move, visits pruned from their counts, children pruned to 0.
+enum { FS_SELECTIONS, FS_SEARCHES, FS_PRUNED, FS_ZEROED, FS_N };
+
+struct ForcedArgs {
+    double k;
+    const uint8_t *full;           // the playout cap's flags (read by the BUDGET builds only): fast searches are not forced
+    unsigned long long *fstats;    // [E][FS_N]
+};
+
 // TSM: the tables live in shared memory (a compile-time fact, so that the loads are LDS, not generic loads)
 // BUDGET (az_set_playout_cap; MOVE = false only): a tree takes part in a simulation only while its root has fewer visits than
 // budget[t] (a trailing argument, so that the other builds keep their parameter layout); the other trees of the warp go on, and a
 // warp whose trees have all reached their budget leaves the loop
-template <int TPW, int EVAL, bool LAT, bool MOVE, bool TSM, bool BUDGET>
-__global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, double c_puct, int K, MoveArgs mv, const uint32_t *budget) {
+// FORCED (az_set_forced_playouts; MOVE = false only): the root selections of the tree's search follow descend()'s forced rule, unless
+// the playout cap made it a fast search; `fa` is a trailing argument like `budget`
+template <int TPW, int EVAL, bool LAT, bool MOVE, bool TSM, bool BUDGET, bool FORCED>
+__global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, double c_puct, int K, MoveArgs mv, const uint32_t *budget,
+                                                 ForcedArgs fa) {
     constexpr int TREES = 2 * TPW;  // per 64-thread block
     constexpr int NL = 32 / TPW;    // lanes per tree
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -494,6 +520,8 @@ __global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, d
     uint32_t used = a.used[tt];
     uint32_t levels = 0, evals = 0, children = 0, scanned = 0;
     const uint32_t bud = BUDGET ? budget[tt] : 0u;
+    const bool force_tree = FORCED && (!BUDGET || fa.full[tt] != 0);
+    unsigned long long *forced = FORCED ? fa.fstats + (size_t)tt * FS_N + FS_SELECTIONS : nullptr;
     double mv_u = 0.0;
     int mv_len = 0;
     if (MOVE && alive) {
@@ -546,7 +574,8 @@ __global__ void __launch_bounds__(64) k_run_sims(Arena a, int n_active, int S, d
         const bool live = BUDGET ? alive && root_n < bud : alive;
         if (BUDGET && !__any_sync(FULL, live)) break;
         RCLK(c0);
-        Leaf L = descend<LAT>(tm, tb, rb0, rb1, rpl, c_puct, root_cb, root_sq, r_legal, rch, live, writer, path, levels, scanned);
+        Leaf L = descend<LAT, FORCED>(tm, tb, rb0, rb1, rpl, c_puct, root_cb, root_sq, r_legal, rch, live, writer, path, levels, scanned,
+                                      force_tree, fa.k, root_n - 1u, forced);
         RCLK(c1);
         RACC(0, c1, c0);
         // Straight-line from here on as well (the four trees of a warp end in different cases).
@@ -916,9 +945,11 @@ __device__ __forceinline__ void cache_publish(const Arena &a, uint32_t claim, in
 // BUDGET (az_set_playout_cap): a tree whose root has reached its visit budget (budget[t], a trailing kernel argument like
 // leaf_mirror) has finished its search of this move step and is idle, as a tree in error is: every simulation adds exactly one
 // visit to the root, so the root's N counts the simulations done
-template <int TPW, bool LAT, bool CACHE, bool SYM, bool BUDGET>
+// FORCED (az_set_forced_playouts): the root selection follows descend()'s forced rule, unless the playout cap made the search fast;
+// `fa` is a trailing argument like `budget`
+template <int TPW, bool LAT, bool CACHE, bool SYM, bool BUDGET, bool FORCED>
 __device__ __forceinline__ bool select_body(const Arena &a, int n_active, double c_puct, uint32_t launch, uint32_t epoch,
-                                            uint8_t *leaf_mirror, const uint32_t *budget) {
+                                            uint8_t *leaf_mirror, const uint32_t *budget, ForcedArgs fa) {
     constexpr int TREES = 2 * TPW;
     constexpr int NL = 32 / TPW;
     const int lane = threadIdx.x & 31;
@@ -942,6 +973,7 @@ __device__ __forceinline__ bool select_body(const Arena &a, int n_active, double
     const int rpl = a.root_player[tt];
     const uint4 rm = tm.gM[0];
     const uint32_t bud = BUDGET ? budget[tt] : 0u;
+    const bool force_tree = FORCED && (!BUDGET || fa.full[tt] != 0);
     const bool alive = in_range && err == 0 && (!BUDGET || rm.x < bud);
     const int lit = lane & (NL - 1);
     if (in_range && !alive && lit == 0) {
@@ -962,7 +994,8 @@ __device__ __forceinline__ bool select_body(const Arena &a, int n_active, double
     if (alive && rm.z != 0 && r_can) rch = load_child<LAT>(tm, rm.z + __popc(r_legal & ((1u << c) - 1u)), tb, c_puct, root_sq);
     if (writer) path[0] = 0;
     uint32_t levels = 0, scanned = 0;
-    Leaf L = descend<LAT>(tm, tb, rb0, rb1, rpl, c_puct, rm.z, root_sq, r_legal, rch, alive, writer, path, levels, scanned);
+    Leaf L = descend<LAT, FORCED>(tm, tb, rb0, rb1, rpl, c_puct, rm.z, root_sq, r_legal, rch, alive, writer, path, levels, scanned,
+                                  force_tree, fa.k, rm.x - 1u, FORCED ? fa.fstats + (size_t)tt * FS_N + FS_SELECTIONS : nullptr);
     uint8_t status = L.term ? AZ_LEAF_TERMINAL : AZ_LEAF_EVAL;
     if (writer) {
         uint32_t *st = a.tstats + (size_t)t * NSTAT;
@@ -991,11 +1024,12 @@ __device__ __forceinline__ bool select_body(const Arena &a, int n_active, double
 }
 
 // split path, step 3: search.py:87-91 with the evaluator's outputs
-template <int TPW, bool LAT, bool CACHE, bool SYM, bool BUDGET>
-__global__ void __launch_bounds__(64) k_select(Arena a, int n_active, double c_puct, uint8_t *leaf_mirror, const uint32_t *budget) {
+template <int TPW, bool LAT, bool CACHE, bool SYM, bool BUDGET, bool FORCED>
+__global__ void __launch_bounds__(64) k_select(Arena a, int n_active, double c_puct, uint8_t *leaf_mirror, const uint32_t *budget,
+                                               ForcedArgs fa) {
     uint32_t launch = 0, epoch = 0;
     if (CACHE) load_cache_ctl(a, launch, epoch);
-    select_body<TPW, LAT, CACHE, SYM, BUDGET>(a, n_active, c_puct, launch, epoch, leaf_mirror, budget);
+    select_body<TPW, LAT, CACHE, SYM, BUDGET, FORCED>(a, n_active, c_puct, launch, epoch, leaf_mirror, budget, fa);
 }
 
 // split path, step 3: search.py:87-91 with the evaluator's outputs
@@ -1127,15 +1161,15 @@ k_expand_backup(Arena a, int n_active, const float *__restrict__ policy, const f
 // outputs to the slots' rows and a position's outputs do not depend on the batch it falls into, so the search is unchanged.
 // CACHE: both halves use the evaluation cache; with COMPACT the last warp also advances the launch number (the ticket atomic is then
 // acq_rel, so that every warp's read of the number at its start precedes the advance).
-template <int TPW, bool LAT, bool COMPACT, bool CACHE, bool SYM, bool BUDGET>
+template <int TPW, bool LAT, bool COMPACT, bool CACHE, bool SYM, bool BUDGET, bool FORCED>
 __global__ void __launch_bounds__(64)
 k_expand_select(Arena a, int n_active, const float *__restrict__ policy, const float *__restrict__ values, int policy_kind, double c_puct,
-                uint8_t *leaf_mirror, const uint32_t *budget) {
+                uint8_t *leaf_mirror, const uint32_t *budget, ForcedArgs fa) {
     uint32_t launch = 0, epoch = 0;
     if (CACHE) load_cache_ctl(a, launch, epoch);
     expand_backup_body<TPW, CACHE, SYM>(a, n_active, policy, values, policy_kind, launch, leaf_mirror);
     __syncwarp();
-    const bool wants = select_body<TPW, LAT, CACHE, SYM, BUDGET>(a, n_active, c_puct, launch, epoch, leaf_mirror, budget);
+    const bool wants = select_body<TPW, LAT, CACHE, SYM, BUDGET, FORCED>(a, n_active, c_puct, launch, epoch, leaf_mirror, budget, fa);
     if (COMPACT) {
         const int lane = threadIdx.x & 31;
         const unsigned m = __ballot_sync(FULL, wants);
@@ -1644,6 +1678,72 @@ k_leaf_info(Arena a, int n, uint64_t *o0, uint64_t *o1, uint8_t *opl, uint8_t *o
 }
 
 // ------------------------------------------------------------------------------------------------
+// Policy target pruning (az_set_forced_playouts; KataGo): cnt[] (the root's child visit counts by column, 0 off `legal`) becomes N'.
+// c* = the most visited legal child (lowest column on ties) keeps its count, s* = its PUCT score from its real statistics with
+// sq = sqt[N_root].  Every other legal child with N > 0 gives back visits one at a time, at most n_f = the least n with
+// RN(n * n) >= RN(RN(k * P) * m) (what the forcing could have added, m = N_root - 1), while N' > 0 and PUCT with N' - 1 visits
+// (q = its real mean) stays below s*; a child left with 1 visit goes to 0.  m = 0 or k = 0 leaves the counts as they are (nothing
+// was forced).  pruned / zeroed: visits taken away, children that went from N > 0 to 0.
+__device__ __forceinline__ void prune_counts(const Arena &a, size_t base, uint32_t cb, uint32_t legal, uint32_t root_n, double c_puct,
+                                             double k, int32_t (&cnt)[7], uint32_t &pruned, uint32_t &zeroed) {
+    if (root_n <= 1u || k == 0.0) return;
+    const uint32_t m = root_n - 1u;
+    double w[7];
+    float p[7];
+    int bc = 0;
+    int32_t best = -1;
+    {
+        int j = 0;
+#pragma unroll
+        for (int c = 0; c < 7; ++c) {
+            w[c] = 0.0;
+            p[c] = 0.0f;
+            if ((legal >> c) & 1u) {
+                w[c] = a.W[base + cb + j];
+                p[c] = __uint_as_float(a.M[base + cb + j].y);
+                if (cnt[c] > best) {  // strict '>': the first maximum
+                    best = cnt[c];
+                    bc = c;
+                }
+                ++j;
+            }
+        }
+    }
+    double wb = 0.0;
+    float pb = 0.0f;
+#pragma unroll
+    for (int c = 0; c < 7; ++c) {  // selects, not indexing: the arrays stay in registers
+        wb = c == bc ? w[c] : wb;
+        pb = c == bc ? p[c] : pb;
+    }
+    const double sq = a.sqt[root_n];
+    const double s_star = puct_score((uint32_t)best, wb, pb, sq, c_puct, a.rcp);
+#pragma unroll
+    for (int c = 0; c < 7; ++c) {
+        if (!((legal >> c) & 1u) || c == bc || cnt[c] <= 0) continue;
+        const uint32_t n = (uint32_t)cnt[c];
+        const double q = (w[c] == 0.0) ? 0.0 : div_tab(w[c], n, a.rcp);
+        const double x = __dmul_rn(__dmul_rn(c_puct, (double)p[c]), sq);
+        const double thr = __dmul_rn(__dmul_rn(k, (double)p[c]), (double)m);
+        uint32_t nf;
+        if (__dmul_rn((double)n, (double)n) < thr) {
+            nf = n + 1u;  // n_f > N: the bound cannot stop the loop
+        } else if (!(thr > 0.0)) {
+            nf = 0u;
+        } else {
+            nf = (uint32_t)__dsqrt_rn(thr);
+            while (nf > 0u && __dmul_rn((double)(nf - 1u), (double)(nf - 1u)) >= thr) --nf;
+            while (__dmul_rn((double)nf, (double)nf) < thr) ++nf;
+        }
+        uint32_t np = n;
+        while (n - np < nf && np > 0u && __dadd_rn(q, div_tab(x, np, a.rcp)) < s_star) --np;  // u(N' - 1) = x / N'
+        if (np == 1u) np = 0u;
+        pruned += n - np;
+        zeroed += np == 0u ? 1u : 0u;
+        cnt[c] = (int32_t)np;
+    }
+}
+
 // This slot's part of a move step: record the sample, draw and play the move, emit the episode header if the game ended.
 // Returns through copy_len / copy_dst the finished game's samples still to be copied into the ring.
 // GREEDY (az_set_greedy_from): from ply `greedy_from` of the game on, the move is the most visited root child, the lowest
@@ -1654,10 +1754,14 @@ constexpr uint32_t REROOT_NONE = 0u;  // node 0 is the root, never a played chil
 
 // BUDGET (az_set_playout_cap): the ply's flag goes into the game log next to the sample, and a finished game emits only the samples
 // of its full searches (ep_len = their number, possibly 0); copy_len stays the number of plies, the copy skips the fast ones.
-template <bool GREEDY, bool REUSE, bool BUDGET>
+// FORCED (az_set_forced_playouts): after a forced search (every search but the playout cap's fast ones) the pruned counts N' are the
+// recorded sample and the move is drawn from them (denominator sum N' instead of N - 1); the greedy move is the same, as c* keeps
+// its count.  The tree keeps its real statistics.
+template <bool GREEDY, bool REUSE, bool BUDGET, bool FORCED>
 __device__ __forceinline__ void sample_move_slot(const Arena &a, int t, const double *__restrict__ uniforms, uint8_t *finished, int step,
                                                  uint64_t init0, uint64_t init1, int initpl, int greedy_from, int &copy_len,
-                                                 long long &copy_dst, uint32_t *reroot, const CapArgs &cp) {
+                                                 long long &copy_dst, uint32_t *reroot, const CapArgs &cp, double c_puct,
+                                                 const ForcedArgs &fa) {
     if (finished) finished[t] = 0;
     if (REUSE) reroot[t] = REROOT_NONE;
     if (a.tree_err[t]) return;
@@ -1690,6 +1794,28 @@ __device__ __forceinline__ void sample_move_slot(const Arena &a, int t, const do
                 ++j;
             }
         }
+    }
+    if (FORCED && (!BUDGET || cp.full[t] != 0)) {
+        uint32_t pruned = 0, zeroed = 0;
+        prune_counts(a, base, cb, legal, rootm.x, c_puct, fa.k, cnt, pruned, zeroed);
+        int32_t sum = 0;
+#pragma unroll
+        for (int c = 0; c < 7; ++c) sum += cnt[c];
+        const double dn = (double)sum;
+        int j = 0;
+#pragma unroll
+        for (int c = 0; c < 7; ++c) {
+            if ((legal >> c) & 1u) {
+                const double p = __ddiv_rn((double)cnt[c], dn);
+                acc = (j == 0) ? p : __dadd_rn(acc, p);
+                cdf[c] = acc;
+                ++j;
+            }
+        }
+        unsigned long long *fs = fa.fstats + (size_t)t * FS_N;
+        fs[FS_SEARCHES] += 1ull;
+        fs[FS_PRUNED] += pruned;
+        fs[FS_ZEROED] += zeroed;
     }
     if (len < MAX_PLIES) {
         const size_t o = (size_t)t * MAX_PLIES + len;
@@ -1777,17 +1903,18 @@ __device__ __forceinline__ void sample_move_slot(const Arena &a, int t, const do
 // `reroot` and `cp` are trailing arguments read by the REUSE / BUDGET builds only, so the other builds keep the parameter layout.
 // BUDGET without REUSE also draws the flag of the slot's next search (step + 1) and writes its budget; with REUSE k_cap_draw does
 // that after k_reroot has fixed the new root's visit count.
-template <bool GREEDY, bool REUSE, bool BUDGET>
+// `c_puct` and `fa` are trailing arguments of the FORCED builds in the same way.
+template <bool GREEDY, bool REUSE, bool BUDGET, bool FORCED>
 __global__ void __launch_bounds__(128)
 k_sample_moves(Arena a, int n, const double *__restrict__ uniforms, uint8_t *finished, int step, uint64_t init0,
-               uint64_t init1, int initpl, int greedy_from, uint32_t *reroot, CapArgs cp) {
+               uint64_t init1, int initpl, int greedy_from, uint32_t *reroot, CapArgs cp, double c_puct, ForcedArgs fa) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
     int copy_len = 0;
     long long copy_dst = 0;
     if (t < n) {
-        sample_move_slot<GREEDY, REUSE, BUDGET>(a, t, uniforms, finished, step, init0, init1, initpl, greedy_from, copy_len, copy_dst,
-                                                reroot, cp);
+        sample_move_slot<GREEDY, REUSE, BUDGET, FORCED>(a, t, uniforms, finished, step, init0, init1, initpl, greedy_from, copy_len,
+                                                        copy_dst, reroot, cp, c_puct, fa);
         if (BUDGET && !REUSE) cap_set(cp, t, cap_draw_full(cp, t, (uint32_t)step + 1u), a.M[(size_t)t * a.cap].x);
     }
     __syncwarp();  // the sample recorded by this step is visible to the lanes that copy it
@@ -1827,6 +1954,28 @@ k_sample_moves(Arena a, int n, const double *__restrict__ uniforms, uint8_t *fin
         }
         for (int i = lane; i < len * 7; i += 32) a.s_counts[dst * 7 + i] = a.g_counts[g0 * 7 + i];
     }
+}
+
+// az_policy_targets: counts[t][c] = the pruned counts N' of the current roots (what k_sample_moves<FORCED> would record), one thread
+// per slot; raw counts where the playout cap made the search fast (fa.full[t] == 0, fa.full null without the cap), 0 for slots
+// without a searched root.  Counters untouched.
+__global__ void __launch_bounds__(256) k_policy_targets(Arena a, int n, double c_puct, ForcedArgs fa, int32_t *__restrict__ counts) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= a.E) return;
+    int32_t cnt[7] = {0, 0, 0, 0, 0, 0, 0};
+    const size_t base = (size_t)t * a.cap;
+    const uint4 rootm = a.M[base];
+    if (t < n && a.tree_err[t] == 0 && rootm.z != 0) {
+        const uint32_t legal = c4::legal_mask(a.root_bb0[t] | a.root_bb1[t]);
+        int j = 0;
+#pragma unroll
+        for (int c = 0; c < 7; ++c)
+            if ((legal >> c) & 1u) cnt[c] = (int32_t)a.M[base + rootm.z + j++].x;
+        uint32_t pruned = 0, zeroed = 0;
+        if (!fa.full || fa.full[t] != 0) prune_counts(a, base, rootm.z, legal, rootm.x, c_puct, fa.k, cnt, pruned, zeroed);
+    }
+#pragma unroll
+    for (int c = 0; c < 7; ++c) counts[(size_t)t * 7 + c] = cnt[c];
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2162,6 +2311,9 @@ struct az_engine {
     unsigned long long *rstats;  // [E][RS_N] k_reroot's counters
     bool cap_on;                 // az_set_playout_cap: self-play searches run to per-tree budgets (the BUDGET kernels)
     CapArgs cap;                 // its arrays (allocated with the first az_set_playout_cap) and configuration, as the kernels take them
+    bool forced_on;              // az_set_forced_playouts: searches force root children and moves prune their counts (the FORCED kernels)
+    double forced_k;
+    unsigned long long *fstats;  // [E][FS_N] (allocated with the first az_set_forced_playouts)
     int64_t bytes;
     int64_t launches;
     unsigned long long *d_tot;   // [16] stats totals (device)
@@ -2301,6 +2453,15 @@ int launch_reroot(az_engine *h, int n, cudaStream_t st) {
     return AZ_OK;
 }
 
+// the trailing argument of the FORCED kernels (the playout cap's flags only while the cap is on)
+ForcedArgs forced_args(const az_engine *h) {
+    ForcedArgs fa;
+    fa.k = h->forced_k;
+    fa.full = h->cap_on ? h->cap.full : nullptr;
+    fa.fstats = h->fstats;
+    return fa;
+}
+
 // the roots changed: no simulation on them yet, no noise on their priors
 void roots_replaced(az_engine *h) {
     h->sims_done = 0;
@@ -2430,6 +2591,13 @@ int32_t az_create(const az_config *cfg, az_engine **out) {
     cudaMemset(a.g_len, 0, (size_t)E * sizeof(int32_t));
     cudaMemset(a.eval_count, 0, 4 * sizeof(int32_t));
     cudaMemset(a.cache_ctl, 0, 4 * sizeof(uint32_t));
+    // a slot whose root has ended never gets a leaf (it stays AZ_LEAF_IDLE): its leaf arrays read as zeros, not as whatever the
+    // allocation held before
+    cudaMemset(a.leaf_node, 0, (size_t)E * sizeof(uint32_t));
+    cudaMemset(a.leaf_bb0, 0, (size_t)E * sizeof(uint64_t));
+    cudaMemset(a.leaf_bb1, 0, (size_t)E * sizeof(uint64_t));
+    cudaMemset(a.leaf_player, 0, (size_t)E);
+    cudaMemset(a.leaf_depth, 0, (size_t)E);
     // every slot starts at the empty board, player 0 (Config.sample_initial_state())
     k_set_roots<<<blocks_for(E, 256), 256>>>(a, nullptr, nullptr, nullptr, 0ull, 0ull, 0, E, 1);
     h->launches++;
@@ -2641,9 +2809,9 @@ int32_t az_run_move_step(az_engine *h, int32_t num_sims, int32_t eval_kind, cons
     if (!uniforms) return fail(h, AZ_E_INVALID, "%s", "az_run_move_step: null uniforms");
     if (!h->have_init) return fail(h, AZ_E_STATE, "%s", "az_run_move_step: call az_reset_games first");
     if (num_sims < 1) return fail(h, AZ_E_INVALID, "%s", "az_run_move_step: num_sims < 1");
-    // the greedy rule, subtree reuse and the playout cap live in k_sample_moves (+ k_reroot) only: the search (its hot prefix written
-    // back), then the move
-    if (h->greedy_from >= 0 || h->reuse_v > 0 || h->cap_on) {
+    // the greedy rule, subtree reuse, the playout cap and policy target pruning live in k_sample_moves (+ k_reroot) only: the search
+    // (its hot prefix written back), then the move
+    if (h->greedy_from >= 0 || h->reuse_v > 0 || h->cap_on || h->forced_on) {
         const int32_t rc = run_sims_impl(h, num_sims, eval_kind, nullptr, nullptr, false, stream);
         if (rc != AZ_OK) return rc;
         return az_sample_moves(h, uniforms, finished, stream);
@@ -2699,16 +2867,21 @@ static int32_t run_sims_impl(az_engine *h, int32_t num_sims, int32_t eval_kind, 
     mv.step = h->step;
     mv.initpl = h->initpl;
     const bool budget = h->cap_on && !move;
+    const bool forced = h->forced_on && !move;
+    const ForcedArgs fa = forced_args(h);
     const int rc = with_tpw(h->G, [&](auto TPW) {
         return with_int<AZ_EVAL_UNIFORM, AZ_EVAL_HASH>(eval_kind, [&](auto EVAL) {
-            return with_flags([&](auto LAT, auto MOVE, auto TSM, auto BUDGET) -> int {
+            return with_flags([&](auto LAT, auto MOVE, auto TSM, auto BUDGET, auto FORCED) -> int {
                 // not built: with a playout cap, az_run_move_step leaves the move to k_sample_moves
-                if constexpr (!(MOVE && BUDGET)) {
-                    AZ_CUDA(h, cudaFuncSetAttribute(k_run_sims<TPW, EVAL, LAT, MOVE, TSM, BUDGET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                    k_run_sims<TPW, EVAL, LAT, MOVE, TSM, BUDGET><<<blocks, 64, smem, S(stream)>>>(h->a, n, num_sims, c, K, mv, h->cap.budget);
+                if constexpr (MOVE && BUDGET) return AZ_OK;
+                // not built either: forced searches prune their counts before the move, which k_sample_moves does
+                else if constexpr (MOVE && FORCED) return AZ_OK;
+                else {
+                    AZ_CUDA(h, cudaFuncSetAttribute(k_run_sims<TPW, EVAL, LAT, MOVE, TSM, BUDGET, FORCED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                    k_run_sims<TPW, EVAL, LAT, MOVE, TSM, BUDGET, FORCED><<<blocks, 64, smem, S(stream)>>>(h->a, n, num_sims, c, K, mv, h->cap.budget, fa);
+                    return AZ_OK;
                 }
-                return AZ_OK;
-            }, lat, move, tabs_in_smem != 0, budget);
+            }, lat, move, tabs_in_smem != 0, budget, forced);
         });
     });
     if (rc != AZ_OK) return rc;
@@ -2733,9 +2906,10 @@ int32_t az_select_leaves(az_engine *h, void *stream) {
     const bool cache = cache_active(h);
     const bool sym = h->sym;
     with_tpw(h->G, [&](auto TPW) {
-        with_flags([&](auto LAT, auto CACHE, auto SYM, auto BUDGET) {
-            k_select<TPW, LAT, CACHE, SYM, BUDGET><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);
-        }, lat, cache, sym, h->cap_on);
+        with_flags([&](auto LAT, auto CACHE, auto SYM, auto BUDGET, auto FORCED) {
+            k_select<TPW, LAT, CACHE, SYM, BUDGET, FORCED><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(h->a, n, h->cfg.c_puct, h->leaf_mirror,
+                                                                                                     h->cap.budget, forced_args(h));
+        }, lat, cache, sym, h->cap_on, h->forced_on);
     });
     AZ_LAUNCH_CHECK(h, "k_select");
     return selection_launched(h, n, cache, sym, h->compact != 0, S(stream));
@@ -2787,10 +2961,10 @@ int32_t az_expand_backup_select(az_engine *h, const float *policy, const float *
         return fail(h, AZ_E_STATE, "%s", "az_expand_backup_select: the evaluation cache or leaf compaction changed between a selection and its expansion");
     const bool sym = h->sym;  // az_set_symmetric_eval refuses while a selection is pending: the expansion matches its selection
     with_tpw(h->G, [&](auto TPW) {
-        with_flags([&](auto LAT, auto COMPACT, auto CACHE, auto SYM, auto BUDGET) {
-            k_expand_select<TPW, LAT, COMPACT, CACHE, SYM, BUDGET><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(
-                h->a, n, policy, values, policy_kind, h->cfg.c_puct, h->leaf_mirror, h->cap.budget);
-        }, lat, fused, cache, sym, h->cap_on);
+        with_flags([&](auto LAT, auto COMPACT, auto CACHE, auto SYM, auto BUDGET, auto FORCED) {
+            k_expand_select<TPW, LAT, COMPACT, CACHE, SYM, BUDGET, FORCED><<<blocks_for(n, tpb), 64, 0, S(stream)>>>(
+                h->a, n, policy, values, policy_kind, h->cfg.c_puct, h->leaf_mirror, h->cap.budget, forced_args(h));
+        }, lat, fused, cache, sym, h->cap_on, h->forced_on);
     });
     AZ_LAUNCH_CHECK(h, "k_expand_select");
     return selection_launched(h, n, cache, sym, h->compact == 1, S(stream));
@@ -2872,11 +3046,11 @@ int32_t az_sample_moves(az_engine *h, const double *uniforms, uint8_t *finished,
     const int n = h->n_active;
     const bool reuse = h->reuse_v > 0;
     const bool budget = h->cap_on;
-    with_flags([&](auto GREEDY, auto REUSE, auto BUDGET) {
-        k_sample_moves<GREEDY, REUSE, BUDGET><<<blocks_for(n, 128), 128, 0, S(stream)>>>(
+    with_flags([&](auto GREEDY, auto REUSE, auto BUDGET, auto FORCED) {
+        k_sample_moves<GREEDY, REUSE, BUDGET, FORCED><<<blocks_for(n, 128), 128, 0, S(stream)>>>(
             h->a, n, uniforms, finished, h->step, h->init0, h->init1, h->initpl, GREEDY ? h->greedy_from : -1, REUSE ? h->reroot : nullptr,
-            h->cap);
-    }, h->greedy_from >= 0, reuse, budget);
+            h->cap, h->cfg.c_puct, forced_args(h));
+    }, h->greedy_from >= 0, reuse, budget, h->forced_on);
     AZ_LAUNCH_CHECK(h, "k_sample_moves");
     if (reuse) {
         if (int rc = launch_reroot(h, n, S(stream))) return rc;
@@ -3132,6 +3306,7 @@ int32_t az_reset_stats(az_engine *h, void *stream) {
     memset(h->acc_tot, 0, sizeof h->acc_tot);
     if (h->rstats) AZ_CUDA(h, cudaMemsetAsync(h->rstats, 0, (size_t)h->a.E * RS_N * sizeof(unsigned long long), S(stream)));
     if (h->cap.cstats) AZ_CUDA(h, cudaMemsetAsync(h->cap.cstats, 0, (size_t)h->a.E * CS_N * sizeof(unsigned long long), S(stream)));
+    if (h->fstats) AZ_CUDA(h, cudaMemsetAsync(h->fstats, 0, (size_t)h->a.E * FS_N * sizeof(unsigned long long), S(stream)));
     return AZ_OK;
 }
 
@@ -3313,6 +3488,50 @@ int32_t az_get_cap_stats(az_engine *h, az_cap_stats *out, void *stream) {
     out->fast_searches = tot[CS_FAST];
     out->samples_recorded = tot[CS_RECORDED];
     out->samples_dropped = tot[CS_DROPPED];
+    return AZ_OK;
+}
+
+int32_t az_set_forced_playouts(az_engine *h, const az_forced_playouts *cfg) {
+    if (!h) return AZ_E_INVALID;
+    if (h->sel_pending) return fail(h, AZ_E_STATE, "%s", "az_set_forced_playouts: a selection's leaves wait for their expansion");
+    if (!cfg) {
+        h->forced_on = false;
+        return AZ_OK;
+    }
+    if (!(cfg->k >= 0.0 && cfg->k <= 1024.0)) return fail(h, AZ_E_INVALID, "%s", "az_set_forced_playouts: k must be finite and in [0, 1024]");
+    if (!h->fstats) {
+        if (int rc = set_device(h)) return rc;
+        unsigned long long *p = nullptr;
+        if (int rc = dev_alloc(h, &p, (size_t)h->a.E * FS_N)) return rc;
+        AZ_CUDA(h, cudaMemset(p, 0, (size_t)h->a.E * FS_N * sizeof(unsigned long long)));
+        h->fstats = p;
+    }
+    h->forced_k = cfg->k;
+    h->forced_on = true;
+    return AZ_OK;
+}
+
+int32_t az_policy_targets(az_engine *h, int32_t *counts, void *stream) {
+    if (!h) return AZ_E_INVALID;
+    if (!counts) return fail(h, AZ_E_INVALID, "%s", "az_policy_targets: null output");
+    if (!h->forced_on) return fail(h, AZ_E_STATE, "%s", "az_policy_targets: forced playouts are off (az_set_forced_playouts)");
+    if (int rc = set_device(h)) return rc;
+    k_policy_targets<<<blocks_for(h->a.E, 256), 256, 0, S(stream)>>>(h->a, h->n_active, h->cfg.c_puct, forced_args(h), counts);
+    AZ_LAUNCH_CHECK(h, "k_policy_targets");
+    return AZ_OK;
+}
+
+int32_t az_get_forced_stats(az_engine *h, az_forced_stats *out, void *stream) {
+    if (!h || !out) return AZ_E_INVALID;
+    memset(out, 0, sizeof *out);
+    if (!h->fstats) return AZ_OK;
+    if (int rc = set_device(h)) return rc;
+    unsigned long long tot[FS_N] = {};
+    if (int rc = sum_slot_counters(h, "az_get_forced_stats: %s", h->fstats, FS_N, tot, S(stream))) return rc;
+    out->forced_selections = tot[FS_SELECTIONS];
+    out->forced_searches = tot[FS_SEARCHES];
+    out->visits_pruned = tot[FS_PRUNED];
+    out->children_zeroed = tot[FS_ZEROED];
     return AZ_OK;
 }
 

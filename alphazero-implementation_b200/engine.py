@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import AzCapStats, AzConfig, AzEvalCacheStats, AzPlayoutCap, AzReuseStats, AzRootNoise, AzStats
+from ._lib import AzCapStats, AzConfig, AzEvalCacheStats, AzForcedPlayouts, AzForcedStats, AzPlayoutCap, AzReuseStats, AzRootNoise, AzStats
 
 EVAL_UNIFORM = 1
 EVAL_HASH = 2
@@ -101,6 +101,7 @@ class Engine:
         self.symmetric_eval = False
         self.subtree_reuse = 0  # max_root_visits, 0 = off
         self.playout_cap = None  # (fast_sims, p_full, seed, slot_offset, visit_budget) while the playout cap is on
+        self.forced_playouts = None  # k while forced playouts and policy target pruning are on
         self.tree_capacity = self.lib.az_tree_capacity(self.h)
 
     # -- plumbing --------------------------------------------------------------------------------
@@ -340,6 +341,33 @@ class Engine:
         st = AzCapStats()
         self._check(self.lib.az_get_cap_stats(self.h, C.byref(st), _stream()), "az_get_cap_stats")
         return {n: int(getattr(st, n)) for n, _ in AzCapStats._fields_}
+
+    def set_forced_playouts(self, k: float | None):
+        """Forced playouts and policy target pruning (`az_set_forced_playouts`, KataGo): every search on this engine gives each root
+        child c at least about sqrt(k P(c) (N_root - 1)) visits (fast searches of the playout cap excepted), and `sample_moves` records
+        and plays from the counts with those extra visits pruned back out (`policy_targets`).  k = 0 gives the same results as off.
+        `k=None` = off (the default).  Call it before a CUDA graph of the search is captured."""
+        if k is None:
+            self._check(self.lib.az_set_forced_playouts(self.h, None), "az_set_forced_playouts")
+            self.forced_playouts = None
+            return
+        cfg = AzForcedPlayouts(float(k))
+        self._check(self.lib.az_set_forced_playouts(self.h, C.byref(cfg)), "az_set_forced_playouts")
+        self.forced_playouts = float(k)
+
+    def policy_targets(self) -> torch.Tensor:
+        """The pruned root child visit counts N' of the active roots by column, int32 [n_active, 7]: what `sample_moves` records as
+        the sample and draws the move from (raw counts after a fast search of the playout cap).  Needs forced playouts on."""
+        out = self.empty((self.num_games, 7), torch.int32)
+        self._check(self.lib.az_policy_targets(self.h, _ptr(out), _stream()), "az_policy_targets")
+        return out[: self.n_active]
+
+    def forced_stats(self) -> dict:
+        """Root selections the forcing rule decided, forced searches that ended in a move, visits pruned from their counts and
+        children pruned to 0 - totals since creation / `reset_stats`."""
+        st = AzForcedStats()
+        self._check(self.lib.az_get_forced_stats(self.h, C.byref(st), _stream()), "az_get_forced_stats")
+        return {n: int(getattr(st, n)) for n, _ in AzForcedStats._fields_}
 
     def run_simulations(self, num_sims: int, eval_kind: int):
         self._check(self.lib.az_run_simulations(self.h, int(num_sims), int(eval_kind), _stream()), "az_run_simulations")

@@ -26,8 +26,9 @@ class EpisodeGenerator:
         """`sampling_moves` = n: the first n plies of every game are sampled from the visit counts as in the reference, later
         ones play the most visited move (lowest column on ties; `num_sampling_moves` of DeepMind's AlphaZero pseudocode).  The
         uniform of every (step, slot) is still drawn, so NumPy's global stream advances exactly as without it.  None = off.
-        Root noise, symmetric leaf evaluation, subtree reuse and playout cap randomization come through `search_kwargs`
-        (`root_noise=RootNoise(...)`, `symmetric=True`, `subtree_reuse=True`, `playout_cap=PlayoutCap(...)`: see `AlphaZeroSearch`).
+        Root noise, symmetric leaf evaluation, subtree reuse, playout cap randomization and forced playouts come through
+        `search_kwargs` (`root_noise=RootNoise(...)`, `symmetric=True`, `subtree_reuse=True`, `playout_cap=PlayoutCap(...)`,
+        `forced_playouts=ForcedPlayouts(...)`: see `AlphaZeroSearch`).
         With the playout cap an episode holds the samples of its full searches only, possibly none; it still counts as an episode."""
         self.sampling_moves = sampling_moves
         self.search = AlphaZeroSearch(model=model, num_simulations=num_simulations, exploration_weight=exploration_weight,

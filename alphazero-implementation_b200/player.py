@@ -54,6 +54,9 @@ class AlphaZeroPlayer(Player):
     `symmetric=True`), and an `Arena` plays through its agents' searches."""
 
     def __init__(self, model, *, mcts_simulation: int = 100, temperature: float = 1.0, **search_kwargs) -> None:
+        if search_kwargs.get("forced_playouts") is not None:
+            raise ValueError("forced_playouts is a self-play option: the player picks its move from the raw root visit counts, and "
+                             "those of a forced search are not a move policy")
         self.model = model
         self.mcts_simulation = mcts_simulation
         self.temperature = temperature
@@ -163,6 +166,8 @@ def elo_ladder(models: dict, initial_state: State, games_per_pair: int = 2, mcts
     """Round robin over named models / checkpoints (src/elo.ipynb#cell4), every pairing played as a batched `Arena`, ratings
     updated game by game from 1500."""
     ratings: dict = defaultdict(lambda: 1500)
+    if search_kwargs.get("forced_playouts") is not None:
+        raise ValueError("forced_playouts is a self-play option: the ladder's players pick their moves from raw root visit counts")
     players = {name: AlphaZeroPlayer(m, mcts_simulation=mcts_simulation, temperature=temperature, **search_kwargs) for name, m in models.items()}
     for n1, n2 in combinations(list(models), 2):
         res = Arena(players[n1], players[n2], initial_state).play(games_per_pair)

@@ -108,6 +108,16 @@ class PlayoutCap:
     visit_budget: bool = False
 
 
+@dataclass(frozen=True)
+class ForcedPlayouts:
+    """Forced playouts and policy target pruning of the self-play searches (KataGo; `Engine.set_forced_playouts`): every root
+    child c gets at least about sqrt(k P(c) (N_root - 1)) visits, so that a move the root noise favours is actually explored, and
+    the recorded policy target (and the move played) takes those extra visits back out as far as PUCT would not have chosen them.
+    The playout cap's fast searches are not forced.  k = 0 gives the same results as off.  Off (None) by default."""
+
+    k: float = 2.0
+
+
 class _GraphedStep:
     """The simulation loop of the network-in-the-loop path, optionally replayed as a CUDA graph.
 
@@ -216,7 +226,7 @@ class AlphaZeroSearch:
                  lanes_per_tree: int = 0, inference_dtype: torch.dtype | None = None, use_cuda_graph: bool = True,
                  use_tensor_core_kernels: bool = True, trunk_variant: int | None = None, eval_cache: bool | int = True,
                  root_noise: RootNoise | None = None, symmetric: bool = False, subtree_reuse: bool | int = False,
-                 playout_cap: PlayoutCap | None = None):
+                 playout_cap: PlayoutCap | None = None, forced_playouts: ForcedPlayouts | None = None):
         """`eval_cache`: serve repeated leaf positions from the engine's evaluation cache (`Engine.set_eval_cache`) when the
         evaluator's outputs depend on the position alone (`InferenceNet.position_only_outputs`); same results, fewer evaluator rows.
         True = a table sized for the engine, False = off, an int = log2 of its entry count.
@@ -231,8 +241,11 @@ class AlphaZeroSearch:
         4 num_simulations, an int = max_root_visits, False (default) = every move step starts from a fresh root, as the reference
         does.  `run_simulations(nodes)` always starts from the given fresh roots.
         `playout_cap`: the self-play move steps run full or fast searches (`PlayoutCap`) and record only the full ones as samples;
-        None (default) = every search is full.  `run_simulations(nodes)` always runs full searches."""
+        None (default) = every search is full.  `run_simulations(nodes)` always runs full searches.
+        `forced_playouts`: the self-play move steps force root visits and record (and play from) the pruned counts
+        (`ForcedPlayouts`); None (default) = off.  `run_simulations(nodes)` always searches unforced."""
         self.symmetric = bool(symmetric)
+        self.forced_playouts = forced_playouts
         self.playout_cap = playout_cap
         self.subtree_reuse = subtree_reuse
         self.inference_model = model.get_inference_clone()
@@ -321,10 +334,11 @@ class AlphaZeroSearch:
         reuse = 1 if self.max_root_visits else 0  # k_reroot after k_sample_moves
         cap = self.playout_cap is not None
         redraw = 1 if cap and reuse else 0  # k_cap_draw after k_reroot (without reuse k_sample_moves draws the next budgets itself)
+        forced = self.forced_playouts is not None
         if self._mode == "builtin":
-            # one k_run_sims per run, the last one with the move fused in - unless the greedy cutoff, subtree reuse, the playout cap (or
-            # a search of one simulation with noise) leaves the move to k_sample_moves
-            return len(runs) + noise + (1 if greedy or reuse or cap or noise and S == 1 else 0) + reuse + redraw
+            # one k_run_sims per run, the last one with the move fused in - unless the greedy cutoff, subtree reuse, the playout cap,
+            # forced playouts (or a search of one simulation with noise) leave the move to k_sample_moves
+            return len(runs) + noise + (1 if greedy or reuse or cap or forced or noise and S == 1 else 0) + reuse + redraw
         # per run of n: k_select; n - 1 x (evaluator or gather, k_expand_select); evaluator, k_expand_backup.  Then k_root_noise
         # between the runs and k_sample_moves.  When the evaluator walks the compacted leaf list: one k_compact_leaves after
         # every k_select (the later lists come out of k_expand_select) or, AZ_COMPACT_FUSED=0, one per selection
@@ -369,6 +383,18 @@ class AlphaZeroSearch:
             engine.set_playout_cap(None)
         else:
             engine.set_playout_cap(*want)
+        if switched and self._graphed is not None and self._graphed.engine is engine:
+            self._graphed = None
+
+    def _configure_forced(self, engine: Engine, on: bool = True):
+        """before a search and any capture of its CUDA graph (switching the mode on or off changes the kernels); `on=False` for the
+        searches outside self-play"""
+        fp = self.forced_playouts
+        want = float(fp.k) if on and fp is not None else None
+        if engine.forced_playouts == want:
+            return
+        switched = (engine.forced_playouts is None) != (want is None)
+        engine.set_forced_playouts(want)
         if switched and self._graphed is not None and self._graphed.engine is engine:
             self._graphed = None
 
@@ -422,6 +448,7 @@ class AlphaZeroSearch:
         (`k_reroot`) for the next step's search."""
         self._configure_reuse(engine)
         self._configure_cap(engine)
+        self._configure_forced(engine)
         if self._mode == "builtin":
             kind = self.inference_model.az_builtin_eval_kind
             self._configure_noise(engine)
@@ -492,6 +519,7 @@ class AlphaZeroSearch:
         bb1 = np.array([nd.state.bb1 for nd in current_nodes], np.uint64)
         pl = np.array([nd.state.player for nd in current_nodes], np.uint8)
         eng.set_roots(bb0, bb1, pl)
+        self._configure_forced(eng, on=False)
         self.simulate(eng)
         st = {k: v.cpu().numpy() for k, v in eng.root_stats().items()}
         if (st["err"] == TREE_ROOT_ENDED).any():

@@ -348,6 +348,43 @@ typedef struct az_cap_stats {
 /* totals since az_create / az_reset_stats.  Synchronises. */
 int32_t az_get_cap_stats(az_engine *h, az_cap_stats *out_host, void *stream);
 
+/* Forced playouts and policy target pruning (KataGo, Wu 2019 section 3.1): every root child gets a minimum number of visits, and
+ * those visits are taken back out of the recorded policy target as far as PUCT would not have chosen them anyway.  All arithmetic
+ * is fp64 with one rounding per operation (RN), as in the PUCT score.
+ *   Forcing, at the root only: with m = N_root - 1 (the root's child visits, retained visits of subtree reuse included) and P(c)
+ *   the child's stored fp32 prior (after root noise), legal child c is forced when RN(N(c) * N(c)) < RN(RN(k * P(c)) * m).  Forced
+ *   children outrank every PUCT score; among several the lowest column wins.  Below the root nothing changes.  Forcing applies to
+ *   every search on the engine while the mode is on (az_run_simulations, the selection kernels, az_run_move_step), except the fast
+ *   searches of the playout cap.
+ *   Pruning of a forced search's counts (c_puct is the engine's, sq = RN(sqrt(N_root))): c* = the most visited legal child, lowest
+ *   column on ties, keeps N(c*); s* = PUCT(c*) from its real statistics.  For every other legal child with N(c) > 0: q = W/N (0 when
+ *   W = 0) stays the real mean, u(n) = RN(RN(RN(c_puct * P) * sq) / (1 + n)), n_f = the least n >= 0 with RN(n * n) >=
+ *   RN(RN(k * P) * m).  From N' = N(c): while N(c) - N' < n_f, N' > 0 and RN(q + u(N' - 1)) < s*, N' -= 1.  Then a child other than
+ *   c* left with exactly 1 visit goes to 0.  Roots with m = 0 keep their counts, and so does every root when k = 0 (nothing was
+ *   forced): k = 0 gives the same bits as the mode off.  The loop follows the paper one playout at a time; KataGo's closed form may
+ *   round differently.
+ *   The pruned counts N' are the sample the game log and the episode ring record, and az_sample_moves draws the move from them
+ *   (p = N' / sum N' through the same cumsum / normalise / searchsorted-right; the greedy move is c* either way).  The tree keeps its
+ *   real statistics (subtree reuse retains them).  Under the playout cap fast plies are played from their raw counts and, as
+ *   always, recorded nowhere.  While the mode is on az_run_move_step runs as the search followed by az_sample_moves. */
+typedef struct az_forced_playouts {
+    double k;  /* finite, [0, 1024]; KataGo uses 2 */
+} az_forced_playouts;
+/* cfg NULL = off (the default).  AZ_E_INVALID for k out of range, AZ_E_STATE while a selection's leaves wait for their expansion.
+ * The kernels a launch uses change with the switch (capture a simulation graph after it). */
+int32_t az_set_forced_playouts(az_engine *h, const az_forced_playouts *cfg);
+/* counts[num_games][7] i32 (device): the pruned counts N' of the current roots by column, what az_sample_moves would record (raw
+ * counts for a fast search of the playout cap, 0 for slots without a searched root).  AZ_E_STATE while the mode is off. */
+int32_t az_policy_targets(az_engine *h, int32_t *counts, void *stream);
+typedef struct az_forced_stats {
+    uint64_t forced_selections;  /* root selections the forcing rule decided */
+    uint64_t forced_searches;    /* forced searches that ended in a move (az_sample_moves) */
+    uint64_t visits_pruned;      /* sum of N - N' over those moves */
+    uint64_t children_zeroed;    /* children that went from N > 0 to N' = 0 */
+} az_forced_stats;
+/* totals since az_create / az_reset_stats.  Synchronises. */
+int32_t az_get_forced_stats(az_engine *h, az_forced_stats *out_host, void *stream);
+
 /* number of finished episodes / samples waiting in the ring.  Synchronises on `stream`. */
 int32_t az_episode_counts(az_engine *h, int64_t *n_episodes_host, int64_t *n_samples_host, void *stream);
 /* copy the ring out (device buffers sized from az_episode_counts) and empty it.  Episodes appear in
