@@ -109,6 +109,11 @@ class AzForcedPlayouts(C.Structure):
     _fields_ = [("k", C.c_double)]
 
 
+class AzOpenings(C.Structure):
+    _fields_ = [("bb0", C.c_void_p), ("bb1", C.c_void_p), ("player", C.c_void_p), ("n_positions", C.c_int32), ("min_plies", C.c_int32),
+                ("max_plies", C.c_int32), ("seed", C.c_uint64), ("slot_offset", C.c_int64)]
+
+
 class AzForcedStats(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in ("forced_selections", "forced_searches", "visits_pruned", "children_zeroed")]
 
@@ -195,6 +200,8 @@ SIGNATURES = {
     "az_set_forced_playouts": (I32, [P, C.POINTER(AzForcedPlayouts)]),
     "az_policy_targets": (I32, [P, P, P]),
     "az_get_forced_stats": (I32, [P, C.POINTER(AzForcedStats), P]),
+    "az_set_openings": (I32, [P, C.POINTER(AzOpenings)]),
+    "az_opening_positions": (I32, [P, I64, I64, C.c_uint32, P, P, P, P]),
     "az_leaf_mirror": (I32, [P, C.POINTER(P)]),
     "az_mirror_states": (I32, [P, P, P, P, I64, P, P, P]),
     "az_trunk_weight_bytes": (I64, [I32]),

@@ -1623,6 +1623,91 @@ __global__ void __launch_bounds__(256) k_cap_draw(Arena a, int n, CapArgs cp, ui
     cap_set(cp, t, all_full || cap_draw_full(cp, t, step), a.M[(size_t)t * a.cap].x);
 }
 
+// Opening positions of self-play games (az_set_openings; the rule is in include/az_engine.h).  The game of global slot g that starts
+// at move step s draws X_j = Philox(key = seed, counter {g lo, g hi, s, OPEN_TAG | j}): X_0 picks the base position of the set and
+// the number of random plies, X_j (j >= 1) the column of ply j among the legal columns whose drop neither wins nor fills the board.
+// OPEN_TAG | j with j <= 40 is neither CAP_TAG nor a noise counter (column << 24 | attempt, column <= 6).
+constexpr uint32_t OPEN_TAG = 0xA0000000u;
+constexpr int OPEN_MAX_PLIES = 40;
+
+struct OpenArgs {
+    const uint64_t *bb0, *bb1;  // the position set, n_positions entries (engine-owned copy)
+    const uint8_t *player;
+    unsigned long long seed;
+    long long slot_offset;      // global index of the engine's slot 0
+    int n_positions, min_plies, max_plies;
+};
+
+__device__ __forceinline__ uint4 open_draw(const OpenArgs &op, unsigned long long g, uint32_t s, uint32_t j) {
+    return philox4x32_10(make_uint4((uint32_t)g, (uint32_t)(g >> 32), s, OPEN_TAG | j), make_uint2((uint32_t)op.seed, (uint32_t)(op.seed >> 32)));
+}
+
+// the opening of the game (g, s) from the base (b0, b1, pl) = the az_reset_games position when the set is empty; a base that has
+// ended gets no plies
+__device__ __forceinline__ void opening_of(const OpenArgs &op, unsigned long long g, uint32_t s, uint64_t &b0, uint64_t &b1, int &pl) {
+    const uint4 x0 = open_draw(op, g, s, 0u);
+    if (op.n_positions > 0) {
+        const int i = (int)(((unsigned long long)x0.x * (unsigned long long)op.n_positions) >> 32);
+        b0 = op.bb0[i];
+        b1 = op.bb1[i];
+        pl = op.player[i];
+    }
+    const int r = op.min_plies + (int)(((unsigned long long)x0.y * (unsigned long long)(op.max_plies - op.min_plies + 1)) >> 32);
+    if (c4::terminal_of(b0, b1).ended) return;
+    for (int j = 1; j <= r; ++j) {
+        const uint64_t occ = b0 | b1;
+        const uint32_t legal = c4::legal_mask(occ);
+        uint32_t cand = 0u;
+#pragma unroll
+        for (int c = 0; c < 7; ++c) {
+            const uint64_t bit = c4::drop_bit(occ, c);
+            if (((legal >> c) & 1u) && !c4::has4((pl ? b1 : b0) | bit) && !c4::is_full(occ | bit)) cand |= 1u << c;
+        }
+        if (!cand) return;
+        const uint4 x = open_draw(op, g, s, (uint32_t)j);
+        const int col = c4::nth_legal_column(cand, (int)(((unsigned long long)x.x * (unsigned long long)__popc(cand)) >> 32));
+        const uint64_t bit = c4::drop_bit(occ, col);
+        if (pl == 0) b0 |= bit; else b1 |= bit;
+        pl ^= 1;
+    }
+}
+
+// One thread per slot t < n: the opening of the game of global slot g0 + t starting at move step `step`, written to (o0, o1, opl)[t]
+// where flags[t] != 0 (flags NULL = every slot).  The engine's call writes the roots (o* = root_bb0 / root_bb1 / root_player, g0 =
+// slot_offset) of slots whose tree is already fresh: after az_reset_games, and of the games k_sample_moves recycled (k_reroot skips
+// them and k_cap_draw reads only the fresh root's visit count, so the order of those launches does not matter); az_opening_positions
+// writes caller arrays.
+__global__ void __launch_bounds__(256)
+k_openings(long long n, const uint8_t *__restrict__ flags, OpenArgs op, unsigned long long g0, uint32_t step, uint64_t init0, uint64_t init1,
+           int initpl, uint64_t *o0, uint64_t *o1, uint8_t *opl) {
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n || (flags && !flags[t])) return;
+    uint64_t b0 = init0, b1 = init1;
+    int pl = initpl;
+    opening_of(op, g0 + (unsigned long long)t, step, b0, b1, pl);
+    o0[t] = b0;
+    o1[t] = b1;
+    opl[t] = (uint8_t)pl;
+}
+
+// az_set_openings' check of the set: *first_bad = min over bad entries of index << 3 | reason (1 overlapping boards, 2 bits off the
+// board, 3 a stone above an empty cell, 4 player not 0 / 1, 5 ended)
+__global__ void __launch_bounds__(256)
+k_check_openings(const uint64_t *__restrict__ bb0, const uint64_t *__restrict__ bb1, const uint8_t *__restrict__ player, int n,
+                 unsigned long long *first_bad) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    const uint64_t b0 = bb0[t], b1 = bb1[t], occ = b0 | b1;
+    bool holes = false;
+#pragma unroll
+    for (int c = 0; c < 7; ++c) {
+        const uint64_t col = (occ >> (c4::STRIDE * c)) & 0x7Full;
+        holes |= (col & (col + 1)) != 0;  // a column's stones are the bits 0 .. h-1
+    }
+    const int reason = (b0 & b1) ? 1 : (occ & ~c4::BOARD) ? 2 : holes ? 3 : player[t] > 1 ? 4 : c4::terminal_of(b0, b1).ended ? 5 : 0;
+    if (reason) atomicMin(first_bad, (unsigned long long)t << 3 | (unsigned long long)reason);
+}
+
 // ------------------------------------------------------------------------------------------------
 // roots / results
 __global__ void __launch_bounds__(256)
@@ -2314,6 +2399,9 @@ struct az_engine {
     bool forced_on;              // az_set_forced_playouts: searches force root children and moves prune their counts (the FORCED kernels)
     double forced_k;
     unsigned long long *fstats;  // [E][FS_N] (allocated with the first az_set_forced_playouts)
+    bool open_on;                // az_set_openings: games start from an opening (k_openings after az_reset_games and k_sample_moves)
+    OpenArgs open;               // its configuration and the engine's copy of the position set
+    uint8_t *open_finished;      // [E] k_sample_moves' finished flags when the caller passes none (allocated with the first az_set_openings)
     int64_t bytes;
     int64_t launches;
     unsigned long long *d_tot;   // [16] stats totals (device)
@@ -2440,6 +2528,14 @@ int launch_encode(az_engine *h, const uint64_t *bb0, const uint64_t *bb1, const 
 int launch_cap_draw(az_engine *h, uint32_t step, bool all_full, cudaStream_t st) {
     k_cap_draw<<<blocks_for(h->a.E, 256), 256, 0, st>>>(h->a, h->a.E, h->cap, step, all_full ? 1 : 0);
     AZ_LAUNCH_CHECK(h, "k_cap_draw");
+    return AZ_OK;
+}
+
+// the openings of the games that start at move step `step` on the first n slots: those flagged in `flags` (NULL = every slot)
+int launch_openings(az_engine *h, int n, const uint8_t *flags, uint32_t step, cudaStream_t st) {
+    k_openings<<<blocks_for(n, 256), 256, 0, st>>>(n, flags, h->open, (unsigned long long)h->open.slot_offset, step, h->init0, h->init1,
+                                                   h->initpl, h->a.root_bb0, h->a.root_bb1, h->a.root_player);
+    AZ_LAUNCH_CHECK(h, "k_openings");
     return AZ_OK;
 }
 
@@ -2751,6 +2847,8 @@ int32_t az_reset_games(az_engine *h, uint64_t init_bb0, uint64_t init_bb1, int32
     h->init0 = init_bb0;
     h->init1 = init_bb1;
     h->initpl = init_player;
+    if (h->open_on)  // every game starts at move step 0
+        if (int rc = launch_openings(h, E, nullptr, 0u, S(stream))) return rc;
     h->have_init = true;
     h->n_active = E;
     h->step = 0;
@@ -2809,9 +2907,9 @@ int32_t az_run_move_step(az_engine *h, int32_t num_sims, int32_t eval_kind, cons
     if (!uniforms) return fail(h, AZ_E_INVALID, "%s", "az_run_move_step: null uniforms");
     if (!h->have_init) return fail(h, AZ_E_STATE, "%s", "az_run_move_step: call az_reset_games first");
     if (num_sims < 1) return fail(h, AZ_E_INVALID, "%s", "az_run_move_step: num_sims < 1");
-    // the greedy rule, subtree reuse, the playout cap and policy target pruning live in k_sample_moves (+ k_reroot) only: the search
-    // (its hot prefix written back), then the move
-    if (h->greedy_from >= 0 || h->reuse_v > 0 || h->cap_on || h->forced_on) {
+    // the greedy rule, subtree reuse, the playout cap, policy target pruning and the openings of recycled slots live in k_sample_moves
+    // (+ k_reroot, k_openings) only: the search (its hot prefix written back), then the move
+    if (h->greedy_from >= 0 || h->reuse_v > 0 || h->cap_on || h->forced_on || h->open_on) {
         const int32_t rc = run_sims_impl(h, num_sims, eval_kind, nullptr, nullptr, false, stream);
         if (rc != AZ_OK) return rc;
         return az_sample_moves(h, uniforms, finished, stream);
@@ -3046,6 +3144,7 @@ int32_t az_sample_moves(az_engine *h, const double *uniforms, uint8_t *finished,
     const int n = h->n_active;
     const bool reuse = h->reuse_v > 0;
     const bool budget = h->cap_on;
+    if (h->open_on && !finished) finished = h->open_finished;  // k_openings reads which games ended
     with_flags([&](auto GREEDY, auto REUSE, auto BUDGET, auto FORCED) {
         k_sample_moves<GREEDY, REUSE, BUDGET, FORCED><<<blocks_for(n, 128), 128, 0, S(stream)>>>(
             h->a, n, uniforms, finished, h->step, h->init0, h->init1, h->initpl, GREEDY ? h->greedy_from : -1, REUSE ? h->reroot : nullptr,
@@ -3057,6 +3156,8 @@ int32_t az_sample_moves(az_engine *h, const double *uniforms, uint8_t *finished,
         if (budget)  // the next search's budget counts from the visits the new root kept
             if (int rc = launch_cap_draw(h, (uint32_t)h->step + 1u, false, S(stream))) return rc;
     }
+    if (h->open_on)  // a recycled slot's game starts at the next move step
+        if (int rc = launch_openings(h, n, finished, (uint32_t)h->step + 1u, S(stream))) return rc;
     h->step++;
     roots_replaced(h);
     return AZ_OK;
@@ -3532,6 +3633,101 @@ int32_t az_get_forced_stats(az_engine *h, az_forced_stats *out, void *stream) {
     out->forced_searches = tot[FS_SEARCHES];
     out->visits_pruned = tot[FS_PRUNED];
     out->children_zeroed = tot[FS_ZEROED];
+    return AZ_OK;
+}
+
+int32_t az_set_openings(az_engine *h, const az_openings *cfg) {
+    if (!h) return AZ_E_INVALID;
+    if (h->sel_pending) return fail(h, AZ_E_STATE, "%s", "az_set_openings: a selection's leaves wait for their expansion");
+    if (!cfg) {
+        h->open_on = false;
+        return AZ_OK;
+    }
+    const int n = cfg->n_positions;
+    if (n < 0 || (n > 0 && (!cfg->bb0 || !cfg->bb1 || !cfg->player)))
+        return fail(h, AZ_E_INVALID, "%s", "az_set_openings: n_positions must be >= 0, with non-null positions when > 0");
+    if (cfg->min_plies < 0 || cfg->min_plies > cfg->max_plies || cfg->max_plies > OPEN_MAX_PLIES)
+        return fail(h, AZ_E_INVALID, "%s", "az_set_openings: need 0 <= min_plies <= max_plies <= 40");
+    if (cfg->slot_offset < 0 || cfg->slot_offset > ((int64_t)1 << 62))
+        return fail(h, AZ_E_INVALID, "%s", "az_set_openings: slot_offset must be in [0, 2^62]");
+    if (int rc = set_device(h)) return rc;
+    uint64_t *b0 = nullptr, *b1 = nullptr;
+    uint8_t *pl = nullptr;
+    unsigned long long *bad = nullptr;
+    auto release = [&]() {
+        if (b0) dev_free(h, b0, (size_t)n * sizeof(uint64_t));
+        if (b1) dev_free(h, b1, (size_t)n * sizeof(uint64_t));
+        if (pl) dev_free(h, pl, (size_t)n);
+        if (bad) dev_free(h, bad, sizeof(unsigned long long));
+    };
+    int rc = AZ_OK;
+    if (!h->open_finished) rc = dev_alloc(h, &h->open_finished, h->a.E);
+    if (n > 0) {
+        if (rc == AZ_OK) rc = dev_alloc(h, &b0, n);
+        if (rc == AZ_OK) rc = dev_alloc(h, &b1, n);
+        if (rc == AZ_OK) rc = dev_alloc(h, &pl, n);
+        if (rc == AZ_OK) rc = dev_alloc(h, &bad, 1);
+        // the copies and the check run on the legacy stream and end in a synchronising read: the caller's buffers are borrowed only
+        // for this call
+        cudaError_t e = cudaSuccess;
+        unsigned long long first = ~0ull;
+        if (rc == AZ_OK) e = cudaMemcpy(b0, cfg->bb0, (size_t)n * sizeof(uint64_t), cudaMemcpyDefault);
+        if (rc == AZ_OK && e == cudaSuccess) e = cudaMemcpy(b1, cfg->bb1, (size_t)n * sizeof(uint64_t), cudaMemcpyDefault);
+        if (rc == AZ_OK && e == cudaSuccess) e = cudaMemcpy(pl, cfg->player, (size_t)n, cudaMemcpyDefault);
+        if (rc == AZ_OK && e == cudaSuccess) e = cudaMemcpy(bad, &first, sizeof first, cudaMemcpyHostToDevice);
+        if (rc == AZ_OK && e == cudaSuccess) {
+            k_check_openings<<<blocks_for(n, 256), 256>>>(b0, b1, pl, n, bad);
+            e = cudaGetLastError();
+            if (e == cudaSuccess) h->launches++;
+        }
+        if (rc == AZ_OK && e == cudaSuccess) e = cudaMemcpy(&first, bad, sizeof first, cudaMemcpyDeviceToHost);
+        if (rc == AZ_OK && e != cudaSuccess) rc = fail(h, AZ_E_CUDA, "az_set_openings: %s", cudaGetErrorString(e));
+        if (rc == AZ_OK && first != ~0ull) {
+            static const char *why[] = {"", "the boards overlap", "a stone lies off the board", "a stone lies above an empty cell",
+                                        "player is not 0 or 1", "the game has ended"};
+            char msg[160];
+            snprintf(msg, sizeof msg, "position %llu: %s", first >> 3, why[first & 7u]);
+            rc = fail(h, AZ_E_INVALID, "az_set_openings: bad position set, %s", msg);
+        }
+        if (bad) {
+            dev_free(h, bad, sizeof(unsigned long long));
+            bad = nullptr;
+        }
+    }
+    if (rc != AZ_OK) {
+        release();
+        return rc;
+    }
+    OpenArgs &op = h->open;
+    if (op.n_positions > 0) {  // the previous set
+        dev_free(h, const_cast<uint64_t *>(op.bb0), (size_t)op.n_positions * sizeof(uint64_t));
+        dev_free(h, const_cast<uint64_t *>(op.bb1), (size_t)op.n_positions * sizeof(uint64_t));
+        dev_free(h, const_cast<uint8_t *>(op.player), (size_t)op.n_positions);
+    }
+    op.bb0 = b0;
+    op.bb1 = b1;
+    op.player = pl;
+    op.n_positions = n;
+    op.min_plies = cfg->min_plies;
+    op.max_plies = cfg->max_plies;
+    op.seed = cfg->seed;
+    op.slot_offset = cfg->slot_offset;
+    h->open_on = true;
+    return AZ_OK;
+}
+
+int32_t az_opening_positions(az_engine *h, int64_t first_slot, int64_t n, uint32_t step, uint64_t *out_bb0, uint64_t *out_bb1,
+                             uint8_t *out_player, void *stream) {
+    if (!h) return AZ_E_INVALID;
+    if (!h->open_on) return fail(h, AZ_E_STATE, "%s", "az_opening_positions: openings are off (az_set_openings)");
+    if (first_slot < 0 || n < 0 || first_slot > ((int64_t)1 << 62) || n > INT32_MAX)
+        return fail(h, AZ_E_INVALID, "%s", "az_opening_positions: need first_slot in [0, 2^62] and 0 <= n < 2^31");
+    if (n > 0 && (!out_bb0 || !out_bb1 || !out_player)) return fail(h, AZ_E_INVALID, "%s", "az_opening_positions: null output");
+    if (n == 0) return AZ_OK;
+    if (int rc = set_device(h)) return rc;
+    k_openings<<<blocks_for(n, 256), 256, 0, S(stream)>>>(n, nullptr, h->open, (unsigned long long)first_slot, step, h->init0, h->init1,
+                                                          h->initpl, out_bb0, out_bb1, out_player);
+    AZ_LAUNCH_CHECK(h, "k_openings");
     return AZ_OK;
 }
 

@@ -11,7 +11,9 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import AzCapStats, AzConfig, AzEvalCacheStats, AzForcedPlayouts, AzForcedStats, AzPlayoutCap, AzReuseStats, AzRootNoise, AzStats
+from ._lib import (AzCapStats, AzConfig, AzEvalCacheStats, AzForcedPlayouts, AzForcedStats, AzOpenings, AzPlayoutCap, AzReuseStats,
+                   AzRootNoise, AzStats)
+from .openings import Openings, position_arrays
 
 EVAL_UNIFORM = 1
 EVAL_HASH = 2
@@ -102,6 +104,7 @@ class Engine:
         self.subtree_reuse = 0  # max_root_visits, 0 = off
         self.playout_cap = None  # (fast_sims, p_full, seed, slot_offset, visit_budget) while the playout cap is on
         self.forced_playouts = None  # k while forced playouts and policy target pruning are on
+        self.openings = None  # the `Openings` while games start from openings
         self.tree_capacity = self.lib.az_tree_capacity(self.h)
 
     # -- plumbing --------------------------------------------------------------------------------
@@ -368,6 +371,35 @@ class Engine:
         st = AzForcedStats()
         self._check(self.lib.az_get_forced_stats(self.h, C.byref(st), _stream()), "az_get_forced_stats")
         return {n: int(getattr(st, n)) for n, _ in AzForcedStats._fields_}
+
+    def set_openings(self, openings: Openings | None):
+        """Opening positions (`az_set_openings`): every self-play game that starts after this call - all of them at `reset_games`,
+        then each slot `sample_moves` recycles - starts from the opening the rule of `Openings` draws for its (global slot, move step),
+        a fresh tree on it.  The position set is checked (legal, not ended) and copied to the device.  None = off (the default)."""
+        if openings is None:
+            self._check(self.lib.az_set_openings(self.h, None), "az_set_openings")
+            self.openings = None
+            return
+        keep = []
+        n = 0
+        if openings.positions is not None:
+            bb0, bb1, pl = position_arrays(openings.positions)
+            n = len(bb0)
+            keep = [self._dev(bb0, torch.int64), self._dev(bb1, torch.int64), self._dev(pl, torch.uint8)]
+        ptrs = [_ptr(t) for t in keep] if n else [None, None, None]
+        cfg = AzOpenings(*ptrs, n, int(openings.min_plies), int(openings.max_plies), int(openings.seed) & (2**64 - 1),
+                         int(openings.slot_offset))
+        torch.cuda.current_stream(self.device).synchronize()  # the engine copies the set on the legacy stream
+        self._check(self.lib.az_set_openings(self.h, C.byref(cfg)), "az_set_openings")
+        self.openings = openings
+
+    def opening_positions(self, first_slot: int, n: int, step: int) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """The openings of the games of global slots first_slot .. first_slot + n - 1 that start at move step `step` under the current
+        `set_openings` (a query: nothing changes) -> (bb0 int64, bb1 int64, player uint8) device tensors of n entries."""
+        out = (self.empty(n, torch.int64), self.empty(n, torch.int64), self.empty(n, torch.uint8))
+        self._check(self.lib.az_opening_positions(self.h, int(first_slot), int(n), int(step), *(_ptr(t) for t in out), _stream()),
+                    "az_opening_positions")
+        return out
 
     def run_simulations(self, num_sims: int, eval_kind: int):
         self._check(self.lib.az_run_simulations(self.h, int(num_sims), int(eval_kind), _stream()), "az_run_simulations")

@@ -16,21 +16,25 @@ import torch
 from .engine import EpisodeBatch
 from .episode import Episode, episodes_from_batch
 from .game import State
+from .openings import Openings
 from .search import AlphaZeroSearch
 
 
 class EpisodeGenerator:
     def __init__(self, *, model, num_simulations: int, num_episodes: int, game_initial_state: State,
                  exploration_weight: float = 1.0, uniform_source: Callable[[int, int], np.ndarray] | None = None,
-                 sampling_moves: int | None = None, **search_kwargs):
+                 sampling_moves: int | None = None, openings: Openings | None = None, **search_kwargs):
         """`sampling_moves` = n: the first n plies of every game are sampled from the visit counts as in the reference, later
         ones play the most visited move (lowest column on ties; `num_sampling_moves` of DeepMind's AlphaZero pseudocode).  The
         uniform of every (step, slot) is still drawn, so NumPy's global stream advances exactly as without it.  None = off.
         Root noise, symmetric leaf evaluation, subtree reuse, playout cap randomization and forced playouts come through
         `search_kwargs` (`root_noise=RootNoise(...)`, `symmetric=True`, `subtree_reuse=True`, `playout_cap=PlayoutCap(...)`,
         `forced_playouts=ForcedPlayouts(...)`: see `AlphaZeroSearch`).
-        With the playout cap an episode holds the samples of its full searches only, possibly none; it still counts as an episode."""
+        With the playout cap an episode holds the samples of its full searches only, possibly none; it still counts as an episode.
+        `openings` (`Openings`): every game starts from an opening drawn for its (slot_offset + slot, move step) - a position of the
+        set or the initial state, then a few random plies - instead of the initial state; its first sample is that opening.  None = off."""
         self.sampling_moves = sampling_moves
+        self.openings = openings
         self.search = AlphaZeroSearch(model=model, num_simulations=num_simulations, exploration_weight=exploration_weight,
                                       **search_kwargs)
         self.num_episodes = int(num_episodes)
@@ -61,6 +65,8 @@ class EpisodeGenerator:
         E = self.num_episodes
         eng = self.search.engine_for(E, exact=True)  # the slots are the games: an engine grown by a larger run_simulations call is replaced
         eng.set_greedy_from(self.sampling_moves)
+        if eng.openings is not self.openings:
+            eng.set_openings(self.openings)
         if reset:
             eng.reset_games(initial_state.bb0, initial_state.bb1, initial_state.player)
         elif eng.n_active != E:

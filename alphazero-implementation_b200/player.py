@@ -20,6 +20,7 @@ from itertools import combinations
 import numpy as np
 
 from .game import Action, State
+from .openings import Openings, position_arrays
 from .search import AlphaZeroSearch, Node
 
 
@@ -108,41 +109,80 @@ def play_game(agent1: Player, agent2: Player, initial_state: State) -> float:
 
 
 class Arena:
-    """G games between two agents, all at once; half of them with agent A moving first, half with agent B."""
+    """G games between two agents, all at once; half of them with agent A moving first, half with agent B.
 
-    def __init__(self, agent_a: AlphaZeroPlayer, agent_b: AlphaZeroPlayer, initial_state: State):
-        self.a, self.b, self.initial_state = agent_a, agent_b, initial_state
+    `openings` (optional): the games start from opening positions instead of `initial_state`, each opening played twice, once with
+    A and once with B as the side to move at the opening - the standard remedy for deterministic agents (temperature 0), which
+    otherwise play the same two games over and over.  A list of `State`s or a (bb0, bb1, player) array triple (for example from
+    `distinct_openings`): games 2i and 2i + 1 of `play` start from opening i mod K; or an `Openings`: opening i is then the one
+    `Engine.opening_positions` draws for slot i at move step 0 from `initial_state`."""
 
-    def _play_group(self, first: AlphaZeroPlayer, second: AlphaZeroPlayer, n: int) -> np.ndarray:
-        """n games with `first` as player 0 -> score of `first` per game."""
-        s0 = self.initial_state
-        bb0 = np.full(n, s0.bb0, np.uint64)
-        bb1 = np.full(n, s0.bb1, np.uint64)
-        pl = np.full(n, s0.player, np.uint8)
+    def __init__(self, agent_a: AlphaZeroPlayer, agent_b: AlphaZeroPlayer, initial_state: State, openings=None):
+        self.a, self.b, self.initial_state, self.openings = agent_a, agent_b, initial_state, openings
+
+    def _starts(self, n: int) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """the start positions of n colour-swapped pairs"""
+        op = self.openings
+        if isinstance(op, Openings):
+            eng = self.a.search.engine_for(1)
+            saved = eng.openings
+            s0 = self.initial_state
+            eng.set_openings(Openings(op.positions if op.positions is not None else [s0], op.min_plies, op.max_plies, op.seed, 0))
+            o0, o1, pl = (t.cpu().numpy() for t in eng.opening_positions(op.slot_offset, n, 0))
+            eng.set_openings(saved)
+            return o0.view(np.uint64), o1.view(np.uint64), pl
+        bb0, bb1, pl = position_arrays(op)
+        if len(bb0) == 0:
+            raise ValueError("Arena: empty opening set")
+        idx = np.arange(n) % len(bb0)
+        return bb0[idx], bb1[idx], pl[idx]
+
+    def _play_group(self, first: AlphaZeroPlayer, second: AlphaZeroPlayer, n: int, starts=None) -> np.ndarray:
+        """n games with `first` as player 0 from `initial_state` -> score of `first` per game.  `starts` = (bb0, bb1, player) of the
+        n games: each starts there, with `first` as its side to move."""
+        if starts is None:
+            s0 = self.initial_state
+            bb0, bb1, pl = np.full(n, s0.bb0, np.uint64), np.full(n, s0.bb1, np.uint64), np.full(n, s0.player, np.uint8)
+            first_pl = np.zeros(n, np.uint8)
+        else:
+            bb0, bb1, pl = (np.array(x) for x in starts)
+            first_pl = pl.copy()
+        fill = bb0.copy(), bb1.copy(), pl.copy()
         score = np.full(n, np.nan)
         live = np.ones(n, bool)
         rules = first.search.engine_for(n)
         while live.any():
             i0 = int(np.argmax(live))
-            mover = first if int(pl[i0]) == 0 else second  # every live game is at the same ply
-            # the batch keeps its size (one engine, one captured graph per agent): finished games sit at the initial position
-            cols = mover.play_many(np.where(live, bb0, s0.bb0), np.where(live, bb1, s0.bb1), np.where(live, pl, s0.player).astype(np.uint8))
+            mover = first if pl[i0] == first_pl[i0] else second  # every live game is at the same ply of its own start
+            # the batch keeps its size (one engine, one captured graph per agent): finished games sit at their start position
+            cols = mover.play_many(np.where(live, bb0, fill[0]), np.where(live, bb1, fill[1]), np.where(live, pl, fill[2]).astype(np.uint8))
             idx = np.nonzero(live)[0]
             nxt = {k: v.cpu().numpy() for k, v in rules.env_step(bb0[idx], bb1[idx], pl[idx], cols[idx]).items()}
             assert (nxt["status"] == 0).all()
             bb0[idx], bb1[idx], pl[idx] = nxt["bb0"].view(np.uint64), nxt["bb1"].view(np.uint64), nxt["player"]
             ended = nxt["ended"].astype(bool)
             r = nxt["reward"][ended]
-            score[idx[ended]] = np.where(r[:, 0] == r[:, 1], 0.5, np.where(r[:, 0] > r[:, 1], 1.0, 0.0))
+            mine = r[np.arange(len(r)), first_pl[idx[ended]]]  # the reward of the side `first` played
+            score[idx[ended]] = np.where(mine > 0, 1.0, np.where(mine < 0, 0.0, 0.5))
             live[idx[ended]] = False
         return score
 
     def play(self, num_games: int) -> dict:
-        """-> wins / draws / losses of agent A and its mean score."""
-        n1 = (num_games + 1) // 2
-        sa = self._play_group(self.a, self.b, n1)
-        sb = 1.0 - self._play_group(self.b, self.a, num_games - n1) if num_games > n1 else np.zeros(0)
-        s = np.concatenate([sa, sb])
+        """-> wins / draws / losses of agent A and its mean score.  With openings, games 2i (A to move at the opening) and 2i + 1 (B)
+        start from opening i and `scores` lists them in that order."""
+        if self.openings is not None:
+            k = (num_games + 1) // 2
+            starts = self._starts(k)
+            sa = self._play_group(self.a, self.b, k, starts)
+            nb = num_games - k
+            sb = 1.0 - self._play_group(self.b, self.a, nb, tuple(x[:nb] for x in starts)) if nb else np.zeros(0)
+            s = np.empty(num_games)
+            s[0::2], s[1::2] = sa, sb
+        else:
+            n1 = (num_games + 1) // 2
+            sa = self._play_group(self.a, self.b, n1)
+            sb = 1.0 - self._play_group(self.b, self.a, num_games - n1) if num_games > n1 else np.zeros(0)
+            s = np.concatenate([sa, sb])
         return dict(games=num_games, a_wins=int((s == 1).sum()), draws=int((s == 0.5).sum()), b_wins=int((s == 0).sum()),
                     a_score=float(s.mean()), scores=s)
 
@@ -162,15 +202,16 @@ def update_elo(rating1: int, rating2: int, score: float, K: int = 32) -> tuple[i
 
 
 def elo_ladder(models: dict, initial_state: State, games_per_pair: int = 2, mcts_simulation: int = 100, temperature: float = 0,
-               K: int = 32, **search_kwargs) -> dict:
+               K: int = 32, openings=None, **search_kwargs) -> dict:
     """Round robin over named models / checkpoints (src/elo.ipynb#cell4), every pairing played as a batched `Arena`, ratings
-    updated game by game from 1500."""
+    updated game by game from 1500.  `openings`: every pairing plays from these opening positions, each twice with the colours
+    swapped (`Arena(openings=)`): at temperature 0 the games are otherwise the same two games repeated."""
     ratings: dict = defaultdict(lambda: 1500)
     if search_kwargs.get("forced_playouts") is not None:
         raise ValueError("forced_playouts is a self-play option: the ladder's players pick their moves from raw root visit counts")
     players = {name: AlphaZeroPlayer(m, mcts_simulation=mcts_simulation, temperature=temperature, **search_kwargs) for name, m in models.items()}
     for n1, n2 in combinations(list(models), 2):
-        res = Arena(players[n1], players[n2], initial_state).play(games_per_pair)
+        res = Arena(players[n1], players[n2], initial_state, openings).play(games_per_pair)
         for s in res["scores"]:
             ratings[n1], ratings[n2] = update_elo(ratings[n1], ratings[n2], float(s), K)
     return {name: ratings[name] for name in models}

@@ -335,14 +335,16 @@ class AlphaZeroSearch:
         cap = self.playout_cap is not None
         redraw = 1 if cap and reuse else 0  # k_cap_draw after k_reroot (without reuse k_sample_moves draws the next budgets itself)
         forced = self.forced_playouts is not None
+        openings = 1 if self._engine is not None and self._engine.openings is not None else 0  # k_openings after the move
         if self._mode == "builtin":
             # one k_run_sims per run, the last one with the move fused in - unless the greedy cutoff, subtree reuse, the playout cap,
-            # forced playouts (or a search of one simulation with noise) leave the move to k_sample_moves
-            return len(runs) + noise + (1 if greedy or reuse or cap or forced or noise and S == 1 else 0) + reuse + redraw
+            # forced playouts, openings (or a search of one simulation with noise) leave the move to k_sample_moves
+            split = greedy or reuse or cap or forced or openings or noise and S == 1
+            return len(runs) + noise + (1 if split else 0) + reuse + redraw + openings
         # per run of n: k_select; n - 1 x (evaluator or gather, k_expand_select); evaluator, k_expand_backup.  Then k_root_noise
         # between the runs and k_sample_moves.  When the evaluator walks the compacted leaf list: one k_compact_leaves after
         # every k_select (the later lists come out of k_expand_select) or, AZ_COMPACT_FUSED=0, one per selection
-        n = sum(2 * r + 1 for r in runs) + noise + 1 + reuse + redraw
+        n = sum(2 * r + 1 for r in runs) + noise + 1 + reuse + redraw + openings
         if not getattr(self._net, "wants_leaf_compaction", False):
             return n
         return n + (len(runs) if os.environ.get("AZ_COMPACT_FUSED", "1") != "0" else S)

@@ -150,7 +150,7 @@ class Trainer:
               overlap: bool = True, inference_dtype: torch.dtype | None = None, precision: str = "32-true",
               cuda_graph: bool = True, trainer_share: float | None = None, save_dir: str | None = None, root_noise=None,
               sampling_moves: int | None = None, symmetric: bool = False, mirror_augment: bool = False,
-              subtree_reuse: bool | int = False, playout_cap=None, forced_playouts=None):
+              subtree_reuse: bool | int = False, playout_cap=None, forced_playouts=None, openings=None):
         """`overlap=True` reproduces the reference's pipeline (datamodule.py:89-101): the self-play of iteration k+1 runs on a
         background thread (own CUDA stream, weights as of the end of iteration k-1's training) while iteration k trains.
         `precision`: "32-true" (the reference's Lightning default) or "bf16-mixed" (forward / backward under bf16 autocast,
@@ -174,7 +174,9 @@ class Trainer:
         (`AlphaZeroSearch(playout_cap=)`); off by default.  Like `root_noise`, its `slot_offset` is set to the rank's first game.
         `forced_playouts` (`search.ForcedPlayouts`): self-play forces root visits and records the pruned counts
         (`AlphaZeroSearch(forced_playouts=)`); off by default.  Pruned counts no longer sum to N - 1, so the replay buffer then divides
-        each sample's counts by their sum, as for subtree reuse."""
+        each sample's counts by their sum, as for subtree reuse.
+        `openings` (`openings.Openings`): self-play games start from opening positions (`EpisodeGenerator(openings=)`); off by
+        default.  Like `root_noise`, its `slot_offset` is set to the rank's first game, so a sharded run starts the same games."""
         import threading
 
         world = dist.get_world_size() if dist.is_initialized() else 1
@@ -199,7 +201,8 @@ class Trainer:
         if forced_playouts is not None:
             kw["forced_playouts"] = forced_playouts
         gen = EpisodeGenerator(model=model, num_simulations=simulations_per_episode, num_episodes=hi - lo,
-                               game_initial_state=initial_state, device=self.device_index, sampling_moves=sampling_moves, **kw)
+                               game_initial_state=initial_state, device=self.device_index, sampling_moves=sampling_moves,
+                               openings=None if openings is None else dataclasses.replace(openings, slot_offset=lo), **kw)
         replay = ReplayBuffer(buffer_size, simulations_per_episode, self.device, subtree_reuse="subtree_reuse" in kw or "forced_playouts" in kw)
         opt = model.configure_optimizers()
         for group in opt.param_groups:  # Adam's step counter on the device, so that optimiser steps can be captured

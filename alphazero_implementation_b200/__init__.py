@@ -16,6 +16,7 @@ from .evaluators import HashEvaluator, UniformEvaluator  # noqa: E402,F401
 from .game import Action, Config, State, canonical_bitboards, mirror_bitboards  # noqa: E402,F401
 from .episode import Episode, Sample  # noqa: E402,F401
 from .search import AlphaZeroSearch, ForcedPlayouts, Node, PlayoutCap, RootNoise  # noqa: E402,F401
+from .openings import Openings, distinct_openings  # noqa: E402,F401
 from .episode_generator import EpisodeGenerator  # noqa: E402,F401
 from .models import BasicNN, CNNModel, Connect4Model, Model, ResNet  # noqa: E402,F401
 from .player import AlphaZeroPlayer, Arena, Player, calculate_expected_score, elo_ladder, play_game, update_elo  # noqa: E402,F401

@@ -348,6 +348,41 @@ typedef struct az_cap_stats {
 /* totals since az_create / az_reset_stats.  Synchronises. */
 int32_t az_get_cap_stats(az_engine *h, az_cap_stats *out_host, void *stream);
 
+/* Opening positions (off by default, and with it off every result is unchanged): each self-play game starts from a position drawn
+ * from a set, or from the az_reset_games position, followed by a few seeded random plies - an arena then plays different games at
+ * temperature 0, and self-play visits more positions.  A game starts on global slot g = slot_offset + slot at move step s, the step of
+ * its first search: s = 0 for every slot after az_reset_games, s = t + 1 for a slot that move step t (az_sample_moves /
+ * az_run_move_step) recycled; (g, s) identifies the game.  Its opening:
+ *   1. X_j = Philox4x32-10(key = {seed lo, seed hi}, counter = {g lo, g hi, s, 0xA0000000 | j}) - never a counter of the playout cap
+ *      (0xC0000000) or of the root noise (column << 24 | attempt, column <= 6);
+ *   2. base = the az_reset_games position when n_positions = 0, else entry (X_0.x * n_positions) >> 32 of the set (64-bit product);
+ *   3. r = min_plies + ((X_0.y * (max_plies - min_plies + 1)) >> 32) random plies (a base that has ended gets none);
+ *   4. ply j = 1 .. r: the candidates are the legal columns, ascending, whose drop neither completes four for the side to move nor
+ *      fills the board; none left ends the opening early, else candidates[(X_j.x * count) >> 32] is played and the side to move flips.
+ * The opening becomes the slot's root with a fresh tree.  The random plies are not in the game log and are not samples: the game's
+ * first sample is the opening, and the greedy cutoff (az_set_greedy_from) counts the game's searched plies.  While the mode is on,
+ * az_run_move_step runs as the search followed by az_sample_moves, and az_sample_moves ends with one k_openings launch over the slots
+ * whose game ended (its `finished` flags, or an engine-owned array when the caller passes NULL).  az_set_roots and az_advance_roots are
+ * not self-play and ignore the mode. */
+typedef struct az_openings {
+    const uint64_t *bb0, *bb1;    /* device, n_positions entries; may be NULL when n_positions = 0 */
+    const uint8_t *player;
+    int32_t n_positions;          /* 0 = the az_reset_games position is the base */
+    int32_t min_plies, max_plies; /* 0 <= min_plies <= max_plies <= 40 */
+    uint64_t seed;
+    int64_t slot_offset;          /* global index of this engine's slot 0, [0, 2^62] */
+} az_openings;
+/* cfg NULL = off (the default); applies to the games that start after the call.  Copies the set into engine memory (the caller's
+ * buffers are borrowed for the call only) and checks every entry: disjoint boards, only bits of the 6 x 7 board, no stone above an
+ * empty cell, player 0 or 1, no four for either side and not full - AZ_E_INVALID naming the first bad index otherwise, and for values
+ * out of range.  Synchronises.  AZ_E_STATE while a selection's leaves wait for their expansion. */
+int32_t az_set_openings(az_engine *h, const az_openings *cfg);
+/* the openings of the games of global slots first_slot .. first_slot + n - 1 that would start at move step `step` (a pure query on
+ * the current configuration and az_reset_games position; the same code as the engine's own draw).  Outputs: device or pinned host
+ * arrays of n entries.  AZ_E_STATE while the mode is off. */
+int32_t az_opening_positions(az_engine *h, int64_t first_slot, int64_t n, uint32_t step, uint64_t *out_bb0, uint64_t *out_bb1,
+                             uint8_t *out_player, void *stream);
+
 /* Forced playouts and policy target pruning (KataGo, Wu 2019 section 3.1): every root child gets a minimum number of visits, and
  * those visits are taken back out of the recorded policy target as far as PUCT would not have chosen them anyway.  All arithmetic
  * is fp64 with one rounding per operation (RN), as in the PUCT score.
